@@ -33,6 +33,7 @@ sys.path.insert(0, ROOT)
 
 INSERT_LO, INSERT_HI = 250, 500
 INSERT_HIGH_OPT = 750           # soap4 -u 750
+DUMP_ROWS = 8192                # --dump-outputs: rows per result array (keeps a dump under 64 MB)
 
 # BASELINE.json configs (SURVEY.md 8d).  `-L` is read length + 1: the reference truncates reads to L - 1 (QueryParser.cpp:188).
 CONFIGS = {
@@ -78,10 +79,15 @@ def parse_args():
                     help="build what the CPU legs need and exit: the workload's index files (GPU builder, reference file formats) and the "
                          "FASTQ samples.  `--impl reference` runs this in a child process, so that the process which times the reference "
                          "never loads this repo's library")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the result arrays of the last timed step as DIR/<array>.<field>.npy (float64; "
+                         "CIGARs as float32 byte rows), at most %d rows per array in a fixed, seeded sample" % DUMP_ROWS)
     ap.add_argument("--profile-step", action="store_true",
                     help="profiling aid (ncu --profile-from-start off): after the warm-up run ONE step on one context between "
                          "cudaProfilerStart/Stop and exit; prints no bench value")
     a = ap.parse_args()
+    if a.dump_outputs and a.steps < 1:
+        ap.error("--dump-outputs writes the results of the last timed step: it needs --steps 1 or more")
     a.cfg = dict(CONFIGS[a.config])
     if a.ref_mbp > 0:
         a.cfg["ref_mbp"] = a.ref_mbp
@@ -247,6 +253,62 @@ def write_fastq_sample(path_prefix, codes_np):
         with open("%s_%d.fq.tmp" % (path_prefix, mate + 1), "wb") as f:
             f.write(rec.tobytes())
         os.replace("%s_%d.fq.tmp" % (path_prefix, mate + 1), "%s_%d.fq" % (path_prefix, mate + 1))
+
+
+def summary_keeping_results(c, P):
+    """Context.align_pairs_summary for the step whose results --dump-outputs writes: the same mp_align_pairs call and counters, but
+    the result set stays in the library's host arena (valid until c's next mp_align_pairs) -> (summary, mp_results)"""
+    import ctypes as C
+    import megapath_b200 as mp
+    res = mp.Results()
+    c._check(c.L.mp_align_pairs(c.h, C.byref(P), C.byref(res)))
+    out = {name: getattr(res, name) for name, _ in mp.Results._fields_[8:]}
+    out.update(c.last_stats())
+    out["n_pairs"], out["n_singles"], out["n_rescued"] = res.n_pairs, res.n_singles, res.n_rescued
+    out["result_bytes"] = (res.n_pairs + res.n_rescued) * mp.PAIR_RESULT.itemsize + res.n_singles * mp.SINGLE_RESULT.itemsize + res.cigar_bytes
+    out["pairs_aligned"] = res.numDPAlignedPair + res.numRescuedPair
+    return out, res
+
+
+def copy_results(c, res):
+    """numpy copies of the arrays of a result set summary_keeping_results left with context c; releases it"""
+    import ctypes as C
+    import megapath_b200 as mp
+
+    def arr(p, n, dt):
+        return np.frombuffer((C.c_char * (n * dt.itemsize)).from_address(p), dtype=dt).copy() if n else np.zeros(0, dtype=dt)
+    out = dict(pairs=arr(res.pairs, res.n_pairs, mp.PAIR_RESULT), rescued=arr(res.rescued, res.n_rescued, mp.PAIR_RESULT),
+               singles=arr(res.singles, res.n_singles, mp.SINGLE_RESULT),
+               cigars=bytes((C.c_char * res.cigar_bytes).from_address(res.cigars)) if res.cigar_bytes else b"")
+    c.L.mp_results_release(c.h, C.byref(res))
+    return out
+
+
+def dump_outputs(path, res):
+    """The result set of mp_align_pairs (what a caller of the timed path receives) -> path/<array>.<field>.npy: the same seeded
+    sample of rows for every field; CIGAR offsets replaced by the CIGAR text (one zero-padded byte row per result), so that two
+    builds compare equal when they print the same alignments.  An array the step left empty (no rescued pairs, say) is not
+    written; counts.npy holds the number of results of each array."""
+    import megapath_b200 as mp
+    os.makedirs(path, exist_ok=True)
+    for seed, name in enumerate(("pairs", "rescued", "singles")):
+        a = res[name]
+        if not len(a):
+            continue
+        rng = np.random.default_rng(seed)
+        rows = np.sort(rng.choice(len(a), size=DUMP_ROWS, replace=False)) if len(a) > DUMP_ROWS else np.arange(len(a))
+        np.save(os.path.join(path, name + ".row.npy"), rows.astype(np.float64))
+        for f in a.dtype.names:
+            col = a[f][rows]
+            if f.startswith("cigar"):
+                text = [mp.cigar_at(res["cigars"], int(o)) for o in col]
+                out = np.zeros((len(text), max([len(t) for t in text] + [1])), dtype=np.float32)
+                for i, t in enumerate(text):
+                    out[i, :len(t)] = np.frombuffer(t, dtype=np.uint8)
+                np.save(os.path.join(path, "%s.%s.npy" % (name, f)), out)
+            else:
+                np.save(os.path.join(path, "%s.%s.npy" % (name, f)), col.astype(np.float64))
+    np.save(os.path.join(path, "counts.npy"), np.array([len(res["pairs"]), len(res["rescued"]), len(res["singles"])], dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -604,13 +666,20 @@ def run(args, saved_stdout):
     nctx = max(1, args.contexts)
     ctxs = [ctx]
 
-    def run_steps(c, ids, upload, acc_out):
-        """steps `ids` on context c; upload=True: host buffers in (pinned -> HBM) every step"""
+    kept = []
+
+    def run_steps(c, ids, upload, acc_out, keep_step=None):
+        """steps `ids` on context c; upload=True: host buffers in (pinned -> HBM) every step; the result set of step `keep_step`
+        stays with c and goes to `kept`"""
         for i in ids:
             if upload:
                 c.batch_upload_ptr(batches[i % nb].data_ptr(), lens, wpq)
             t_call = time.perf_counter()
-            s = c.align_pairs_summary(P)
+            if i == keep_step:
+                s, res = summary_keeping_results(c, P)
+                kept.append((c, res))
+            else:
+                s = c.align_pairs_summary(P)
             if os.environ.get("MP_BENCH_VERBOSE"):
                 sys.stderr.write("  ctx %d step %d upload=%d: call %.1f ms (lib wall %.1f, seed %.1f, dp %.1f, fill %.1f, tb %.1f)\n" % (
                     ctxs.index(c) if c in ctxs else -1, i, int(upload), (time.perf_counter() - t_call) * 1e3, s["ms_wall"], s["ms_seed"], s["ms_dp"], s["ms_fill"], s["ms_tb"]))
@@ -648,7 +717,7 @@ def run(args, saved_stdout):
     if os.environ.get("MP_BENCH_VERBOSE"):
         sys.stderr.write("rank %d loop R: %s\n" % (rank, json.dumps(dict({k: round(v / args.steps, 3) for k, v in acc.items() if k.startswith("ms_")}, exact=acc.get("dp_tasks_exact", 0) / max(1, acc.get("dp_tasks", 1))))))
 
-    def pipelined(upload):
+    def pipelined(upload, keep_step=None):
         """K steps pulled from one queue by the contexts (one host thread each), so that a K that is not a multiple of the
         number of contexts leaves no context idle longer than one step; -> wall seconds between device syncs"""
         accs = [dict() for _ in ctxs]
@@ -663,7 +732,7 @@ def run(args, saved_stdout):
                 if i >= args.warmup + args.steps:
                     return
                 yield i
-        ths = [threading.Thread(target=run_steps, args=(c, ids(), upload, accs[ci])) for ci, c in enumerate(ctxs)]
+        ths = [threading.Thread(target=run_steps, args=(c, ids(), upload, accs[ci], keep_step)) for ci, c in enumerate(ctxs)]
         barrier()
         t0 = time.perf_counter()
         for t in ths:
@@ -681,9 +750,13 @@ def run(args, saved_stdout):
     dev_ms = dev_s * 1e3
     pairs_aligned_A = sum(a.get("pairs_aligned", 0) for a in accsA)
     # ---- loop B (e2e): the same through host buffers: pinned-host -> HBM upload of every batch, results in host memory ----
-    e2e_s, accsB = pipelined(True)
+    last_step = args.warmup + args.steps - 1
+    e2e_s, accsB = pipelined(True, last_step if args.dump_outputs else None)
     d2h = sum(a.get("result_bytes", 0) for a in accsB) / max(1, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        # loop B is the last timed pass; its last step aligned batch last_step % nb, the same batch on every run with these arguments
+        dump_outputs(os.path.join(args.dump_outputs, "rank%d" % rank) if world > 1 else args.dump_outputs, copy_results(*kept[0]))
 
     from megapath_b200 import shard
     dev_ms_max, e2e_ms_max = shard.max_over_ranks([dev_ms, e2e_s * 1e3], device=device)     # slowest rank decides

@@ -139,12 +139,10 @@ LSAM_CASES = (b"@r1\tSCORE:50;50,seqA;48,seqB,seqC;\nACGT\n+\nIIII\n@r1\tIGNORE\
 @pytest.mark.parametrize("output_seq", ["1", "0"])
 def test_lsam_mode_matches_reference_fastq2lsam(tmp_path, output_seq):
     """-lsam (the fused fastq2lsam step) prints what the reference's own cc/fastq2lsam prints for the same annotated FASTQ"""
-    ref = os.path.join(ROOT, "oracle", "_ref", "fastq2lsam")
-    if not os.path.exists(ref):
-        pytest.skip("oracle/_ref/fastq2lsam not built")
+    from conftest import run_ref_fastq2lsam
     f = tmp_path / "a.fq"
     f.write_bytes(LSAM_CASES)
-    want = subprocess.run([ref, output_seq], stdin=open(f, "rb"), capture_output=True, check=True, timeout=60).stdout
+    want = run_ref_fastq2lsam("cases", LSAM_CASES, output_seq, str(tmp_path))
     got = subprocess.run([EXE, "__lsam", str(f), output_seq], capture_output=True, check=True, timeout=60).stdout
     assert want.count(b"\n") == 10
     assert got == want
@@ -249,9 +247,7 @@ def test_lsam_mode_randomized_against_reference_fastq2lsam(tmp_path, output_seq)
     """20 000 records with generated comments -- IGNORE, zero / negative / signed scores, lists with several accessions per score, empty
     fields, long scores with dozens of one-letter accessions (the list outgrows twice the comment), names with and without /1 /2,
     unpaired names -- through -lsam and through the reference's own cc/fastq2lsam"""
-    ref = os.path.join(ROOT, "oracle", "_ref", "fastq2lsam")
-    if not os.path.exists(ref):
-        pytest.skip("oracle/_ref/fastq2lsam not built")
+    from conftest import run_ref_fastq2lsam
     rng = np.random.default_rng(int(output_seq) + 5)
     out = []
     for i in range(10000):
@@ -282,7 +278,7 @@ def test_lsam_mode_randomized_against_reference_fastq2lsam(tmp_path, output_seq)
             out.append(b"@" + name + b"\t" + c + b"\n" + b"ACGT"[m:m + 1] * L + b"\n+\n" + b"I" * L + b"\n")
     f = tmp_path / "r.fq"
     f.write_bytes(b"".join(out))
-    want = subprocess.run([ref, output_seq], stdin=open(f, "rb"), capture_output=True, check=True, timeout=120).stdout
+    want = run_ref_fastq2lsam("randomized", b"".join(out), output_seq, str(tmp_path))
     got = subprocess.run([EXE, "__lsam", str(f), output_seq], capture_output=True, check=True, timeout=120).stdout
     assert want.count(b"\n") == 20000 and want.count(b"\t64\t") > 8000 and want.count(b"\t0\t") > 1000
     assert got == want

@@ -6,7 +6,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import make_reads, run_ref_soap4, run_our_soap4, canon_fastq, needs_ref, deinterleave, run_ref_raw
+from conftest import make_reads, run_ref_soap4, run_our_soap4, canon_fastq, deinterleave, run_ref_raw
 
 pytestmark = pytest.mark.gpu
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -30,7 +30,6 @@ def first_diff(a, b):
     return min(len(la), len(lb)), b"<end>", b"<end>"
 
 
-@needs_ref
 @pytest.mark.parametrize("name,rlen,lopt,kw,ini,extra", E2E_SETS)
 def test_e2e_stdout_matches_reference(workdir, small_ref, name, rlen, lopt, kw, ini, extra):
     npairs = 3000 if name != "long" else 800
@@ -73,7 +72,6 @@ BAM_SETS = [
 ]
 
 
-@needs_ref
 @pytest.mark.parametrize("name,rlen,lopt,kw,ini,extra", BAM_SETS)
 def test_e2e_bam_matches_reference(workdir, small_ref, name, rlen, lopt, kw, ini, extra):
     """-b: decoded records of .dpout.1 + .gout.* + .unpair (flag, pos, MAPQ, CIGAR, mate fields, isize, seq, qual, every tag)
@@ -89,13 +87,10 @@ def test_e2e_bam_matches_reference(workdir, small_ref, name, rlen, lopt, kw, ini
                               extra=[x for x in extra if x not in ("-F", "-nc")])
     # run_ref_soap4 always passes -F -nc; the "nofq" set needs a run without them
     if "-F" not in extra:
-        import subprocess
-        from conftest import REF_DIR
         for f in glob.glob(pre_r + ".*"):
             if os.path.isfile(f) and not f.endswith(".fq"):
                 os.remove(f)
-        subprocess.check_call([os.path.join(REF_DIR, "soap4"), "pair", small_ref["prefix"], fq1, fq2, "-o", pre_r, "-C", os.path.join(REF_DIR, ini),
-                               "-L", str(lopt), "-T", "3", "-u", "750"] + list(extra), stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, cwd=workdir)
+        run_ref_raw(workdir, small_ref["prefix"], fq1, fq2, "bamref_" + name, lopt, ini, list(extra))
     got_fq = run_our_soap4(workdir, small_ref["prefix"], fq1, fq2, "bamour_" + name, lopt, ini=ini, extra=extra)
     if "-F" in extra:
         assert canon_fastq(got_fq) == canon_fastq(open(ref_fq, "rb").read())
@@ -113,7 +108,6 @@ def _write_fq(path, recs, mate):
             f.write(b"@e%d/%d\n" % (i, mate) + s + b"\n+\n" + b"I" * len(s) + b"\n")
 
 
-@needs_ref
 def test_e2e_edge_cases_match_reference(workdir, small_ref):
     """Ragged and degenerate inputs: reads longer than -L (truncated to L-1, QueryParser.cpp:188), short reads, all-N reads
     (N -> G, IndexHandler.cpp:41-45), a read made of the last bases of the text, lower-case bases.
@@ -148,7 +142,6 @@ def test_e2e_edge_cases_match_reference(workdir, small_ref):
         assert got == want, first_diff(got, want)
 
 
-@needs_ref
 def test_e2e_empty_input(workdir, small_ref):
     fq1, fq2 = os.path.join(workdir, "empty_1.fq"), os.path.join(workdir, "empty_2.fq")
     open(fq1, "wb").close()
@@ -170,7 +163,6 @@ def _edit_comments(k, mate, comm):
     return comm
 
 
-@needs_ref
 @pytest.mark.parametrize("mode", ["F", "P", "Fb"])
 def test_e2e_chained_comments_match_reference(workdir, small_ref, second_ref, mode):
     import glob
@@ -197,7 +189,6 @@ def test_e2e_chained_comments_match_reference(workdir, small_ref, second_ref, mo
             assert a == b, (a, b)
 
 
-@needs_ref
 @pytest.mark.parametrize("lopt", [76, 121, 201])
 def test_e2e_max_read_length_sweep(workdir, small_ref, lopt):
     """-L sweep (BASELINE config 5): reads of exactly L-1 bases and mixed shorter ones, margins 25 / 30, K = 5 and 8 column strips"""
@@ -211,7 +202,6 @@ def test_e2e_max_read_length_sweep(workdir, small_ref, lopt):
     assert got == want, first_diff(got, want)
 
 
-@needs_ref
 def test_e2e_threads_and_contexts(workdir, small_ref, monkeypatch):
     """-T 7 and two contexts on one GPU (MP_CONTEXTS_PER_GPU=2) over several small batches (MP_BATCH_READS) give the single-context
     output: batches alternate between contexts that share the resident index (mp_clone)."""
@@ -225,7 +215,6 @@ def test_e2e_threads_and_contexts(workdir, small_ref, monkeypatch):
         assert got == want, (nctx, first_diff(got, want))
 
 
-@needs_ref
 def test_e2e_cigar_text_fallback(workdir, small_ref, monkeypatch):
     """The traceback leaves each special CIGAR at the end of its pattern row and stage-S1 assembly copies it; when pattern and text
     would not both fit the row the assembly encodes from the pattern instead.  MP_CIG_TEXT=0 forces that path for every result:
@@ -235,14 +224,12 @@ def test_e2e_cigar_text_fallback(workdir, small_ref, monkeypatch):
     test_e2e_bam_matches_reference(workdir, small_ref, "cigfb_" + name, rlen, lopt, kw, ini, extra)
 
 
-@needs_ref
 def test_e2e_lsam_mode_matches_reference_pipe(workdir, small_ref):
     """`soap4 ... -F -lsam 1` == `reference soap4 ... -F | cc/fastq2lsam 1` (runMegaPath.sh:136), pair lines sorted by name"""
-    import subprocess
-    from conftest import REF_DIR
+    from conftest import run_ref_fastq2lsam
     fq1, fq2 = make_reads(workdir, small_ref, "lsam", 2000, 150, seed=5, model="divergent", one_random=0.10, unalignable=0.05)
     first = run_ref_raw(workdir, small_ref["prefix"], fq1, fq2, "lsamref", 151, "soap4-nt2.ini", ["-F", "-nc", "-top", "95"])
-    want = subprocess.run([os.path.join(REF_DIR, "fastq2lsam"), "1"], input=first, capture_output=True, check=True).stdout
+    want = run_ref_fastq2lsam("e2e_lsam", first, "1", workdir, ordered=False)
     got = run_our_soap4(workdir, small_ref["prefix"], fq1, fq2, "lsamour", 151, ini="soap4-nt2.ini", extra=("-F", "-nc", "-top", "95", "-lsam", "1"))
 
     def canon(data):
@@ -253,14 +240,12 @@ def test_e2e_lsam_mode_matches_reference_pipe(workdir, small_ref):
     assert canon(got) == canon(want)
 
 
-@needs_ref
 def test_e2e_builder_with_ambiguity_runs(workdir):
     """bin/2bwt-builder on a FASTA with short / long N runs, IUPAC codes and lower case: every index file equals the reference
     builder's (HSP.c:486-528 cut-outs + translate table), and soap4 on that index prints the reference's records (positions behind
     cut-out runs go through the translate table's corrections)."""
-    import shutil
     import subprocess
-    from conftest import REF_DIR, ROOT
+    from conftest import ROOT, build_index
     from test_builder_fasta import fasta_with_ambiguity
     d = os.path.join(workdir, "amb")
     os.makedirs(d, exist_ok=True)
@@ -268,8 +253,7 @@ def test_e2e_builder_with_ambiguity_runs(workdir):
     fa_ref, fa_our = os.path.join(d, "ref.fa"), os.path.join(d, "our.fa")
     for p in (fa_ref, fa_our):
         open(p, "wb").write(raw)
-    shutil.copy(os.path.join(REF_DIR, "2bwt-builder.ini"), os.path.join(d, "2bwt-builder.ini"))
-    subprocess.check_call([os.path.join(REF_DIR, "2bwt-builder"), fa_ref], cwd=d, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    build_index(fa_ref, "amb")
     subprocess.check_call([os.path.join(ROOT, "megapath_b200", "bin", "2bwt-builder"), fa_our], cwd=d, stdout=subprocess.DEVNULL)
     for ext in ("pac", "bwt", "fmv", "sa", "lkt", "tra", "amb"):
         assert open(fa_ref + ".index." + ext, "rb").read() == open(fa_our + ".index." + ext, "rb").read(), ext
@@ -316,7 +300,6 @@ def test_e2e_builder_with_ambiguity_runs(workdir):
         assert x == y, (x, y)
 
 
-@needs_ref
 def test_e2e_text_beyond_2_to_32(workdir):
     """BASELINE config 3 in small: a 4.4 Gbp synthetic reference (> 2^32 bases: 64-bit positions everywhere, bucketed index builder, sampled
     suffix array with LF walks, no dense 32-bit SA), soap4-nt2.ini -F -top 95, against the reference binary on the same index files.
@@ -326,7 +309,6 @@ def test_e2e_text_beyond_2_to_32(workdir):
     import torch
     import megapath_b200 as mp
     import bench
-    from conftest import REF_DIR
     if os.environ.get("MP_SKIP_HUGE"):
         pytest.skip("MP_SKIP_HUGE set")
     free, total = torch.cuda.mem_get_info(0)

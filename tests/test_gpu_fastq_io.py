@@ -8,7 +8,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from conftest import ROOT, make_reads, canon_fastq, needs_ref, deinterleave, run_ref_raw, load_pairs
+from conftest import ROOT, make_reads, canon_fastq, deinterleave, run_ref_raw, load_pairs
 
 pytestmark = pytest.mark.gpu
 
@@ -47,7 +47,6 @@ SETS = [
 CASES = [(s, 0) for s in SETS] + [(s, 1024) for s in SETS if s[0] in ("mixed", "var", "nt2")]
 
 
-@needs_ref
 @pytest.mark.parametrize("case", CASES, ids=["%s-%d" % (s[0], b) for s, b in CASES])
 def test_device_io_is_byte_identical_to_host_io(workdir, small_ref, case):
     (name, rlen, lopt, kw, ini, flags), batch = case
@@ -83,7 +82,6 @@ def _edit_comments(k, mate, comm, unsafe=False):
     return comm
 
 
-@needs_ref
 @pytest.mark.parametrize("mode", ["-F", "-P"])
 def test_device_io_chained_comments(workdir, small_ref, second_ref, mode):
     """Without -nc (every NT chunk after the first, runMegaPath.sh:199): previous SCORE: lists merged on the device ==
@@ -107,7 +105,6 @@ def test_device_io_chained_comments(workdir, small_ref, second_ref, mode):
     assert dev == host, first_diff(dev, host)
 
 
-@needs_ref
 def test_device_io_falls_back_on_anything_but_strict_fastq(workdir, small_ref):
     """CRLF line ends, multi-line records and a missing final newline are not for the kernels: the driver says so and the host
     parser takes the run -- same output as with MP_HOST_IO=1."""
@@ -132,7 +129,6 @@ def test_device_io_falls_back_on_anything_but_strict_fastq(workdir, small_ref):
         assert got == want, (tag, first_diff(got, want))
 
 
-@needs_ref
 def test_fastq_upload_equals_batch_upload(workdir, small_ref):
     """Kernel seam: mp_fastq_upload leaves the batch exactly as the host packing + mp_batch_upload does -- same clamped lengths,
     same SeedPos arrays and candidates from the seeding stage -- for names with and without /1, comments, variable lengths,
@@ -181,7 +177,6 @@ def test_fastq_upload_equals_batch_upload(workdir, small_ref):
         c.close()
 
 
-@needs_ref
 def test_format_fastq_through_the_library(workdir, small_ref):
     """The C-ABI calls on their own (no driver): fastq_upload + align_pairs + format_fastq == bin/soap4 with the host loops."""
     import megapath_b200 as mp
@@ -207,7 +202,6 @@ def test_format_fastq_through_the_library(workdir, small_ref):
     c.close()
 
 
-@needs_ref
 def test_device_io_on_two_gpus(workdir, small_ref):
     """-G 2: batches dealt to the contexts of two GPUs (staging buffers are page-locked once, for every device) print the stream
     one GPU prints."""
@@ -222,13 +216,11 @@ def test_device_io_on_two_gpus(workdir, small_ref):
     assert two == one, first_diff(two, one)
 
 
-@needs_ref
 def test_device_io_long_score_lists(workdir):
     """Eight near-identical sequences with long names: every read has a SCORE: list of several entries, far longer than the 64-byte
     slot k_fmt_measure composes header tails in, so k_fmt_write's in-place path (and the staging buffer's growth allowance) is what
     prints them.  Device == host formatter byte for byte, == reference after the canonical sort."""
-    import shutil
-    from conftest import REF_DIR
+    from conftest import build_index
     from tools import synth
     rng = np.random.default_rng(99)
     base = synth.ALPHA[rng.integers(0, 4, size=30000)]
@@ -243,8 +235,7 @@ def test_device_io_long_score_lists(workdir):
             s[m] = synth.ALPHA[rng.integers(0, 4, size=int(m.sum()))]
             seqs.append(s)
             f.write(b">copy_%d_of_the_same_genome_with_a_long_description_line strain %d\n" % (i + 1, i) + s.tobytes() + b"\n")
-    shutil.copy(os.path.join(REF_DIR, "2bwt-builder.ini"), os.path.join(d, "2bwt-builder.ini"))
-    subprocess.check_call([os.path.join(REF_DIR, "2bwt-builder"), fa], cwd=d, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    build_index(fa, "copies")
     seq = np.concatenate(seqs)
     bounds = np.arange(9, dtype=np.int64) * 30000
     r1, r2 = synth.make_pairs(seq, bounds, 1500, 100, 5, model="clean")
@@ -263,7 +254,6 @@ def test_device_io_long_score_lists(workdir):
     assert got == want, first_diff(got, want)
 
 
-@needs_ref
 @pytest.mark.parametrize("output_seq", ["0", "1"])
 def test_device_io_lsam_mode(workdir, small_ref, output_seq):
     """-lsam: the device-made text, cut at pair boundaries and rewritten into fastq2lsam's lines by host threads, is byte-identical to
@@ -278,7 +268,6 @@ def test_device_io_lsam_mode(workdir, small_ref, output_seq):
         assert dev == host, first_diff(dev, host)
 
 
-@needs_ref
 def test_device_io_mid_file_fallback(workdir, small_ref):
     """A file that stops being strict four-line FASTQ after the first batch: a CR inside a later batch sends that batch (only) through
     the host parser and formatter -- same stream as the all-host run; a folded record, which moves the batch boundaries the newline

@@ -124,13 +124,9 @@ def test_gpu_index_build_matches_reference_builder(workdir, total, nseq, repeat_
     """mp_index_build + mp_index_save against the files 2bwt-builder writes for the same text
     (2BWT-Builder.c; BWTConstruct.c:994-1393; LTConstruct.c:46-96; HSP.c:560-699): byte-identical."""
     import os
-    import shutil
-    import subprocess
     import megapath_b200 as mp
-    from conftest import REF_DIR, have_ref
+    from conftest import build_index
     from tools import synth
-    if not have_ref():
-        pytest.skip("oracle/_ref not built")
     if large:
         monkeypatch.setenv("MP_BUILD_LARGE", "1")       # the bucketed builder that texts >= 2^32 take (mp_build_large.cu)
     d = os.path.join(workdir, "b%d" % total)
@@ -138,8 +134,7 @@ def test_gpu_index_build_matches_reference_builder(workdir, total, nseq, repeat_
     seq, bounds = synth.make_ref(total, nseq, seed=seed, repeat_frac=repeat_frac)
     fa = os.path.join(d, "r.fa")
     synth.write_fasta(fa, seq, bounds)
-    shutil.copy(os.path.join(REF_DIR, "2bwt-builder.ini"), os.path.join(d, "2bwt-builder.ini"))
-    subprocess.check_call([os.path.join(REF_DIR, "2bwt-builder"), fa], cwd=d, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    build_index(fa, "b%d" % total)
     codes = np.searchsorted(np.frombuffer(b"ACGT", dtype=np.uint8), seq).astype(np.uint8)
     c = mp.Context(0)
     c.index_build(mp.pack_text(codes), total)
