@@ -266,6 +266,20 @@ int  mp_format_fetch(mp_context *ctx, char *dst, uint64_t bytes);
 void *mp_host_alloc(uint64_t bytes);
 void  mp_host_free(void *p);
 
+/* ---- BGZF compression on the device: replaces the zlib deflate behind BgzfWriter (bgzf_write / bgzf_flush of samtools 0.1.18,
+ *      which the reference links for -b).  Any byte string in, a run of complete BGZF members out: each covers the next piece of at
+ *      most 0xff00 input bytes with the gzip header and its "BC" extra subfield (BSIZE), one final raw DEFLATE block (dynamic Huffman,
+ *      fixed Huffman or stored, whichever is smallest), CRC-32 and ISIZE.  No EOF marker: the writer appends it when it closes the
+ *      file.  The output depends on the input bytes only (the same on every call, context and GPU).
+ *      src and dst are host memory; page-locked memory from mp_host_alloc makes each copy one DMA.  Everything runs on the context's
+ *      stream and ends with a synchronise of that stream; no index or batch is needed and a resident batch or result set is left as it
+ *      is.  n == 0 writes nothing (*outBytes = 0); dstCap below MP_BGZF_BOUND(n) returns MP_ERR_ARG before anything is written. */
+#define MP_BGZF_BOUND(n) ((((uint64_t)(n) + 0xff00u - 1) / 0xff00u) * 65536u)
+int  mp_bgzf_compress(mp_context *ctx, const uint8_t *src, uint64_t n, uint8_t *dst, uint64_t dstCap, uint64_t *outBytes);
+/* sizes the context's compression buffers for calls of up to maxBytes input bytes before the batch loop (like mp_reserve: an
+ * allocation inside the loop stalls every context of the GPU while it runs); larger inputs are best fed in pieces of maxBytes */
+int  mp_bgzf_reserve(mp_context *ctx, uint64_t maxBytes);
+
 /* ---- roofline denominators measured on the spot (bench.py): kind 0 = random 32-byte gathers over an 8 GB table,
  *      1 = random 64-byte gathers (GB/s of requested bytes), 2 = packed 16-bit DPX issue rate (1e9 thread-instr/s) ---- */
 int  mp_microbench(mp_context *ctx, int kind, double *result);

@@ -136,6 +136,8 @@ def lib():
         L.mp_host_alloc.argtypes = [C.c_uint64]
         L.mp_host_alloc.restype = C.c_void_p
         L.mp_host_free.argtypes = [C.c_void_p]
+        L.mp_bgzf_reserve.argtypes = [C.c_void_p, C.c_uint64]
+        L.mp_bgzf_compress.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
         _lib = L
     return _lib
 
@@ -162,6 +164,11 @@ def pack_text(codes):
     c[:n] = codes
     c = c.reshape(-1, 4)
     return ((c[:, 0] << 6) | (c[:, 1] << 4) | (c[:, 2] << 2) | c[:, 3]).astype(np.uint8)
+
+
+def bgzf_bound(n):
+    """MP_BGZF_BOUND(n): output capacity mp_bgzf_compress needs for n input bytes."""
+    return (n + 0xff00 - 1) // 0xff00 * 65536
 
 
 def _ptr(a):
@@ -366,6 +373,19 @@ class Context:
         self._check(self.L.mp_format_fastq(self.h, C.byref(f), C.byref(n)))
         buf = C.create_string_buffer(max(int(n.value), 1))
         self._check(self.L.mp_format_fetch(self.h, buf, n.value))
+        return buf.raw[:n.value]
+
+    def bgzf_reserve(self, max_bytes):
+        """Pre-sizes the compression buffers for inputs of up to max_bytes (mp_bgzf_reserve)."""
+        self._check(self.L.mp_bgzf_reserve(self.h, int(max_bytes)))
+
+    def bgzf_compress(self, data):
+        """Device BGZF compression (mp_bgzf_compress): any bytes -> a run of complete BGZF members (no EOF marker)."""
+        data = bytes(data)
+        cap = bgzf_bound(len(data))
+        buf = C.create_string_buffer(max(cap, 1))
+        n = C.c_uint64()
+        self._check(self.L.mp_bgzf_compress(self.h, C.c_char_p(data), len(data), buf, cap, C.byref(n)))
         return buf.raw[:n.value]
 
     def seed_pairs(self, params):

@@ -9,8 +9,10 @@
 //   cigar / MD / mismatch counts   convertToCigarStr, getMisInfoForDP, readLengthWithCigar   PE.cpp:381-446, 459-625; BGS-IO.cpp:1917-1947
 //   MAPQ                           bwaLikeSingleQualScore, bwaLikePairQualScore, getMapQualScoreForDP(2), getMapQualScoreForSingleDP,
 //                                  getMapQualScoreForPair               BGS-IO.cpp:679-980
-// The BGZF container is written with zlib (the reference links samtools 0.1.18 for it); block boundaries are free,
-// the decoded byte stream is what must match.
+// The BGZF container: BgzfWriter writes the header and the EOF marker with zlib, and copies through blocks compressed elsewhere --
+// by the device (mp_bgzf_compress, csrc/mp_bgzf.cu) in the driver's default -b path, or by the formatting threads with zlib
+// (compress_all) under MP_HOST_IO=1 (the reference links samtools 0.1.18 for it).  Block boundaries are free, the decoded byte
+// stream is what must match.
 #pragma once
 #include <math.h>
 #include <stdint.h>

@@ -20,7 +20,9 @@
 // (stage_file / locate_records) and writes the finished text; records are indexed and packed, and the output text is composed, by
 // kernels (mp_fastq_upload, mp_format_fastq; csrc/mp_fastq.cu; with -lsam host threads rewrite that text).  Everything else -- .gz, pipes, BAM, text that is not strict
 // four-line FASTQ -- goes through the host parser (SeqReader, load_batch) and formatter (header_line, output_pair, output_unpaired)
-// below, which are also what MP_HOST_IO=1 forces and what the device path is tested against.
+// below, which are also what MP_HOST_IO=1 forces and what the device path is tested against.  With -b the formatting threads write
+// raw BAM records and each worker has its own context compress them into BGZF members (mp_bgzf_compress, csrc/mp_bgzf.cu);
+// MP_HOST_IO=1 keeps zlib on the formatting threads instead.
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -1295,6 +1297,16 @@ int main(int argc, char **argv)
             for (mp_context *c : contexts) if (mp_reserve(c, &P, batchReads)) { fprintf(stderr, "%s\n", mp_last_error()); return 1; }
         }
     }
+    // -b: BAM records are compressed on the device, by the worker's own context, in pieces of at most bgzfPiece bytes staged in
+    // page-locked buffers of the pool (two per context, made here so that the loop allocates nothing)
+    const bool deviceBgzf = opt.outputBAM && !getenv("MP_HOST_IO");
+    const uint64_t bgzfPiece = 512ull * 0xff00, bgzfCap = MP_BGZF_BOUND(bgzfPiece);
+    if (deviceBgzf) {
+        for (mp_context *c : contexts) {
+            if (mp_bgzf_reserve(c, bgzfPiece)) { fprintf(stderr, "%s\n", mp_last_error()); return 1; }
+            for (int k = 0; k < 2; ++k) { char *p = (char *)mp_host_alloc(bgzfCap); if (!p) { fprintf(stderr, "%s\n", mp_last_error()); return 1; } pin_give(p, bgzfCap); }
+        }
+    }
     if (pinThread.joinable()) pinThread.join();
     Annotation ann;
     if (!ann.load(opt.indexName)) return 1;
@@ -1493,7 +1505,7 @@ int main(int argc, char **argv)
             const uint32_t numQueries = j->nReads, nPairs = numQueries / 2;
             mp_results R;
             static const bool timing = getenv("MP_DRIVER_TIMING") != nullptr;      // per-batch host breakdown on stderr
-            double tUp = 0, tAl = 0, tFmt = 0, libWallMs = 0;
+            double tUp = 0, tAl = 0, tFmt = 0, libWallMs = 0, tCmp = 0;
             int rcUp = 0;
             if (j->dev && !j->uploaded) {
                 rcUp = mp_fastq_upload(gpu, j->raw.pin, j->raw.bytes1, j->raw.pin + j->raw.off2, j->raw.bytes2, nPairs, ((uint32_t)maxLen + 15) / 16, (uint32_t)maxLen, nullptr);
@@ -1606,12 +1618,35 @@ int main(int argc, char **argv)
                             chunks[c].fq.reserve((size_t)(cut[c + 1] - cut[c]) * (size_t)(4 * maxLen + 160));
                             body(occ, chunks[c].fq, cut[c], cut[c + 1]);
                             if (opt.lsam >= 0 && !chunks[c].fq.empty()) { std::string ls; fastq_chunk_to_lsam(chunks[c].fq.data(), chunks[c].fq.size(), opt.lsam != 0, ls); chunks[c].fq.swap(ls); }
-                            if (!chunks[c].bam.empty()) { BgzfWriter::compress_all(chunks[c].bam.data(), chunks[c].bam.size(), chunks[c].bamz); std::vector<uint8_t>().swap(chunks[c].bam); }
+                            if (!deviceBgzf && !chunks[c].bam.empty()) { BgzfWriter::compress_all(chunks[c].bam.data(), chunks[c].bam.size(), chunks[c].bamz); std::vector<uint8_t>().swap(chunks[c].bam); }
                         };
                         std::vector<std::thread> ths;
                         for (unsigned c = 1; c < nc; ++c) ths.emplace_back(one, c);
                         one(0);
                         for (std::thread &t : ths) t.join();
+                        if (deviceBgzf) {
+                            // the chunks' records, in order, through one staging buffer: every full piece is compressed as it fills
+                            const double tc0 = now_s();
+                            auto sp = pin_take(bgzfCap), dp = pin_take(bgzfCap);
+                            int rc = (!sp.first || !dp.first) ? MP_ERR_CUDA : 0;
+                            size_t fill = 0;
+                            auto flush = [&]() {
+                                uint64_t ob = 0;
+                                rc = mp_bgzf_compress(gpu, (const uint8_t *)sp.first, fill, (uint8_t *)dp.first, dp.second, &ob);
+                                if (!rc) j->bam[bamSlot].insert(j->bam[bamSlot].end(), (const uint8_t *)dp.first, (const uint8_t *)dp.first + ob);
+                                fill = 0;
+                            };
+                            for (Chunk &c : chunks)
+                                for (size_t at = 0; at < c.bam.size() && !rc;) {
+                                    const size_t k = std::min<size_t>(c.bam.size() - at, bgzfPiece - fill);
+                                    memcpy(sp.first + fill, c.bam.data() + at, k); fill += k; at += k;
+                                    if (fill == bgzfPiece) flush();
+                                }
+                            if (fill && !rc) flush();
+                            pin_give(sp.first, sp.second); pin_give(dp.first, dp.second);
+                            if (rc) { j->log += std::string(mp_last_error()) + "\n"; j->failed = true; }
+                            tCmp += now_s() - tc0;
+                        }
                         // the chunks stay separate strings (no 700 MB concatenation): the writer emits them in this order
                         for (Chunk &c : chunks) { j->fqParts.emplace_back(std::move(c.fq)); j->bam[bamSlot].insert(j->bam[bamSlot].end(), c.bamz.begin(), c.bamz.end()); }
                     };
@@ -1658,8 +1693,8 @@ int main(int argc, char **argv)
                 tFmt = now_s();
                 mp_results_release(gpu, &R);
             }
-            if (timing) fprintf(stderr, "[timing] batch %llu: upload %.3f align %.3f (lib wall %.3f) format %.3f release %.3f s; started at %.3f\n", (unsigned long long)j->seq,
-                                tUp - ts, tAl - tUp, libWallMs / 1e3, tFmt - tAl, now_s() - tFmt, ts - t0);
+            if (timing) fprintf(stderr, "[timing] batch %llu: upload %.3f align %.3f (lib wall %.3f) format %.3f (bgzf compress %.3f) release %.3f s; started at %.3f\n",
+                                (unsigned long long)j->seq, tUp - ts, tAl - tUp, libWallMs / 1e3, tFmt - tAl, tCmp, now_s() - tFmt, ts - t0);
             j->alignSeconds = now_s() - ts;
             std::lock_guard<std::mutex> lk(mu);
             if (j->b) { batchPool.push_back(j->b); j->b = nullptr; }   // the text output no longer refers to the batch

@@ -373,7 +373,8 @@ extern "C" void mp_destroy(mp_context *ctx)
                        &ctx->dRes, &ctx->dCig, &ctx->dExFlag, &ctx->dExPos, &ctx->dExIdx, &ctx->dAligned, &ctx->dGather, &ctx->dHintTest, &ctx->dRes2, &ctx->dKeep, &ctx->dKeepPos, &ctx->dTotals, &ctx->dS2Counts, &ctx->dS2Start, &ctx->dS2Tasks, &ctx->dS2Res,
                        &ctx->dRsSlotTasks, &ctx->dRsSlotInfo, &ctx->dRsFlag, &ctx->dRsPos, &ctx->dRsTasks, &ctx->dRsInfo, &ctx->dRsRec, &ctx->dRsOut, &ctx->dRsKeep, &ctx->dRsKeepPos,
                        &ctx->dFqText, &ctx->dFqCnt, &ctx->dFqCntPos, &ctx->dFqLines, &ctx->dFqRec, &ctx->dFqFlags, &ctx->dAnnGrid, &ctx->dAnnTrStart, &ctx->dAnnTrChr,
-                       &ctx->dAnnNames, &ctx->dAnnNameOff, &ctx->dFmtKeys, &ctx->dFmtGroups, &ctx->dFmtRecLen, &ctx->dFmtTail, &ctx->dFmtTailText, &ctx->dFmtSeg, &ctx->dFmtDst, &ctx->dFmtLen, &ctx->dFmtOff, &ctx->dFmtOut };
+                       &ctx->dAnnNames, &ctx->dAnnNameOff, &ctx->dFmtKeys, &ctx->dFmtGroups, &ctx->dFmtRecLen, &ctx->dFmtTail, &ctx->dFmtTailText, &ctx->dFmtSeg, &ctx->dFmtDst, &ctx->dFmtLen, &ctx->dFmtOff, &ctx->dFmtOut,
+                       &ctx->dBgzfIn, &ctx->dBgzfSlots, &ctx->dBgzfOut, &ctx->dBgzfSizes, &ctx->dBgzfOffs, &ctx->dBgzfScratch };
     for (DevBuf *b : bufs) b->release();
     for (int i = 0; i < 8; ++i) cudaEventDestroy(ctx->ev[i]);
     cudaStreamDestroy(ctx->stream);

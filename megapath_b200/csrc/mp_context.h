@@ -165,6 +165,9 @@ struct mp_context {
     DevBuf dAnnGrid, dAnnTrStart, dAnnTrChr, dAnnNames, dAnnNameOff;
     DevBuf dFmtKeys, dFmtGroups, dFmtRecLen, dFmtTail, dFmtTailText, dFmtSeg, dFmtDst, dFmtLen, dFmtOff, dFmtOut;
     uint64_t fmtBytes = 0; bool fmtReady = false;
+    // BGZF compression (mp_bgzf.cu): input, one 64 KiB member slot per 0xff00-byte piece, the packed stream, member sizes / offsets,
+    // and a match row per resident CTA
+    DevBuf dBgzfIn, dBgzfSlots, dBgzfOut, dBgzfSizes, dBgzfOffs, dBgzfScratch;
 };
 
 // mp_index.cu
