@@ -1,6 +1,7 @@
 """GPU suite: BGZF compression on the device (mp_bgzf_compress, csrc/mp_bgzf.cu) checked with an independent inflater (Python's
 zlib / gzip), member by member, against zlib's ratio on the same pieces, for determinism, and through the driver's -b output against
-the zlib path that MP_HOST_IO=1 keeps."""
+the zlib path that MP_HOST_IO=1 keeps; and byte for byte against the restatement oracle/pybgzf.py on the corpus of
+tests/test_bgzf_model.py, across grids, contexts and reserve sizes."""
 import ctypes
 import gzip
 import os
@@ -12,6 +13,7 @@ import numpy as np
 import pytest
 
 from conftest import ROOT, make_reads
+from test_bgzf_model import CORPUS, model_of
 
 pytestmark = pytest.mark.gpu
 
@@ -203,6 +205,137 @@ def test_argument_errors(ctx):
     assert L.mp_bgzf_compress(ctx.h, None, 10, buf, bound, ctypes.byref(n)) == -3
     assert L.mp_bgzf_reserve(ctx.h, 0) == -3
     ctx.bgzf_reserve(1 << 20)
+
+
+# ---- byte for byte against the restatement (oracle/pybgzf.py; its own checks are in tests/test_bgzf_model.py) ----
+
+def first_difference(got, want):
+    """where two member runs part: the first differing member, with what parse_member makes of each side"""
+    from oracle import pybgzf
+    gm, wm = pybgzf.split_members(got), pybgzf.split_members(want)
+    k = next((k for k, (g, w) in enumerate(zip(gm, wm)) if g != w), None)
+    if k is None:
+        return "%d members from the device, %d from the model" % (len(gm), len(wm))
+    msg, tokens = "member %d differs" % k, []
+    for side, m in (("device", gm[k]), ("model", wm[k])):
+        try:
+            P = pybgzf.parse_member(m)
+        except pybgzf.DeflateError as e:
+            msg += "\n  %s: undecodable: %s" % (side, e)
+            continue
+        tokens.append(P["tokens"])
+        msg += "\n  %s: %d bytes, btype %d, HLIT %s HDIST %s HCLEN %s, %d tokens, lit lens %s, dist lens %s, cl lens %s" % (
+            side, len(m), P["btype"], P["hlit"], P["hdist"], P["hclen"], len(P["tokens"]), P["lit_lens"], P["dist_lens"], P["cl_lens"])
+    if len(tokens) == 2:
+        a, b = tokens
+        j = next((j for j, (x, y) in enumerate(zip(a, b)) if x != y), min(len(a), len(b)))
+        msg += "\n  first differing token #%d: device %s, model %s" % (j, a[j] if j < len(a) else None, b[j] if j < len(b) else None)
+    return msg
+
+
+def assert_same_stream(got, want):
+    assert got == want, first_difference(got, want)
+
+
+@pytest.mark.parametrize("kind", KINDS)
+@pytest.mark.parametrize("size", SIZES)
+def test_device_equals_model(ctx, kind, size):
+    from oracle import pybgzf
+    data = contents(kind, size)
+    assert_same_stream(ctx.bgzf_compress(data), pybgzf.compress(data))
+
+
+@pytest.mark.parametrize("name", CORPUS)
+def test_device_equals_model_on_the_corpus(ctx, name):
+    """inputs that limit the literal/length and code-length trees, every length and distance code, the 32768 / 32769 window edge,
+    hash collisions, piece lengths at the ok3 / ok4 and tile edges"""
+    data, want, _ = model_of(name)
+    assert_same_stream(ctx.bgzf_compress(data), want)
+
+
+def sm_count():
+    import torch
+    return torch.cuda.get_device_properties(0).multi_processor_count
+
+
+def test_many_pieces_equal_the_model_at_sampled_pieces(ctx):
+    """64 MiB (about a thousand pieces, several per CTA): the first and last pieces, pieces sms - 1, sms, sms + 1 and 2 sms (the
+    second and third rounds of the persistent loop) and a seeded dozen, member bytes against the model"""
+    from oracle import pybgzf
+    one = bam_like(3000, seed=11) + fastq_text(2000, seed=12)
+    data = (one * ((64 << 20) // len(one) + 1))[:(64 << 20) + 4321]
+    members = pybgzf.split_members(ctx.bgzf_compress(data))
+    n = len(members)
+    assert n == (len(data) + PIECE - 1) // PIECE
+    sms = sm_count()
+    sample = {0, n - 1, sms - 1, sms, sms + 1, 2 * sms} | set(np.random.default_rng(8).choice(n, 12, replace=False).tolist())
+    for k in sorted(sample):
+        assert members[k] == pybgzf.member(data[k * PIECE:(k + 1) * PIECE]), "piece %d of %d (%d SMs)" % (k, n, sms)
+
+
+def test_output_does_not_depend_on_the_grid(ctx):
+    """one call over 3 sms + 5 pieces (sms CTAs, three or four pieces each) == calls on slices cut at piece boundaries (grids of 1,
+    2, 7, sms - 1, sms, sms + 1 CTAs), concatenated"""
+    sms = sm_count()
+    data = contents("fastq", (3 * sms + 5) * PIECE - 77)
+    whole = ctx.bgzf_compress(data)
+    parts, at = [], 0
+    for pieces in (1, 2, 7, sms - 1, sms, sms + 1, None):
+        end = len(data) if pieces is None else at + pieces * PIECE
+        parts.append(ctx.bgzf_compress(data[at:end]))
+        at = end
+    assert at == len(data)
+    assert_same_stream(b"".join(parts), whole)
+
+
+def test_two_contexts_at_once():
+    """two clones of one index owner compress different inputs at the same time from two threads (one context per worker thread,
+    as the driver runs them); each result equals the model's"""
+    import threading
+    import megapath_b200 as mp
+    from oracle import pybgzf
+    from tools import synth
+    owner = mp.Context(0)
+    seq, _ = synth.make_ref(20000, 1, seed=3, repeat_frac=0.0)
+    owner.index_build(mp.pack_text(np.searchsorted(np.frombuffer(b"ACGT", dtype=np.uint8), seq).astype(np.uint8)), len(seq))
+    clones = [owner.clone(), owner.clone()]
+    inputs = [contents("bam", 20 * PIECE + 999), contents("fastq", 23 * PIECE - 5)]
+    want = [pybgzf.compress(d) for d in inputs]
+    got = [[], []]
+    start = threading.Barrier(2)
+
+    def work(k):
+        start.wait()
+        for _ in range(4):
+            got[k].append(clones[k].bgzf_compress(inputs[k]))
+
+    threads = [threading.Thread(target=work, args=(k,)) for k in range(2)]
+    for t in threads:
+        t.start()
+    for t in threads:
+        t.join()
+    for k in range(2):
+        assert len(got[k]) == 4
+        for g in got[k]:
+            assert_same_stream(g, want[k])
+    for c in clones:
+        c.close()
+    owner.close()
+
+
+def test_reserve_sizes():
+    """a call after reserving more than it needs, and a call larger than the last reserve, both equal the model"""
+    import megapath_b200 as mp
+    from oracle import pybgzf
+    c = mp.Context(0)
+    c.bgzf_reserve(16 << 20)
+    small = contents("bam", 5 * PIECE + 17)
+    assert_same_stream(c.bgzf_compress(small), pybgzf.compress(small))
+    c.bgzf_reserve(PIECE)
+    big = contents("fastq", 30 * PIECE + 1)
+    assert_same_stream(c.bgzf_compress(big), pybgzf.compress(big))
+    assert_same_stream(c.bgzf_compress(small), pybgzf.compress(small))
+    c.close()
 
 
 # ---- the driver's -b output: device compression (default) against zlib on the formatting threads (MP_HOST_IO=1) ----
