@@ -280,6 +280,44 @@ int  mp_bgzf_compress(mp_context *ctx, const uint8_t *src, uint64_t n, uint8_t *
  * allocation inside the loop stalls every context of the GPU while it runs); larger inputs are best fed in pieces of maxBytes */
 int  mp_bgzf_reserve(mp_context *ctx, uint64_t maxBytes);
 
+/* ---- gzip inflated on the device: replaces gzread for regular .gz read files.  Single- and multi-member streams (gzip, pigz,
+ *      bgzip / BGZF, concatenated files).  Each call cuts its compressed bytes into chunks of MP_GUNZIP_CHUNK bytes, finds in every
+ *      chunk after the first the first bit offset where a dynamic-Huffman block header is valid (exactly as zlib's inflate accepts
+ *      one), decodes the chunks in parallel from there into slots of MP_GUNZIP_SLOT symbols, and keeps a chunk's output only when
+ *      it starts where the verified chunk before it ended; otherwise the chunk is decoded again from that end.  Every byte returned
+ *      was therefore decoded from a true block boundary, whatever the CRC says.  CRC-32 and ISIZE are checked per member.
+ *      src holds the file's next n bytes, starting at the previous call's *consumed (the bit offset inside the first byte is kept in
+ *      the handle); fin != 0: these bytes reach the end of the file.  At most dstCap (>= MP_GUNZIP_MIN_DST) bytes are written.
+ *      *done = 1: the end of the file was reached and every member's CRC-32 and ISIZE verified.  Bytes after the last member that
+ *      do not start with the gzip magic are ignored, as gzread ignores them.  The call makes progress whenever n >= 64 KiB or fin.
+ *      MP_ERR_FORMAT: anything zlib refuses (bad magic, method or flags, header CRC, an invalid code, a distance too far back, a
+ *      CRC-32 or ISIZE mismatch, a truncated member when fin is set); *produced then holds exactly the bytes zlib delivers before
+ *      the error, and later calls on the handle return MP_ERR_FORMAT.  Host buffers in and out; the call runs on the context's stream
+ *      and leaves a resident batch or result set as it is. */
+#define MP_GUNZIP_CHUNK 65536u          /* compressed bytes per chunk; the block search covers the chunk's bit offsets */
+#define MP_GUNZIP_SLOT (1u << 20)       /* decoded bytes a chunk holds before it stops (slot overflow) and is resumed */
+#define MP_GUNZIP_EVENTS (MP_GUNZIP_CHUNK / 16u + 8u)   /* member starts / ends a chunk records before it stops the same way */
+#define MP_GUNZIP_MIN_DST 65536u
+#define MP_GUNZIP_MAX_IN (1ull << 30)   /* largest maxIn of mp_gunzip_open: 16384 chunks, 32 GiB of slots */
+typedef struct mp_gunzip mp_gunzip;      /* one gzip file being inflated by the kernels of one context */
+typedef struct mp_gunzip_stats_t {       /* counters of the last mp_gunzip_run call */
+    uint64_t in_bytes, out_bytes;        /* compressed bytes consumed, decompressed bytes produced */
+    uint64_t chunks;                     /* chunks the input was cut into */
+    uint64_t candidates_tested;          /* bit offsets examined by the block search (up to and including the accepted one) */
+    uint64_t candidates;                 /* chunks where the search accepted a block start */
+    uint64_t false_candidates;           /* accepted starts the verified chain did not reach: those chunks were decoded again */
+    uint64_t merged;                     /* chunks without a candidate, decoded as part of the chunk before */
+    uint64_t overflows;                  /* times a verified chunk filled its slot (or event list) and was resumed */
+    uint64_t rounds;                     /* decode launches: 1 + repairs + resumes */
+    uint64_t members;                    /* gzip members whose CRC-32 and ISIZE were verified */
+    float ms_total, reserved_;           /* host wall clock of the call */
+} mp_gunzip_stats_t;
+int  mp_gunzip_open(mp_context *ctx, uint64_t maxIn, mp_gunzip **g);   /* sizes the device buffers for calls of up to maxIn bytes */
+int  mp_gunzip_run(mp_gunzip *g, const uint8_t *src, uint64_t n, int fin,
+                   uint8_t *dst, uint64_t dstCap, uint64_t *consumed, uint64_t *produced, int *done);
+int  mp_gunzip_stats(mp_gunzip *g, mp_gunzip_stats_t *s);
+void mp_gunzip_close(mp_gunzip *g);
+
 /* ---- roofline denominators measured on the spot (bench.py): kind 0 = random 32-byte gathers over an 8 GB table,
  *      1 = random 64-byte gathers (GB/s of requested bytes), 2 = packed 16-bit DPX issue rate (1e9 thread-instr/s) ---- */
 int  mp_microbench(mp_context *ctx, int kind, double *result);

@@ -78,6 +78,28 @@ class FastqFormatError(MegapathError):
 
 MP_ERR_FORMAT = -6
 
+# mp_gunzip constants (include/megapath_b200.h); the CPU model of the decoder (oracle/pygunzip.py) plans with them
+GUNZIP_CHUNK = 65536
+GUNZIP_SLOT = 1 << 20
+GUNZIP_EVENTS = GUNZIP_CHUNK // 16 + 8
+GUNZIP_MIN_DST = 65536
+
+
+class GzipFormatError(MegapathError):
+    """mp_gunzip_run refused the stream (MP_ERR_FORMAT); .partial holds the bytes zlib delivers before the error"""
+
+    def __init__(self, msg, partial=b""):
+        super().__init__(msg)
+        self.partial = partial
+
+
+class GunzipStats(C.Structure):         # mp_gunzip_stats_t
+    _fields_ = [(f, C.c_uint64) for f in ("in_bytes", "out_bytes", "chunks", "candidates_tested", "candidates", "false_candidates",
+                                          "merged", "overflows", "rounds", "members")] + [("ms_total", C.c_float), ("reserved_", C.c_float)]
+
+    def as_dict(self):
+        return {f: getattr(self, f) for f, _ in self._fields_ if f != "reserved_"}
+
 
 class Annotation(C.Structure):          # mp_annotation
     _fields_ = [("dnaLength", C.c_uint64), ("numSeq", C.c_uint32), ("gridEntries", C.c_uint32), ("numTranslate", C.c_uint32), ("reserved_", C.c_uint32),
@@ -138,6 +160,11 @@ def lib():
         L.mp_host_free.argtypes = [C.c_void_p]
         L.mp_bgzf_reserve.argtypes = [C.c_void_p, C.c_uint64]
         L.mp_bgzf_compress.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+        L.mp_gunzip_open.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p)]
+        L.mp_gunzip_run.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_void_p, C.c_uint64,
+                                    C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_int)]
+        L.mp_gunzip_stats.argtypes = [C.c_void_p, C.c_void_p]
+        L.mp_gunzip_close.argtypes = [C.c_void_p]
         _lib = L
     return _lib
 
@@ -388,6 +415,19 @@ class Context:
         self._check(self.L.mp_bgzf_compress(self.h, C.c_char_p(data), len(data), buf, cap, C.byref(n)))
         return buf.raw[:n.value]
 
+    def gunzip_stream(self, max_in):
+        """A Gunzip handle on this context for calls of up to max_in compressed bytes (mp_gunzip_open)."""
+        return Gunzip(self, max_in)
+
+    def gunzip(self, data, piece=None, out_cap=None):
+        """Device gzip inflate of a whole file (mp_gunzip_run): fed piece bytes at a time (default: all at once), writing at most
+        out_cap bytes per call (default: 64 MiB).  Raises GzipFormatError (with .partial) where zlib refuses the stream."""
+        data = memoryview(bytes(data))
+        piece = int(piece or max(len(data), GUNZIP_MIN_DST))
+        with Gunzip(self, piece) as g:
+            return g.inflate(data, out_cap)
+
+
     def seed_pairs(self, params):
         self._check(self.L.mp_seed_pairs(self.h, C.byref(params)))
 
@@ -472,3 +512,65 @@ Context.align_pairs_summary = _summary
 def cigar_at(cigars, off):
     end = cigars.index(b"\0", off)
     return cigars[off:end]
+
+
+class Gunzip:
+    """One gzip stream inflated on the device (mp_gunzip handle): run() one call at a time, or inflate() a whole buffer."""
+
+    def __init__(self, ctx, max_in):
+        self.ctx, self.L, self.max_in = ctx, ctx.L, int(max_in)
+        self.h = C.c_void_p()
+        ctx._check(self.L.mp_gunzip_open(ctx.h, self.max_in, C.byref(self.h)))
+
+    def run(self, src, fin, out_cap=GUNZIP_MIN_DST):
+        """One mp_gunzip_run call -> (output bytes, consumed, done).  src: the file's bytes from the previous call's consumed on."""
+        src = bytes(src)
+        dst = C.create_string_buffer(int(out_cap))
+        consumed, produced, done = C.c_uint64(), C.c_uint64(), C.c_int()
+        rc = self.L.mp_gunzip_run(self.h, C.c_char_p(src), len(src), int(bool(fin)), dst, int(out_cap), C.byref(consumed),
+                                  C.byref(produced), C.byref(done))
+        out = dst.raw[:produced.value]
+        if rc == MP_ERR_FORMAT:
+            raise GzipFormatError(self.L.mp_last_error().decode(), out)
+        self.ctx._check(rc)
+        return out, consumed.value, bool(done.value)
+
+    def inflate(self, data, out_cap=None):
+        data = memoryview(data)
+        out_cap = int(out_cap or 64 << 20)
+        parts, pos = [], 0
+        while True:
+            src = data[pos:pos + self.max_in]
+            try:
+                out, used, done = self.run(src, pos + len(src) == len(data), out_cap)
+            except GzipFormatError as e:
+                e.partial = b"".join(parts) + e.partial
+                raise
+            parts.append(out)
+            pos += used
+            if done:
+                return b"".join(parts)
+            if not out and not used:
+                raise MegapathError("mp_gunzip_run made no progress")
+
+    def stats(self):
+        s = GunzipStats()
+        self.ctx._check(self.L.mp_gunzip_stats(self.h, C.byref(s)))
+        return s.as_dict()
+
+    def close(self):
+        if self.h:
+            self.L.mp_gunzip_close(self.h)
+            self.h = C.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass

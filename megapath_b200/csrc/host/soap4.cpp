@@ -195,13 +195,79 @@ struct Annotation {
 
 // ------------------------------------------------------------------------------------------------
 // FASTA/FASTQ reader with kseq semantics (name up to the first blank, comment = rest of the header)
+static size_t count_newlines(const char *p, size_t n);
 struct SeqReader {
+    SeqReader() = default;
+    SeqReader(const SeqReader &) = delete;
+    SeqReader &operator=(const SeqReader &) = delete;
     gzFile f = nullptr; std::vector<char> own; char *base = nullptr; size_t pos = 0, end = 0; bool eof = false; int last = 0;
     // A plain regular file is memory-mapped instead: the whole file is the buffer (nothing left to fill), the record parsers below work
     // on it unchanged, and load_batch can locate a batch's records and parse them with several threads (parse_mapped).
     bool mapped = false;
     int fd = -1;                   // kept open beside the mapping: batches are staged with pread (no page faults on the source side)
-    bool open(const std::string &path) {
+    // A regular gzip file is inflated on the device (mp_gunzip_run on a context of its own, compressed bytes read with pread into a
+    // page-locked buffer) into `own`, which then stands in for the mapping: [pos, end) holds the inflated text not yet consumed, and
+    // ensure_lines tops it up to the next batch's records before a batch is located in it.  MP_HOST_IO=1 and pipes keep gzread.
+    mp_context *gzCtx = nullptr; mp_gunzip *gz = nullptr; int gzFd = -1; uint64_t gzOff = 0, gzSize = 0; bool gzDone = false;
+    char *gzIn = nullptr; double gzSeconds = 0;                     // page-locked compressed window; inflate wall time so far
+    static constexpr uint64_t GZ_IN = 32ull << 20, GZ_OUT = 128ull << 20;
+    ~SeqReader() {
+        if (gz) mp_gunzip_close(gz);
+        if (gzCtx) mp_destroy(gzCtx);
+        if (gzIn) mp_host_free(gzIn);
+        if (gzFd >= 0) ::close(gzFd);
+    }
+    // one mp_gunzip_run call appended at end (own grows as needed) -> bytes appended; 0 at the end of the file.  A stream the inflater
+    // refuses delivers the bytes before the error and then ends, as gzread's reader does (unexpected end of file / data error).
+    size_t gz_append() {
+        if (gzDone) return 0;
+        const double t = now_s();
+        if (own.size() - end < GZ_OUT) { own.resize(std::max(own.size() + own.size() / 2, end + GZ_OUT)); base = own.data(); }
+        const uint64_t n = std::min<uint64_t>(GZ_IN, gzSize - gzOff);
+        size_t got = 0;
+        while (got < n) { const ssize_t g = pread(gzFd, gzIn + got, n - got, (off_t)(gzOff + got)); if (g <= 0) break; got += (size_t)g; }
+        uint64_t used = 0, produced = 0; int done = 0;
+        const int rc = mp_gunzip_run(gz, (const uint8_t *)gzIn, got, gzOff + got >= gzSize, (uint8_t *)base + end, own.size() - end, &used, &produced, &done);
+        gzOff += used; end += produced;
+        if (rc || done || (produced == 0 && used == 0)) gzDone = true;
+        eof = gzDone;
+        gzSeconds += now_s() - t;
+        return produced;
+    }
+    // device-inflated file: [pos, end) holds at least `lines` newlines or the rest of the file
+    void ensure_lines(uint64_t lines) {
+        if (!gz || gzDone) return;
+        if (pos > 0) { memmove(base, base + pos, end - pos); end -= pos; pos = 0; }
+        uint64_t have = count_newlines(base, end);
+        while (have < lines && !gzDone) { const size_t e0 = end; gz_append(); have += count_newlines(base + e0, end - e0); }
+    }
+    bool open_gz_device(const std::string &path, int device) {
+        gzFd = ::open(path.c_str(), O_RDONLY);
+        struct stat sb;
+        if (gzFd < 0 || fstat(gzFd, &sb) != 0) return false;
+        gzSize = (uint64_t)sb.st_size;
+        if (mp_init(device, &gzCtx) || mp_gunzip_open(gzCtx, GZ_IN, &gz) || !(gzIn = (char *)mp_host_alloc(GZ_IN))) return false;
+        own.resize(GZ_OUT); base = own.data(); pos = end = 0;
+        if (gz_append() == 0 && gzDone && gzOff == 0) return false;     // refused on the first call
+        mapped = true;
+        return true;
+    }
+    bool open(const std::string &path, int gzDevice = -1) {
+        if (gzDevice >= 0 && !getenv("MP_HOST_IO")) {
+            int f0 = ::open(path.c_str(), O_RDONLY);
+            struct stat sb; unsigned char magic[2] = { 0, 0 };
+            const bool isGz = f0 >= 0 && fstat(f0, &sb) == 0 && S_ISREG(sb.st_mode) && pread(f0, magic, 2, 0) == 2 && magic[0] == 0x1f && magic[1] == 0x8b;
+            if (f0 >= 0) ::close(f0);
+            if (isGz) {
+                if (open_gz_device(path, gzDevice)) return true;
+                fprintf(stderr, "[Main] %s: device inflate refused (%s), reading it with zlib\n", path.c_str(), mp_last_error());
+                if (gz) { mp_gunzip_close(gz); gz = nullptr; }
+                if (gzCtx) { mp_destroy(gzCtx); gzCtx = nullptr; }
+                if (gzIn) { mp_host_free(gzIn); gzIn = nullptr; }
+                if (gzFd >= 0) { ::close(gzFd); gzFd = -1; }
+                gzDone = false; pos = end = 0; eof = false;
+            }
+        }
         if (!getenv("MP_NO_MMAP")) {
             int fd = ::open(path.c_str(), O_RDONLY);
             if (fd >= 0) {
@@ -220,7 +286,11 @@ struct SeqReader {
         }
         f = gzopen(path.c_str(), "rb"); if (!f) return false; gzbuffer(f, 1 << 22); own.resize(1 << 22); base = own.data(); return true;
     }
-    bool fill() { if (eof) return false; int n = gzread(f, base, (unsigned)own.size()); if (n <= 0) { eof = true; return false; } pos = 0; end = (size_t)n; return true; }
+    bool fill() {
+        if (eof) return false;
+        if (gz) { pos = end = 0; gz_append(); return end > 0; }
+        int n = gzread(f, base, (unsigned)own.size()); if (n <= 0) { eof = true; return false; } pos = 0; end = (size_t)n; return true;
+    }
     int getc_() { if (pos >= end && !fill()) return -1; return (unsigned char)base[pos++]; }
     // reads up to the delimiter class: 0 = blank (space/tab/newline), 2 = newline; returns delimiter or -1.  Whole buffer ranges
     // are appended at once (the per-character version of this loop was the slowest part of the driver).
@@ -274,6 +344,7 @@ struct SeqReader {
             const size_t rest = (size_t)(e - b);
             if (rest == own.size()) return 0;                  // a record larger than the buffer: leave it to read()
             memmove(base, b, rest); pos = 0; end = rest;
+            if (gz) { if (gz_append() == 0) return 0; continue; }
             int n = gzread(f, base + end, (unsigned)(own.size() - end));
             if (n <= 0) { eof = true; return 0; }
             end += (size_t)n;
@@ -1215,7 +1286,7 @@ int main(int argc, char **argv)
 
     fill_char_map();
     SeqReader r1, r2;
-    if (!r1.open(opt.query1) || !r2.open(opt.query2)) { fprintf(stderr, "Cannot open the read files\n"); return 1; }
+    if (!r1.open(opt.query1, opt.device) || !r2.open(opt.query2, opt.device)) { fprintf(stderr, "Cannot open the read files\n"); return 1; }
     uint32_t maxNumQueries = 12 * 8192 * 128 / 6;                  // SOAP4.cpp:206
     if (const char *e = getenv("MP_BATCH_READS")) {                // smaller batches (multi-batch / multi-context tests on small inputs)
         const long v = atol(e); if (v >= 64 && v <= 12 * 8192 * 128 / 6) maxNumQueries = (uint32_t)v & ~63u;
@@ -1254,6 +1325,13 @@ int main(int argc, char **argv)
     // begin with; batches with long SCORE: lists raise it for the buffers taken after them)
     std::atomic<size_t> growPerRead(64);
     auto batch_need = [&]() -> size_t { return window_cap(0, r1) + window_cap(1, r2) + (size_t)maxNumQueries * growPerRead.load() + ((size_t)1 << 20); };
+    // device-inflated .gz inputs: [pos, end) must hold a whole batch before a batch is located in it
+    auto ensure_batch = [&]() {
+        std::thread e2([&] { r2.ensure_lines(4ull * (maxNumQueries / 2) + 4); });
+        r1.ensure_lines(4ull * ((maxNumQueries + 1) / 2) + 4);
+        e2.join();
+    };
+    ensure_batch();
     std::thread pinThread;
     if (deviceIO) {
         SeqReader::View v; const char *nx = nullptr;
@@ -1313,7 +1391,9 @@ int main(int argc, char **argv)
     // -> 1: the next batch staged in page-locked memory (file positions advanced), 0: end of both files, -1: not for the device path
     auto stage_raw = [&](RawBatch &rb) -> int {
         static const bool ltiming = getenv("MP_DRIVER_TIMING") != nullptr;
-        const double ts0 = now_s();
+        const double ts0 = now_s(), gz0 = r1.gzSeconds + r2.gzSeconds;
+        ensure_batch();
+        const double tInflate = r1.gzSeconds + r2.gzSeconds - gz0;
         const size_t cap1 = window_cap(0, r1), cap2 = window_cap(1, r2);
         auto pc = pin_take(cap1 + cap2 + (size_t)maxNumQueries * growPerRead.load() + ((size_t)1 << 20));
         if (!pc.first) { fprintf(stderr, "%s\n", mp_last_error()); exit(1); }
@@ -1352,7 +1432,8 @@ int main(int argc, char **argv)
         rb.nReads = 2 * (uint32_t)n1;
         bytesPerRec[0] = (double)rb.bytes1 / (double)n1; bytesPerRec[1] = (double)rb.bytes2 / (double)n2;
         r1.pos = p1; r2.pos = p2;
-        if (ltiming) fprintf(stderr, "[timing] stage: buffer %.3f copy + count %.3f rest %.3f s (%.0f MB)\n", ts1 - ts0, ts2 - ts1, now_s() - ts2, (rb.bytes1 + rb.bytes2) / 1e6);
+        if (ltiming) fprintf(stderr, "[timing] stage: inflate %.3f buffer %.3f copy + count %.3f rest %.3f s (%.0f MB)\n", tInflate, ts1 - ts0 - tInflate, ts2 - ts1,
+                             now_s() - ts2, (rb.bytes1 + rb.bytes2) / 1e6);
         return 1;
     };
     RawBatch firstRaw; bool haveFirstRaw = false;
@@ -1468,6 +1549,9 @@ int main(int argc, char **argv)
             { std::lock_guard<std::mutex> lk(mu); if (!batchPool.empty()) { j->b = batchPool.back(); batchPool.pop_back(); } }
             if (!j->b) j->b = new ReadBatch;
             j->b->maxReadLength = (uint32_t)maxLen; j->b->wpq = ((uint32_t)maxLen + 15) / 16;
+            const double gz0 = r1.gzSeconds + r2.gzSeconds;
+            ensure_batch();
+            if (getenv("MP_DRIVER_TIMING") && (r1.gz || r2.gz)) fprintf(stderr, "[timing] load: inflate %.3f s\n", r1.gzSeconds + r2.gzSeconds - gz0);
             if (load_batch(r1, r2, *j->b, maxNumQueries, ioThreads) == 0) { delete j->b; delete j; break; }
             j->nReads = j->b->nReads;
             }

@@ -22,6 +22,7 @@
 // Every tie (hash heads, equal-length matches, equal frequencies in the Huffman construction) is broken by position or symbol
 // number, so the output depends on the input bytes only.
 #include "mp_context.h"
+#include "mp_crc32.h"
 #include <cub/cub.cuh>
 
 namespace {
@@ -61,28 +62,6 @@ struct BgSmem {
     typename BgScan::TempStorage scan;
     uint32_t nRle, hlit, hdist, hclen, mode, headerBits, crc, totalBits;
 };
-
-__device__ __forceinline__ uint32_t bg_multmodp(uint32_t a, uint32_t b)      // a * b mod P, reflected (zlib crc32.c)
-{
-    uint32_t m = 1u << 31, p = 0;
-    for (;;) {
-        if (a & m) { p ^= b; if ((a & (m - 1)) == 0) break; }
-        m >>= 1;
-        b = b & 1 ? (b >> 1) ^ 0xEDB88320u : b >> 1;
-    }
-    return p;
-}
-__device__ uint32_t bg_x8n(uint32_t n)                                         // x^(8n) mod P
-{
-    uint32_t p = 1u << 31, sq = 1u << 30;                                      // sq = x^(2^k) while k walks up from 0
-    for (int k = 0; k < 3; ++k) sq = bg_multmodp(sq, sq);                       // x^8
-    while (n) {
-        if (n & 1) p = bg_multmodp(sq, p);
-        n >>= 1;
-        if (n) sq = bg_multmodp(sq, sq);
-    }
-    return p;
-}
 
 __device__ __forceinline__ void bg_or_byte(uint32_t *slot, uint32_t at, uint32_t v) { atomicOr(slot + (at >> 2), (v & 0xffu) << ((at & 3) * 8)); }
 
@@ -303,11 +282,11 @@ k_bgzf_member(const uint8_t *__restrict__ src, uint64_t n, uint32_t nPieces, uin
             for (uint32_t p = 0; p < len;) { const uint32_t v = lens[p]; lens[p] = (uint16_t)(v | 0x8000); p += v ? v : 1; }
         } else if (t == 32) {
             uint32_t c = S.sliceCrc[0];
-            const uint32_t shiftPer = bg_x8n(per);
+            const uint32_t shiftPer = mp_crc32_x8n(per);
             for (uint32_t k = 1; k < BG_THREADS; ++k) {
                 const uint32_t a = min(len, k * per), b = min(len, a + per);
                 if (b == a) break;
-                c = bg_multmodp(b - a == per ? shiftPer : bg_x8n(b - a), c) ^ S.sliceCrc[k];
+                c = mp_crc32_mulmod(b - a == per ? shiftPer : mp_crc32_x8n(b - a), c) ^ S.sliceCrc[k];
             }
             S.crc = c;
         }
