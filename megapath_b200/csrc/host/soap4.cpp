@@ -446,13 +446,67 @@ static size_t count_newlines(const char *p, size_t n)
     return c;
 }
 
-// A batch out of a memory-mapped FASTQ file, parsed by several threads.  Records are located, not guessed: the newlines of the
-// region are counted in 256 KiB blocks (in parallel), which gives the byte offset of every 4k-th line, and every thread then parses
-// its run of four-line records with the same record view as the sequential reader.  If anything is not a plain four-line record (a
-// multi-line FASTA / FASTQ, a quality string of another length, a missing final newline) nothing is consumed and the caller parses the
-// batch sequentially -- same records either way (tests/test_driver_host.py).
-// -> records parsed, *newPos = offset behind them; -1: use the sequential parser
-static long parse_mapped(const SeqReader &r, ReadBatch &b, uint32_t first, uint32_t maxRec, unsigned nThr, size_t *newPos)
+// fn(k) for k in [0, n), strided over min(nThr, n) threads (at least one); slice 0 runs on the calling thread
+static void parallel_for(size_t n, unsigned nThr, const std::function<void(size_t)> &fn)
+{
+    const unsigned T = (unsigned)std::min<size_t>(std::max(1u, nThr), std::max<size_t>(n, 1));
+    std::vector<std::thread> th;
+    for (unsigned t = 1; t < T; ++t) th.emplace_back([&, t] { for (size_t k = t; k < n; k += T) fn(k); });
+    for (size_t k = 0; k < n; k += T) fn(k);
+    for (std::thread &x : th) x.join();
+}
+
+// The newlines of [base, base + bytes), counted in 256 KiB blocks by several threads: after(L) finds the byte behind any line without
+// a second pass over the text.  This is how the driver finds where a batch of four-line records ends and where each parser thread's
+// run of records starts.
+struct LineBlocks {
+    static constexpr size_t B = (size_t)1 << 18;
+    const char *base = nullptr; size_t bytes = 0;
+    std::vector<uint32_t> cnt; std::vector<uint64_t> pre;          // newlines per block; pre[k] = newlines before block k
+    // (re)counts blocks [from, ...) of the first n bytes with count(offset, len) -> newlines of that block
+    void count(size_t n, size_t from, unsigned nThr, const std::function<uint32_t(size_t, size_t)> &fn) {
+        bytes = n; cnt.resize((n + B - 1) / B);
+        parallel_for(cnt.size() - from, nThr, [&](size_t k) { const size_t o = (from + k) * B; cnt[from + k] = fn(o, std::min(B, n - o)); });
+        pre.assign(cnt.size() + 1, 0);
+        for (size_t k = 0; k < cnt.size(); ++k) pre[k + 1] = pre[k] + cnt[k];
+    }
+    uint64_t lines() const { return pre.back(); }
+    // first byte after the L-th newline (L <= lines()); base for L = 0
+    const char *after(uint64_t L) const {
+        if (L == 0) return base;
+        const size_t k = (size_t)(std::lower_bound(pre.begin(), pre.end(), L) - pre.begin()) - 1;     // pre[k] < L <= pre[k+1]
+        const char *q = base + k * B;
+        for (uint64_t need = L - pre[k]; need; --need) q = (const char *)memchr(q, '\n', (size_t)(base + bytes - q)) + 1;
+        return q;
+    }
+};
+
+// Counts the next maxRec four-line records of `remaining` bytes into lb: the window starts at maxRec records of bytesPerRec (+2 %, + a
+// block) and grows by an eighth until it holds 4·maxRec lines or all the bytes; each round counts only the blocks not counted yet (the
+// partial last block again).  count(offset, len) counts one block and may do more with it first (stage_file copies it).
+// -> records (at most maxRec) then end at lb.after(4·records); -1: the text ends inside the window, not after a whole record (or holds
+// none); -2: the window would exceed cap bytes
+static long count_records(LineBlocks &lb, size_t remaining, double bytesPerRec, size_t cap, uint32_t maxRec, unsigned nThr,
+                          const std::function<uint32_t(size_t, size_t)> &count)
+{
+    const size_t B = LineBlocks::B;
+    size_t window = std::min(remaining, (size_t)((double)maxRec * bytesPerRec * 1.02) + B), counted = 0;
+    for (;;) {
+        if (window > cap) return -2;
+        lb.count(window, counted, nThr, count);
+        if (lb.lines() >= 4ull * maxRec || window == remaining) break;
+        counted = window / B;
+        window = std::min(remaining, window + window / 8 + B);
+    }
+    if (lb.lines() < 4ull * maxRec && (lb.lines() & 3)) return -1;
+    const uint64_t nRec = std::min<uint64_t>(maxRec, lb.lines() / 4);
+    return nRec == 0 ? -1 : (long)nRec;
+}
+
+// The byte range of the next maxRec four-line records of a memory-mapped file, located by count_records.  Whether the range really is
+// strict four-line FASTQ is checked by whoever reads it: the kernels that index it (device ingest) or parse_mapped.
+// -> records in [r.pos, *newPos), 0 at the end of the file, -1: this file needs the sequential parser; lb: the range's newline index
+static long locate_records(const SeqReader &r, uint32_t maxRec, unsigned nThr, size_t *newPos, LineBlocks &lb)
 {
     const char *beg = r.base + r.pos, *lim = r.base + r.end;
     *newPos = r.pos;
@@ -461,45 +515,31 @@ static long parse_mapped(const SeqReader &r, ReadBatch &b, uint32_t first, uint3
     if (lim[-1] != '\n') return -1;
     SeqReader::View v0; const char *next0 = nullptr;
     if (SeqReader::view_record(beg, lim, v0, &next0) != 1) return -1;
-    const size_t B = (size_t)1 << 18, remaining = (size_t)(lim - beg), rec0 = (size_t)(next0 - beg);
-    nThr = std::max(1u, nThr);
-    auto par = [&](size_t n, const std::function<void(size_t)> &fn) {       // fn(k) for k in [0, n), strided over the threads
-        const unsigned T = (unsigned)std::min<size_t>(nThr, std::max<size_t>(n, 1));
-        std::vector<std::thread> th;
-        for (unsigned t = 1; t < T; ++t) th.emplace_back([&, t] { for (size_t k = t; k < n; k += T) fn(k); });
-        for (size_t k = 0; k < n; k += T) fn(k);
-        for (std::thread &x : th) x.join();
-    };
-    // ---- newline counts per block, over a window that grows until it holds the batch (or the rest of the file) ----
-    size_t window = std::min(remaining, (size_t)((double)maxRec * (double)rec0 * 1.02) + B), fullCounted = 0;
-    std::vector<uint32_t> cnt;
-    uint64_t lines = 0;
-    for (;;) {
-        const size_t nBlocks = (window + B - 1) / B;
-        cnt.resize(nBlocks);
-        par(nBlocks - fullCounted, [&](size_t k) { const size_t blk = fullCounted + k; cnt[blk] = (uint32_t)count_newlines(beg + blk * B, std::min(B, window - blk * B)); });
-        lines = 0; for (uint32_t c : cnt) lines += c;
-        if (lines >= 4ull * maxRec || window == remaining) break;
-        fullCounted = window / B;                                            // the partial last block is counted again
-        window = std::min(remaining, window + window / 8 + B);
-    }
-    if (lines < 4ull * maxRec && (lines & 3)) return -1;                      // the file ends inside the window, not after a whole record
-    const uint64_t nRec = std::min<uint64_t>(maxRec, lines / 4);
-    if (nRec == 0) return -1;
-    std::vector<uint64_t> pre(cnt.size() + 1, 0);
-    for (size_t k = 0; k < cnt.size(); ++k) pre[k + 1] = pre[k] + cnt[k];
-    auto after_line = [&](uint64_t L) -> const char * {                      // first byte after the L-th newline of the region (L >= 1)
-        const size_t k = (size_t)(std::lower_bound(pre.begin(), pre.end(), L) - pre.begin()) - 1;     // pre[k] < L <= pre[k+1]
-        const char *q = beg + k * B;
-        for (uint64_t need = L - pre[k]; need; --need) q = (const char *)memchr(q, '\n', (size_t)(lim - q)) + 1;
-        return q;
-    };
-    const unsigned T = (unsigned)std::min<uint64_t>(nThr, std::max<uint64_t>(1, nRec / 256));
+    lb.base = beg;
+    const long nRec = count_records(lb, (size_t)(lim - beg), (double)(next0 - beg), SIZE_MAX, maxRec, nThr,
+                                    [&](size_t o, size_t len) { return (uint32_t)count_newlines(beg + o, len); });
+    if (nRec > 0) *newPos = (size_t)(lb.after(4 * (uint64_t)nRec) - r.base);
+    return nRec;
+}
+
+// A batch out of a memory-mapped FASTQ file, parsed by several threads.  Records are located, not guessed (locate_records), and every
+// thread then parses its run of four-line records with the same record view as the sequential reader.  If anything is not a plain
+// four-line record (a multi-line FASTA / FASTQ, a quality string of another length, a missing final newline) nothing is consumed and the
+// caller parses the batch sequentially -- same records either way (tests/test_driver_host.py).
+// -> records parsed, *newPos = offset behind them; -1: use the sequential parser
+static long parse_mapped(const SeqReader &r, ReadBatch &b, uint32_t first, uint32_t maxRec, unsigned nThr, size_t *newPos)
+{
+    *newPos = r.pos;
+    LineBlocks lb; size_t end = 0;
+    const long n = locate_records(r, maxRec, nThr, &end, lb);
+    if (n <= 0) return n;
+    const uint64_t nRec = (uint64_t)n;
+    const unsigned T = (unsigned)std::min<uint64_t>(std::max(1u, nThr), std::max<uint64_t>(1, nRec / 256));
     std::vector<const char *> start(T + 1);
     std::vector<uint64_t> firstRec(T + 1);
-    for (unsigned t = 0; t <= T; ++t) { firstRec[t] = nRec * t / T; start[t] = firstRec[t] == 0 ? beg : after_line(4 * firstRec[t]); }
+    for (unsigned t = 0; t <= T; ++t) { firstRec[t] = nRec * t / T; start[t] = lb.after(4 * firstRec[t]); }
     std::atomic<bool> bad(false);
-    par(T, [&](size_t t) {
+    parallel_for(T, T, [&](size_t t) {
         const char *q = start[t], *e = start[t + 1];
         SeqReader::View v;
         for (uint64_t rec = firstRec[t]; rec < firstRec[t + 1]; ++rec) {
@@ -511,62 +551,8 @@ static long parse_mapped(const SeqReader &r, ReadBatch &b, uint32_t first, uint3
         if (q != e) bad.store(true);
     });
     if (bad.load()) return -1;
-    *newPos = (size_t)(start[T] - r.base);
-    return (long)nRec;
-}
-
-// Device ingest (mp_fastq_upload): the byte range of the next maxRec four-line records of a memory-mapped file, found by counting
-// newlines in 256 KiB blocks with several threads (the same location step as parse_mapped).  Whether the range really is strict
-// four-line FASTQ is checked by the kernels that index it.
-// -> records in [r.pos, *newPos), 0 at the end of the file, -1: this file needs the sequential parser
-static long locate_records(const SeqReader &r, uint32_t maxRec, unsigned nThr, size_t *newPos)
-{
-    const char *beg = r.base + r.pos, *lim = r.base + r.end;
-    *newPos = r.pos;
-    if (r.last != 0) return -1;
-    if (beg >= lim || maxRec == 0) return 0;
-    if (lim[-1] != '\n') return -1;
-    SeqReader::View v0; const char *next0 = nullptr;
-    if (SeqReader::view_record(beg, lim, v0, &next0) != 1) return -1;
-    const size_t B = (size_t)1 << 18, remaining = (size_t)(lim - beg), rec0 = (size_t)(next0 - beg);
-    nThr = std::max(1u, nThr);
-    size_t window = std::min(remaining, (size_t)((double)maxRec * (double)rec0 * 1.02) + B), fullCounted = 0;
-    std::vector<uint32_t> cnt;
-    uint64_t lines = 0;
-    for (;;) {
-        const size_t nBlocks = (window + B - 1) / B;
-        cnt.resize(nBlocks);
-        const size_t n = nBlocks - fullCounted;
-        const unsigned T = (unsigned)std::min<size_t>(nThr, std::max<size_t>(n, 1));
-        auto run = [&](unsigned t) { for (size_t k = t; k < n; k += T) { const size_t blk = fullCounted + k; cnt[blk] = (uint32_t)count_newlines(beg + blk * B, std::min(B, window - blk * B)); } };
-        std::vector<std::thread> th;
-        for (unsigned t = 1; t < T; ++t) th.emplace_back(run, t);
-        run(0);
-        for (std::thread &x : th) x.join();
-        lines = 0; for (uint32_t c : cnt) lines += c;
-        if (lines >= 4ull * maxRec || window == remaining) break;
-        fullCounted = window / B;
-        window = std::min(remaining, window + window / 8 + B);
-    }
-    if (lines < 4ull * maxRec && (lines & 3)) return -1;
-    const uint64_t nRec = std::min<uint64_t>(maxRec, lines / 4);
-    if (nRec == 0) return -1;
-    uint64_t need = 4 * nRec, pre = 0; size_t k = 0;
-    while (pre + cnt[k] < need) pre += cnt[k++];
-    const char *q = beg + k * B;
-    for (need -= pre; need; --need) q = (const char *)memchr(q, '\n', (size_t)(lim - q)) + 1;
-    *newPos = (size_t)(q - r.base);
-    return (long)nRec;
-}
-static void parallel_copy(char *dst, const char *src, size_t n, unsigned nThr)
-{
-    const size_t piece = (size_t)4 << 20, nPieces = (n + piece - 1) / piece;
-    const unsigned T = (unsigned)std::min<size_t>(std::max(1u, nThr), std::max<size_t>(nPieces, 1));
-    auto run = [&](unsigned t) { for (size_t k = t; k < nPieces; k += T) memcpy(dst + k * piece, src + k * piece, std::min(piece, n - k * piece)); };
-    std::vector<std::thread> th;
-    for (unsigned t = 1; t < T; ++t) th.emplace_back(run, t);
-    run(0);
-    for (std::thread &x : th) x.join();
+    *newPos = end;
+    return n;
 }
 
 // One mate file's next batch: every 256 KiB block is copied into the staging buffer and its newlines are counted in the copy while
@@ -579,42 +565,15 @@ static long stage_file(const SeqReader &r, double bytesPerRec, uint32_t maxRec, 
     if (r.last != 0) return -1;
     if (beg >= lim || maxRec == 0) return 0;
     if (lim[-1] != '\n' || *beg != '@') return -1;
-    const size_t B = (size_t)1 << 18, remaining = (size_t)(lim - beg);
-    size_t window = std::min(remaining, (size_t)((double)maxRec * bytesPerRec * 1.02) + B), done = 0;
-    std::vector<uint32_t> cnt;
-    uint64_t lines = 0;
-    for (;;) {
-        if (window > cap) return -2;
-        const size_t nBlocks = (window + B - 1) / B, n = nBlocks - done;
-        cnt.resize(nBlocks);
-        const unsigned T = (unsigned)std::min<size_t>(stageThreads, std::max<size_t>(n, 1));
-        auto run = [&](unsigned t) {
-            for (size_t k = t; k < n; k += T) {
-                const size_t blk = done + k, o = blk * B, len = std::min(B, window - o);
-                size_t got = 0;                                           // pread: the kernel copies from the page cache, no faults on a mapping
-                while (r.fd >= 0 && got < len) { const ssize_t g = pread(r.fd, dst + o + got, len - got, (off_t)(r.pos + o + got)); if (g <= 0) break; got += (size_t)g; }
-                if (got < len) memcpy(dst + o + got, beg + o + got, len - got);
-                cnt[blk] = (uint32_t)count_newlines(dst + o, len);
-            }
-        };
-        std::vector<std::thread> th;
-        for (unsigned t = 1; t < T; ++t) th.emplace_back(run, t);
-        run(0);
-        for (std::thread &x : th) x.join();
-        lines = 0; for (uint32_t c : cnt) lines += c;
-        if (lines >= 4ull * maxRec || window == remaining) break;
-        done = window / B;                                               // the partial last block is copied and counted again
-        window = std::min(remaining, window + window / 8 + B);
-    }
-    if (lines < 4ull * maxRec && (lines & 3)) return -1;
-    const uint64_t nRec = std::min<uint64_t>(maxRec, lines / 4);
-    if (nRec == 0) return -1;
-    uint64_t need = 4 * nRec, pre = 0; size_t k = 0;
-    while (pre + cnt[k] < need) pre += cnt[k++];
-    const char *q = dst + k * B;
-    for (need -= pre; need; --need) q = (const char *)memchr(q, '\n', (size_t)(dst + window - q)) + 1;
-    *bytes = (size_t)(q - dst);
-    return (long)nRec;
+    LineBlocks lb; lb.base = dst;
+    const long nRec = count_records(lb, (size_t)(lim - beg), bytesPerRec, cap, maxRec, stageThreads, [&](size_t o, size_t len) {
+        size_t got = 0;                                                  // pread: the kernel copies from the page cache, no faults on a mapping
+        while (r.fd >= 0 && got < len) { const ssize_t g = pread(r.fd, dst + o + got, len - got, (off_t)(r.pos + o + got)); if (g <= 0) break; got += (size_t)g; }
+        if (got < len) memcpy(dst + o + got, beg + o + got, len - got);
+        return (uint32_t)count_newlines(dst + o, len);
+    });
+    if (nRec > 0) *bytes = (size_t)(lb.after(4 * (uint64_t)nRec) - dst);
+    return nRec;
 }
 
 static uint32_t load_batch(SeqReader &r1, SeqReader &r2, ReadBatch &b, uint32_t maxReads, unsigned packThreads = 4)
@@ -647,10 +606,7 @@ static uint32_t load_batch(SeqReader &r1, SeqReader &r2, ReadBatch &b, uint32_t 
             b.nReads = 2 * (uint32_t)n1;
             const double tl1 = now_s();
             const uint32_t nGroups = (b.nReads + 31) / 32, T = std::min<uint32_t>(2 * team, std::max(1u, nGroups / 64));
-            std::vector<std::thread> th;
-            for (uint32_t t = 1; t < T; ++t) th.emplace_back([&, t] { pack_reads(b, (uint32_t)((uint64_t)nGroups * t / T) * 32, std::min(b.nReads, (uint32_t)((uint64_t)nGroups * (t + 1) / T) * 32)); });
-            pack_reads(b, 0, std::min(b.nReads, (uint32_t)((uint64_t)nGroups / T) * 32));
-            for (std::thread &x : th) x.join();
+            parallel_for(T, T, [&](size_t t) { pack_reads(b, (uint32_t)((uint64_t)nGroups * t / T) * 32, std::min(b.nReads, (uint32_t)((uint64_t)nGroups * (t + 1) / T) * 32)); });
             if (ltiming) fprintf(stderr, "[load] setup %.3f parse %.3f pack %.3f s\n", tl0 - tSetup0, tl1 - tl0, now_s() - tl1);
             return b.nReads;
         }
@@ -706,7 +662,7 @@ static uint32_t load_batch(SeqReader &r1, SeqReader &r2, ReadBatch &b, uint32_t 
     return b.nReads;
 }
 
-static uint32_t detect_read_length(const std::vector<uint32_t> &lens, uint32_t numQueries, uint32_t start)   // GetReadLength (QueryParser.cpp:2253-2277)
+static uint32_t detect_read_length(const uint32_t *lens, uint32_t numQueries, uint32_t start)   // GetReadLength (QueryParser.cpp:2253-2277)
 {
     if (numQueries == 0) return 100;
     uint32_t i = 0, j = 1, mx = lens[start];
@@ -1153,6 +1109,19 @@ static void fastq_chunk_to_lsam(const char *fqData, size_t fqSize, bool outputSe
     }
     if (hasLast) print(last, 0);
 }
+// A batch's text of whole pairs, cut at pair boundaries (every eighth line) into up to nThr pieces of at least 4096 pairs, each
+// rewritten into fastq2lsam's lines by a thread of its own: parts[c] holds piece c's lines.
+static void lsam_pieces(const char *text, size_t bytes, unsigned nThr, bool outputSeq, std::vector<std::string> &parts)
+{
+    LineBlocks lb; lb.base = text;
+    lb.count(bytes, 0, nThr, [&](size_t o, size_t len) { return (uint32_t)count_newlines(text + o, len); });
+    const uint64_t nPairs = lb.lines() / 8;
+    const unsigned nc = (unsigned)std::min<uint64_t>(std::max(1u, nThr), std::max<uint64_t>(1, nPairs / 4096));
+    std::vector<const char *> cut(nc + 1, text + bytes);
+    for (unsigned c = 0; c < nc; ++c) cut[c] = lb.after(8 * (nPairs * c / nc));
+    parts.assign(nc, std::string());
+    parallel_for(nc, nc, [&](size_t c) { if (cut[c + 1] > cut[c]) fastq_chunk_to_lsam(cut[c], (size_t)(cut[c + 1] - cut[c]), outputSeq, parts[c]); });
+}
 
 int main(int argc, char **argv)
 {
@@ -1205,15 +1174,15 @@ int main(int argc, char **argv)
         w.close();
         return 0;
     }
-    if (argc >= 4 && !strcmp(argv[1], "__lsam")) {           // hidden: annotated FASTQ file -> the -lsam lines (no GPU): __lsam file outputSeq
+    if (argc >= 4 && !strcmp(argv[1], "__lsam")) {           // hidden: annotated FASTQ file -> the -lsam lines (no GPU): __lsam file outputSeq [threads]
         FILE *in = fopen(argv[2], "rb"); if (!in) return 1;
         std::string data; char tmp[65536]; size_t n;
         while ((n = fread(tmp, 1, sizeof tmp, in)) > 0) data.append(tmp, n);
         fclose(in);
         const double tc = now_s();
-        std::string out; fastq_chunk_to_lsam(data.data(), data.size(), atoi(argv[3]) != 0, out);
+        std::vector<std::string> parts; lsam_pieces(data.data(), data.size(), argc >= 5 ? (unsigned)atoi(argv[4]) : 1u, atoi(argv[3]) != 0, parts);
         fprintf(stderr, "converted %.1f MB in %.3f s\n", data.size() / 1e6, now_s() - tc);
-        fwrite(out.data(), 1, out.size(), stdout);
+        for (const std::string &p : parts) fwrite(p.data(), 1, p.size(), stdout);
         return 0;
     }
     if (argc >= 5 && !strcmp(argv[1], "__stage")) {          // hidden: batch boundaries of the device-ingest staging (no GPU): __stage file maxRec threads [bytesPerRec]
@@ -1223,7 +1192,7 @@ int main(int argc, char **argv)
         double bpr = argc >= 6 ? atof(argv[5]) : 0;
         for (;;) {
             // exact location, then the fused copy + count with the running estimate: both must name the same byte range
-            size_t np = 0; const long n = locate_records(r, maxRec, thr, &np);
+            size_t np = 0; LineBlocks lb; const long n = locate_records(r, maxRec, thr, &np, lb);
             if (bpr <= 0) { SeqReader::View v; const char *nx = nullptr; if (r.pos < r.end && SeqReader::view_record(r.base + r.pos, r.base + r.end, v, &nx) == 1) bpr = (double)(nx - (r.base + r.pos)); else bpr = 64; }
             const size_t cap = std::min<size_t>((size_t)((double)maxRec * bpr * 1.03) + ((size_t)2 << 18), r.end - r.pos + 64);
             std::vector<char> dst(cap + 64);
@@ -1253,11 +1222,12 @@ int main(int argc, char **argv)
     Options opt;
     if (!parse_args(argc, argv, opt)) return 1;
     const double t0 = now_s();
-    {   // large inputs: every kernel is loaded with the library, not at its first launch inside the batch loop (must be set before the
-        // first CUDA call); small runs keep lazy loading, which starts the process faster
-        struct stat sb0;
-        if (stat(opt.query1.c_str(), &sb0) == 0 && sb0.st_size > (off_t)(48 << 20)) setenv("CUDA_MODULE_LOADING", "EAGER", 0);
-    }
+    // large inputs: every kernel is loaded with the library, not at its first launch inside the batch loop (must be set before the
+    // first CUDA call), and every context's batch buffers are sized before the loop; small runs keep lazy loading, which starts the
+    // process faster, and lazy sizing
+    struct stat sb0;
+    const bool largeInput = stat(opt.query1.c_str(), &sb0) == 0 && sb0.st_size > (off_t)(48 << 20);
+    if (largeInput) setenv("CUDA_MODULE_LOADING", "EAGER", 0);
     Ini ini;
     std::string iniPath = opt.iniFile.empty() ? std::string(argv[0]) + ".ini" : opt.iniFile;
     if (!ini.load(iniPath)) { fprintf(stderr, "Failed to open config file ... %s\n", iniPath.c_str()); return 1; }
@@ -1283,6 +1253,12 @@ int main(int argc, char **argv)
     P.skipDefaultDP = ini.geti("OtherSettings:SkipDefaultDP", 0);
     P.maxReadLength = maxLen; P.insert_high = opt.insert_high;
     const double top = opt.top / 100.0;
+    auto first_batch = [&](const uint32_t *lens, uint32_t nReads) {   // first-batch read-length detection and insert_low clamp (SOAP4.cpp:458-474)
+        const uint32_t d1 = detect_read_length(lens, nReads, 0), d2 = detect_read_length(lens, nReads, 1);
+        if (opt.insert_low < (int)d2) opt.insert_low = (int)d2;
+        if (opt.insert_low < (int)d1) opt.insert_low = (int)d1;
+        P.insert_low = opt.insert_low;
+    };
 
     fill_char_map();
     SeqReader r1, r2;
@@ -1324,7 +1300,7 @@ int main(int argc, char **argv)
     // the formatted text of a batch comes back into the buffer its input came from: room for what the headers grow by (64 bytes per read to
     // begin with; batches with long SCORE: lists raise it for the buffers taken after them)
     std::atomic<size_t> growPerRead(64);
-    auto batch_need = [&]() -> size_t { return window_cap(0, r1) + window_cap(1, r2) + (size_t)maxNumQueries * growPerRead.load() + ((size_t)1 << 20); };
+    auto out_room = [&]() -> size_t { return (size_t)maxNumQueries * growPerRead.load() + ((size_t)1 << 20); };
     // device-inflated .gz inputs: [pos, end) must hold a whole batch before a batch is located in it
     auto ensure_batch = [&]() {
         std::thread e2([&] { r2.ensure_lines(4ull * (maxNumQueries / 2) + 4); });
@@ -1338,7 +1314,7 @@ int main(int argc, char **argv)
         if (r1.end > r1.pos && r2.end > r2.pos && SeqReader::view_record(r1.base + r1.pos, r1.base + r1.end, v, &nx) == 1) bytesPerRec[0] = (double)(nx - (r1.base + r1.pos));
         if (bytesPerRec[0] > 0 && SeqReader::view_record(r2.base + r2.pos, r2.base + r2.end, v, &nx) == 1) bytesPerRec[1] = (double)(nx - (r2.base + r2.pos));
         if (bytesPerRec[0] > 0 && bytesPerRec[1] > 0) {
-            const size_t need = batch_need(), cap = need + need / 16;
+            const size_t need = window_cap(0, r1) + window_cap(1, r2) + out_room(), cap = need + need / 16;
             const size_t batches = (size_t)((double)(r1.end - r1.pos) / (bytesPerRec[0] * (double)(maxNumQueries / 2))) + 1;
             const size_t count = std::min<size_t>((size_t)opt.numGpus * (size_t)opt.contextsPerGpu + 3, batches);
             pinThread = std::thread([&, cap, count] { for (size_t k = 0; k < count; ++k) { char *p = (char *)mp_host_alloc(cap); if (p) pin_give(p, cap); } });
@@ -1366,15 +1342,8 @@ int main(int argc, char **argv)
             }
         }
     }
-    {   // large inputs: size every context's batch buffers before the batch loop (part of the set-up time, like the index load) so that
-        // no batch pays for allocations; small inputs keep the lazy sizing
-        struct stat sb;
-        if (stat(opt.query1.c_str(), &sb) == 0 && sb.st_size > (off_t)(48 << 20)) {
-            uint32_t batchReads = 12 * 8192 * 128 / 6;
-            if (const char *e = getenv("MP_BATCH_READS")) { const long v = atol(e); if (v >= 64 && v <= (long)batchReads) batchReads = (uint32_t)v & ~63u; }
-            for (mp_context *c : contexts) if (mp_reserve(c, &P, batchReads)) { fprintf(stderr, "%s\n", mp_last_error()); return 1; }
-        }
-    }
+    if (largeInput)         // part of the set-up time, like the index load, so that no batch pays for allocations
+        for (mp_context *c : contexts) if (mp_reserve(c, &P, maxNumQueries)) { fprintf(stderr, "%s\n", mp_last_error()); return 1; }
     // -b: BAM records are compressed on the device, by the worker's own context, in pieces of at most bgzfPiece bytes staged in
     // page-locked buffers of the pool (two per context, made here so that the loop allocates nothing)
     const bool deviceBgzf = opt.outputBAM && !getenv("MP_HOST_IO");
@@ -1395,7 +1364,7 @@ int main(int argc, char **argv)
         ensure_batch();
         const double tInflate = r1.gzSeconds + r2.gzSeconds - gz0;
         const size_t cap1 = window_cap(0, r1), cap2 = window_cap(1, r2);
-        auto pc = pin_take(cap1 + cap2 + (size_t)maxNumQueries * growPerRead.load() + ((size_t)1 << 20));
+        auto pc = pin_take(cap1 + cap2 + out_room());
         if (!pc.first) { fprintf(stderr, "%s\n", mp_last_error()); exit(1); }
         rb.pin = pc.first; rb.pinCap = pc.second; rb.off2 = cap1;
         const double ts1 = now_s();
@@ -1407,20 +1376,25 @@ int main(int argc, char **argv)
         size_t p1 = r1.pos + rb.bytes1, p2 = r2.pos + rb.bytes2;
         if (n1 == -2 || n2 == -2) {
             // records much longer than the estimate: locate the batch exactly, then copy it
-            std::thread l2([&] { n2 = locate_records(r2, maxNumQueries / 2, stageThreads, &p2); });
-            n1 = locate_records(r1, (maxNumQueries + 1) / 2, stageThreads, &p1);
+            LineBlocks lb1, lb2;
+            std::thread l2([&] { n2 = locate_records(r2, maxNumQueries / 2, stageThreads, &p2, lb2); });
+            n1 = locate_records(r1, (maxNumQueries + 1) / 2, stageThreads, &p1, lb1);
             l2.join();
             if (n1 > 0 && n2 > 0) {
                 rb.bytes1 = p1 - r1.pos; rb.bytes2 = p2 - r2.pos; rb.off2 = (rb.bytes1 + 63) & ~(size_t)63;
-                const size_t need = rb.off2 + rb.bytes2 + (size_t)maxNumQueries * growPerRead.load() + ((size_t)1 << 20);
+                const size_t need = rb.off2 + rb.bytes2 + out_room();
                 if (need > rb.pinCap) {
                     pin_give(rb.pin, rb.pinCap);
                     pc = pin_take(need);
                     if (!pc.first) { fprintf(stderr, "%s\n", mp_last_error()); exit(1); }
                     rb.pin = pc.first; rb.pinCap = pc.second;
                 }
-                std::thread c2([&] { parallel_copy(rb.pin + rb.off2, r2.base + r2.pos, rb.bytes2, stageThreads); });
-                parallel_copy(rb.pin, r1.base + r1.pos, rb.bytes1, stageThreads);
+                auto copy = [&](char *dst, const char *src, size_t n) {         // in 4 MiB pieces
+                    const size_t piece = (size_t)4 << 20;
+                    parallel_for((n + piece - 1) / piece, stageThreads, [&](size_t k) { memcpy(dst + k * piece, src + k * piece, std::min(piece, n - k * piece)); });
+                };
+                std::thread c2([&] { copy(rb.pin + rb.off2, r2.base + r2.pos, rb.bytes2); });
+                copy(rb.pin, r1.base + r1.pos, rb.bytes1);
                 c2.join();
             }
         }
@@ -1458,11 +1432,7 @@ int main(int argc, char **argv)
             const int rc = mp_fastq_upload(contexts[0], firstRaw.pin, firstRaw.bytes1, firstRaw.pin + firstRaw.off2, firstRaw.bytes2, firstRaw.nReads / 2,
                                            ((uint32_t)maxLen + 15) / 16, (uint32_t)maxLen, &lens);
             if (rc == 0) {
-                std::vector<uint32_t> lv(lens, lens + firstRaw.nReads);
-                const uint32_t d1 = detect_read_length(lv, firstRaw.nReads, 0), d2 = detect_read_length(lv, firstRaw.nReads, 1);
-                if (opt.insert_low < (int)d2) opt.insert_low = (int)d2;
-                if (opt.insert_low < (int)d1) opt.insert_low = (int)d1;
-                P.insert_low = opt.insert_low;
+                first_batch(lens, firstRaw.nReads);
                 haveFirstRaw = true;
                 // every context's ingest / egress buffers sized like the first batch (no cudaMalloc inside the batch loop)
                 if (r1.pos < r1.end)
@@ -1527,6 +1497,9 @@ int main(int argc, char **argv)
     Job *firstJob = nullptr;                                       // the batch already uploaded to contexts[0] (device ingest)
     const size_t maxInflight = contexts.size() + 2;
     const int stageUnpaired = P.skipDefaultDP ? 2 : 3;
+    // host threads that format (or -lsam rewrite) one batch: -T, but no more than a context's share of the cores
+    const unsigned fmtThreads = std::min<unsigned>((unsigned)std::max(1, opt.numCpuThreads),
+                                                   std::max<unsigned>(1u, std::max(1u, std::thread::hardware_concurrency()) / (unsigned)contexts.size()));
 
     std::thread reader([&]() {
         uint64_t seq = 0; bool detected = false; double last = now_s();
@@ -1557,13 +1530,7 @@ int main(int argc, char **argv)
             }
             j->seq = seq++;
             double t = now_s(); j->loadSeconds = t - last;
-            if (!detected) {                                       // first batch: read-length detection and insert_low clamp (SOAP4.cpp:458-474)
-                uint32_t d1 = detect_read_length(j->b->lens, j->b->nReads, 0), d2 = detect_read_length(j->b->lens, j->b->nReads, 1);
-                if (opt.insert_low < (int)d2) opt.insert_low = (int)d2;
-                if (opt.insert_low < (int)d1) opt.insert_low = (int)d1;
-                P.insert_low = opt.insert_low;
-                detected = true;
-            }
+            if (!detected) { first_batch(j->b->lens.data(), j->b->nReads); detected = true; }
             std::unique_lock<std::mutex> lk(mu);
             cvRoom.wait(lk, [&] { return inflight < maxInflight; });
             ++inflight; inq.push_back(j);
@@ -1646,56 +1613,22 @@ int main(int argc, char **argv)
                     if (timing) fprintf(stderr, "[timing]  batch %llu: format (device) %.3f fetch %.3f s (%.0f MB)\n", (unsigned long long)j->seq, tf1 - tf0, now_s() - tf1, ob / 1e6);
                     if (rc) { j->log += std::string(mp_last_error()) + "\n"; j->failed = true; }
                     else if (opt.lsam < 0) j->outBytes = ob;
-                    else {
-                        // -lsam: the device-made text is cut at pair boundaries (every eighth line, found by counting newlines in blocks) and
-                        // each piece rewritten into fastq2lsam's lines by one of the -T threads
-                        const char *txt = j->raw.pin;
-                        const size_t B = (size_t)1 << 18, nBlocks = ((size_t)ob + B - 1) / B;
-                        const unsigned hw = std::max(1u, std::thread::hardware_concurrency());
-                        const unsigned nThr = std::min<unsigned>((unsigned)std::max(1, opt.numCpuThreads), std::max<unsigned>(1u, hw / (unsigned)contexts.size()));
-                        std::vector<uint32_t> cnt(nBlocks);
-                        auto par = [&](size_t n, const std::function<void(size_t)> &fn) {
-                            const unsigned T = (unsigned)std::min<size_t>(nThr, std::max<size_t>(n, 1));
-                            std::vector<std::thread> th;
-                            for (unsigned t = 1; t < T; ++t) th.emplace_back([&, t] { for (size_t k = t; k < n; k += T) fn(k); });
-                            for (size_t k = 0; k < n; k += T) fn(k);
-                            for (std::thread &x : th) x.join();
-                        };
-                        par(nBlocks, [&](size_t k) { cnt[k] = (uint32_t)count_newlines(txt + k * B, std::min(B, (size_t)ob - k * B)); });
-                        std::vector<uint64_t> pre(nBlocks + 1, 0);
-                        for (size_t k = 0; k < nBlocks; ++k) pre[k + 1] = pre[k] + cnt[k];
-                        const uint64_t nPairsOut = pre[nBlocks] / 8;
-                        const unsigned nc = (unsigned)std::min<uint64_t>(nThr, std::max<uint64_t>(1, nPairsOut / 4096));
-                        std::vector<size_t> cut(nc + 1, (size_t)ob);
-                        cut[0] = 0;
-                        for (unsigned c = 1; c < nc; ++c) {
-                            const uint64_t L = 8 * (nPairsOut * c / nc);            // the piece starts behind the L-th newline
-                            if (L == 0) { cut[c] = 0; continue; }
-                            const size_t k = (size_t)(std::lower_bound(pre.begin(), pre.end(), L) - pre.begin()) - 1;
-                            const char *q = txt + k * B;
-                            for (uint64_t need = L - pre[k]; need; --need) q = (const char *)memchr(q, '\n', (size_t)(txt + ob - q)) + 1;
-                            cut[c] = (size_t)(q - txt);
-                        }
-                        j->fqParts.assign(nc, std::string());
-                        par(nc, [&](size_t c) { if (cut[c + 1] > cut[c]) fastq_chunk_to_lsam(txt + cut[c], cut[c + 1] - cut[c], opt.lsam != 0, j->fqParts[c]); });
-                    }
+                    else lsam_pieces(j->raw.pin, (size_t)ob, fmtThreads, opt.lsam != 0, j->fqParts);      // -lsam: rewritten by the -T threads
                 } else if (opt.megapathMode || opt.outputBAM) {
                     ReadBatch &b = *j->b;
                     oc.b = &b;
                     // Formatting is spread over the -T host threads: every chunk of pairs writes its own text / BAM records, and the
                     // chunks are concatenated in order, so the stream is the one a single thread would have produced.
-                    const unsigned hw = std::max(1u, std::thread::hardware_concurrency());
-                    const unsigned nThr = std::min<unsigned>((unsigned)std::max(1, opt.numCpuThreads), std::max<unsigned>(1u, hw / (unsigned)contexts.size()));
                     struct Chunk { std::string fq; std::vector<uint8_t> bam, bamz; };   // bamz: the chunk's BAM records as BGZF blocks
                     auto run_chunks = [&](uint64_t nItems, int bamSlot, const std::function<uint64_t(uint64_t)> &alignStart,
                                           const std::function<void(OutCtx &, std::string &, uint64_t, uint64_t)> &body) {
                         if (nItems == 0) return;
-                        const unsigned nc = (unsigned)std::min<uint64_t>(nThr, (nItems + 4095) / 4096);
+                        const unsigned nc = (unsigned)std::min<uint64_t>(fmtThreads, (nItems + 4095) / 4096);
                         std::vector<uint64_t> cut(nc + 1, nItems);
                         cut[0] = 0;
                         for (unsigned c = 1; c < nc; ++c) cut[c] = std::max(cut[c - 1], alignStart(nItems * c / nc));
                         std::vector<Chunk> chunks(nc);
-                        auto one = [&](unsigned c) {
+                        parallel_for(nc, fmtThreads, [&](size_t c) {
                             OutCtx occ = oc; BamWriter capw; capw.capture = &chunks[c].bam;
                             OutScratch scr; occ.scratch = &scr;
                             occ.bam = opt.outputBAM ? &capw : nullptr;
@@ -1703,11 +1636,7 @@ int main(int argc, char **argv)
                             body(occ, chunks[c].fq, cut[c], cut[c + 1]);
                             if (opt.lsam >= 0 && !chunks[c].fq.empty()) { std::string ls; fastq_chunk_to_lsam(chunks[c].fq.data(), chunks[c].fq.size(), opt.lsam != 0, ls); chunks[c].fq.swap(ls); }
                             if (!deviceBgzf && !chunks[c].bam.empty()) { BgzfWriter::compress_all(chunks[c].bam.data(), chunks[c].bam.size(), chunks[c].bamz); std::vector<uint8_t>().swap(chunks[c].bam); }
-                        };
-                        std::vector<std::thread> ths;
-                        for (unsigned c = 1; c < nc; ++c) ths.emplace_back(one, c);
-                        one(0);
-                        for (std::thread &t : ths) t.join();
+                        });
                         if (deviceBgzf) {
                             // the chunks' records, in order, through one staging buffer: every full piece is compressed as it fills
                             const double tc0 = now_s();

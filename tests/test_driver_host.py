@@ -195,7 +195,8 @@ def test_parallel_mapped_parser_equals_sequential(tmp_path, kind):
     assert got == want
 
 
-# ---- device ingest: the staging step that hands mp_fastq_upload the exact byte range of a batch (locate_records / stage_file) ----
+# ---- device ingest: the staging step that hands mp_fastq_upload the exact byte range of a batch.  The exact location and the fused
+#      copy + count take the same block-wise newline index with different block counters; both must name the same bytes ----
 def _stage(path, max_rec, threads, bpr=None):
     out = subprocess.run([EXE, "__stage", str(path), str(max_rec), str(threads)] + ([str(bpr)] if bpr else []), capture_output=True, check=True, timeout=120).stdout
     return [tuple(int(x) for x in l.split()) for l in out.decode().splitlines()]
@@ -242,11 +243,12 @@ def test_staging_refuses_what_the_kernels_cannot_index(tmp_path, name):
     assert rows[0][0] == -1 and rows[0][2] == -1
 
 
-@pytest.mark.parametrize("output_seq", ["1", "0"])
-def test_lsam_mode_randomized_against_reference_fastq2lsam(tmp_path, output_seq):
+@pytest.mark.parametrize("output_seq,threads", [("1", 1), ("0", 1), ("1", 5), ("0", 5)], ids=["1", "0", "1-5threads", "0-5threads"])
+def test_lsam_mode_randomized_against_reference_fastq2lsam(tmp_path, output_seq, threads):
     """20 000 records with generated comments -- IGNORE, zero / negative / signed scores, lists with several accessions per score, empty
     fields, long scores with dozens of one-letter accessions (the list outgrows twice the comment), names with and without /1 /2,
-    unpaired names -- through -lsam and through the reference's own cc/fastq2lsam"""
+    unpaired names -- through -lsam and through the reference's own cc/fastq2lsam.  Records come two by two (a pair, or two unpaired
+    names), so with several threads the text is cut every eighth line as the driver cuts a batch, and the pieces join to the same lines."""
     from conftest import run_ref_fastq2lsam
     rng = np.random.default_rng(int(output_seq) + 5)
     out = []
@@ -279,6 +281,6 @@ def test_lsam_mode_randomized_against_reference_fastq2lsam(tmp_path, output_seq)
     f = tmp_path / "r.fq"
     f.write_bytes(b"".join(out))
     want = run_ref_fastq2lsam("randomized", b"".join(out), output_seq, str(tmp_path))
-    got = subprocess.run([EXE, "__lsam", str(f), output_seq], capture_output=True, check=True, timeout=120).stdout
+    got = subprocess.run([EXE, "__lsam", str(f), output_seq, str(threads)], capture_output=True, check=True, timeout=120).stdout
     assert want.count(b"\n") == 20000 and want.count(b"\t64\t") > 8000 and want.count(b"\t0\t") > 1000
     assert got == want
