@@ -141,6 +141,12 @@ void mp_destroy(mp_context *ctx);
  * latency-bound traceback with the other batch's compute-bound kernels (the reference double-buffers batches the same
  * way, SOAP4.cpp:424-441, 576-585).  `src` must outlive the clone. */
 int  mp_clone(mp_context *src, mp_context **ctx);
+/* points a clone (mp_clone) at the resident index of `owner`, a context on the same GPU that owns one: from then on the clone uses
+ * owner's index, its K-mer filter (borrowed, as mp_clone borrows it) and, if owner has one, its annotation (mp_annotation_upload on
+ * owner) -- until the next mp_index_bind.  The uploaded batch and its FASTQ text stay; seeding and results are invalidated.  One
+ * worker context thus carries a batch through several chunk indexes with one set of work buffers (soap4 -chain).
+ * MP_ERR_STATE: ctx is not a clone; MP_ERR_ARG: owner owns no index or is on another device.  owner must outlive the binding. */
+int  mp_index_bind(mp_context *ctx, mp_context *owner);
 const char *mp_last_error(void);
 /* number of this library's own CUDA kernels launched so far in the process (bench.py "gpu_launches") */
 uint64_t mp_launch_count(void);
@@ -149,6 +155,11 @@ uint64_t mp_launch_count(void);
  * Host reads <prefix>.{bwt,fmv,sa,lkt,pac}; the library owns the HBM copies (re-laid out).
  * .ann/.amb/.tra (chromosome translation) stay with the caller: they are host-side output data. */
 int  mp_index_load(mp_context *ctx, const char *prefix);
+/* mp_index_load whose resident index -- and the K-mer filter mp_index_prepare adds later -- stay within maxBytes of HBM (hbmBytes of
+ * mp_index_info): the SA takes the densest form that fits beside the BWT, LKT and text (a u32 entry per position for texts below
+ * 2^32, else 40-bit samples at the densest rate that fits, else the file's samples), and the filter what is left, or none.  Results
+ * do not depend on either.  MP_ERR_CAPACITY: the index does not fit even with the file's samples.  maxBytes = 0: mp_index_load. */
+int  mp_index_load_budget(mp_context *ctx, const char *prefix, uint64_t maxBytes);
 int  mp_index_info(mp_context *ctx, uint64_t *textLength, uint64_t *inverseSa0, uint64_t cumFreq[5], uint64_t *hbmBytes);
 /* ---- index built in HBM from a packed text (GPU index builder; replaces 2bwt-builder,
  *      2bwt-lib/2BWT-Builder.c, for the bench/synthetic path).  text2bit: 4 bases per byte,
@@ -229,6 +240,15 @@ int  mp_last_stats(mp_context *ctx, mp_stats *stats);
 #define MP_ERR_FORMAT (-6)
 int  mp_fastq_upload(mp_context *ctx, const char *text1, uint64_t bytes1, const char *text2, uint64_t bytes2,
                      uint32_t nPairs, uint32_t wordPerQuery, uint32_t maxReadLength, const uint32_t **readLengths);
+
+/* The context's last mp_format_fastq text (still on the device) becomes its next batch, as the next chunk of a chunked index reads it
+ * (`soap4 -F ... | deinterleave | soap4 ...`, runMegaPath.sh:184-226): every record's header "@NAME<blanks>TAIL" is rewritten to
+ * "@NAME'/<mate> TAIL" (NAME' is NAME without one trailing "/1" or "/2"; records alternate mate 1, mate 2; no TAIL: "@NAME'/<mate>"),
+ * records go to the text of their mate, and the two texts are ingested exactly as mp_fastq_upload ingests host text (same checks,
+ * lengths, record views and 2-bit rows).  Nothing crosses PCIe.  MP_ERR_STATE: nothing formatted since the last upload.
+ * MP_ERR_FORMAT: the rewritten text is not what the ingest takes (a header of 60000 bytes or more); mp_format_fetch then still returns
+ * the formatted text, so that the caller can take the batch on through its own parser and mp_batch_upload. */
+int  mp_fastq_chain(mp_context *ctx, uint32_t wordPerQuery, uint32_t maxReadLength, const uint32_t **readLengths);
 
 /* sizes a context's ingest / egress buffers for batches of nPairs pairs and textBytes of FASTQ text (both mates) before the batch loop */
 int  mp_fastq_reserve(mp_context *ctx, uint64_t textBytes, uint32_t nPairs);

@@ -125,6 +125,9 @@ def lib():
         L.mp_init.argtypes = [C.c_int, C.POINTER(C.c_void_p)]
         L.mp_destroy.argtypes = [C.c_void_p]
         L.mp_clone.argtypes = [C.c_void_p, C.POINTER(C.c_void_p)]
+        L.mp_index_bind.argtypes = [C.c_void_p, C.c_void_p]
+        L.mp_index_load_budget.argtypes = [C.c_void_p, C.c_char_p, C.c_uint64]
+        L.mp_fastq_chain.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p]
         L.mp_index_prepare.argtypes = [C.c_void_p, C.c_void_p]
         L.mp_reserve.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
         L.mp_index_load.argtypes = [C.c_void_p, C.c_char_p]
@@ -283,6 +286,16 @@ class Context:
         self._check(self.L.mp_index_load(self.h, prefix.encode()))
         self._has_index = True
 
+    def index_load_budget(self, prefix, max_bytes):
+        """mp_index_load with the resident index and its K-mer filter kept within max_bytes of HBM."""
+        self._check(self.L.mp_index_load_budget(self.h, prefix.encode(), int(max_bytes)))
+        self._has_index = True
+
+    def index_bind(self, owner):
+        """Points this clone at owner's resident index, K-mer filter and annotation (mp_index_bind)."""
+        self._check(self.L.mp_index_bind(self.h, owner.h))
+        self._bound = owner                   # the owner must outlive the binding
+
     def index_build(self, text2bit, n):
         """GPU FM-index construction from a .pac-packed text (replaces 2bwt-builder)."""
         text2bit = np.ascontiguousarray(text2bit, dtype=np.uint8)
@@ -357,6 +370,7 @@ class Context:
         read_lengths = np.ascontiguousarray(read_lengths, dtype=np.uint32)
         self._keep = (queries, read_lengths)
         self._check(self.L.mp_batch_upload(self.h, _ptr(queries), _ptr(read_lengths), len(read_lengths), wpq))
+        self._n_reads = len(read_lengths)
 
     def batch_upload_ptr(self, host_ptr, read_lengths, wpq):
         """Same call with a raw host pointer (e.g. a pinned torch tensor's data_ptr())."""
@@ -374,7 +388,18 @@ class Context:
         if rc == MP_ERR_FORMAT:
             raise FastqFormatError(self.L.mp_last_error().decode())
         self._check(rc)
+        self._n_reads = 2 * n_pairs
         return np.ctypeslib.as_array(lens, shape=(2 * n_pairs,)).copy()
+
+    def fastq_chain(self, max_read_length):
+        """mp_fastq_chain: the batch's last formatted text, rewritten as the next chunk reads it, becomes the batch -> clamped read
+        lengths.  Raises FastqFormatError when the ingest refuses the rewritten text (the formatted text is still fetchable then)."""
+        lens = C.POINTER(C.c_uint32)()
+        rc = self.L.mp_fastq_chain(self.h, words_per_query(max_read_length), max_read_length, C.byref(lens))
+        if rc == MP_ERR_FORMAT:
+            raise FastqFormatError(self.L.mp_last_error().decode())
+        self._check(rc)
+        return np.ctypeslib.as_array(lens, shape=(self._n_reads,)).copy()
 
     def annotation_upload(self, prefix):
         """mp_annotation_upload from <prefix>.ann / .tra (the tables getChrAndPos reads, BGS-IO.cpp:163-190)."""

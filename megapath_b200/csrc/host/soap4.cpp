@@ -46,6 +46,7 @@
 #include <functional>
 #include <mutex>
 #include <thread>
+#include <cuda_runtime_api.h>
 #include "megapath_b200.h"
 #include "bam_out.h"
 
@@ -58,12 +59,14 @@ struct Options {
     int megapathMode = 0, top = 95, ignoreComments = 0, alignmentType = 2, printMDNM = 0;
     int numGpus = 1, contextsPerGpu = 3;       // extensions: -G <n> uses GPUs device..device+n-1; MP_CONTEXTS_PER_GPU overrides 3
     int lsam = -1;                             // extension: -lsam <0|1> prints what `soap4 -F | fastq2lsam <0|1>` prints (cc/fastq2lsam.cpp)
+    // extension: -chain <index prefix> <output prefix>, repeatable: the next chunk index of an NT chunk chain (runMegaPath.sh:184-226)
+    std::vector<std::pair<std::string, std::string>> chain;
 };
 
 static bool parse_args(int argc, char **argv, Options &o)
 {
     if (argc < 2 || strcmp(argv[1], "pair") != 0) {
-        fprintf(stderr, "Usage: %s pair <index prefix> <reads_1.fq[.gz]> <reads_2.fq[.gz]> [-o prefix] [-C ini] [-L len] [-T n] [-u n] [-v n] [-b] [-F|-P] [-nc] [-top n] [-c gpu]\n", argv[0]);
+        fprintf(stderr, "Usage: %s pair <index prefix> <reads_1.fq[.gz]> <reads_2.fq[.gz]> [-o prefix] [-C ini] [-L len] [-T n] [-u n] [-v n] [-b] [-F|-P] [-nc] [-top n] [-c gpu] [-chain <index prefix> <output prefix>]...\n", argv[0]);
         if (argc >= 2) fprintf(stderr, "Only 'pair' mode is supported (the reference asserts readType == PAIR_END_READ, SOAP4.cpp:554).\n");
         return false;
     }
@@ -90,9 +93,14 @@ static bool parse_args(int argc, char **argv, Options &o)
         else if (!strcmp(a, "-top")) { if (!need("the value of '-top'")) return false; o.top = atoi(argv[i + 1]); }   // the reference does not consume the value (IniParam.cpp:885-892)
         else if (!strcmp(a, "-nc")) o.ignoreComments = 1;
         else if (!strcmp(a, "-lsam")) { if (!need("0 or 1 (outputSeq)")) return false; o.lsam = atoi(argv[++i]) != 0; }
+        else if (!strcmp(a, "-chain")) {
+            if (i + 2 >= argc) { fprintf(stderr, "Please specify the index prefix and the output prefix after '-chain'\n"); return false; }
+            o.chain.emplace_back(argv[i + 1], argv[i + 2]); i += 2;
+        }
         else if (!strcmp(a, "-D") || !strcmp(a, "-A") || !strcmp(a, "-R") || !strcmp(a, "-e")) { if (i + 1 < argc) ++i; }
         else if (!strcmp(a, "-I")) { fprintf(stderr, "illumina quality is not supported yet\n"); return false; }
     }
+    if (!o.chain.empty() && o.megapathMode == 0) { fprintf(stderr, "-chain needs -F or -P: the chunks pass their scores through the FASTQ comments\n"); return false; }
     if (o.insert_low > o.insert_high) { fprintf(stderr, "The minimum value of insert size should not be greater than the maximum value of insert size.\n"); return false; }
     return true;
 }
@@ -1123,6 +1131,38 @@ static void lsam_pieces(const char *text, size_t bytes, unsigned nThr, bool outp
     parallel_for(nc, nc, [&](size_t c) { if (cut[c + 1] > cut[c]) fastq_chunk_to_lsam(cut[c], (size_t)(cut[c + 1] - cut[c]), outputSeq, parts[c]); });
 }
 
+// What the next chunk of a chunk chain reads from a chunk's stdout (cc/deinterleave.cpp, as tests/conftest.py's deinterleave restates
+// it): records are taken in pairs (mate 1, mate 2) and appended to out[mate - 1] as "@NAME'/<mate> TAIL", the bases, "+", the qualities.
+// NAME is the first blank-delimited word of the header after '@', NAME' is NAME without one trailing "/1" or "/2", TAIL the rest of
+// the header after the blanks that follow NAME (no TAIL: "@NAME'/<mate>").  A trailing incomplete record or unpaired record is dropped.
+static void deinterleave_text(const char *p, size_t n, std::string out[2])
+{
+    const char *end = p + n;
+    const char *l[8], *e[8];
+    for (;;) {
+        int k = 0;
+        for (const char *q = p; k < 8; ++k) {
+            const char *nl = (const char *)memchr(q, '\n', (size_t)(end - q));
+            if (!nl) break;
+            l[k] = q; e[k] = nl; q = nl + 1;
+        }
+        if (k < 8) return;
+        for (int m = 0; m < 2; ++m) {
+            const char *h = l[4 * m] + 1, *he = e[4 * m];
+            while (h < he && isspace((unsigned char)*h)) ++h;
+            const char *ne = h; while (ne < he && !isspace((unsigned char)*ne)) ++ne;
+            const char *c = ne; while (c < he && isspace((unsigned char)*c)) ++c;
+            size_t nameLen = (size_t)(ne - h);
+            if (nameLen >= 2 && h[nameLen - 2] == '/' && (h[nameLen - 1] == '1' || h[nameLen - 1] == '2')) nameLen -= 2;
+            std::string &o = out[m];
+            o += '@'; o.append(h, nameLen); o += '/'; o += (char)('1' + m);
+            if (c < he) { o += ' '; o.append(c, (size_t)(he - c)); }
+            o += '\n'; o.append(l[4 * m + 1], (size_t)(e[4 * m + 1] - l[4 * m + 1])); o += "\n+\n"; o.append(l[4 * m + 3], (size_t)(e[4 * m + 3] - l[4 * m + 3])); o += '\n';
+        }
+        p = e[7] + 1;
+    }
+}
+
 int main(int argc, char **argv)
 {
 #ifdef MP_TEST_HOOKS
@@ -1183,6 +1223,18 @@ int main(int argc, char **argv)
         std::vector<std::string> parts; lsam_pieces(data.data(), data.size(), argc >= 5 ? (unsigned)atoi(argv[4]) : 1u, atoi(argv[3]) != 0, parts);
         fprintf(stderr, "converted %.1f MB in %.3f s\n", data.size() / 1e6, now_s() - tc);
         for (const std::string &p : parts) fwrite(p.data(), 1, p.size(), stdout);
+        return 0;
+    }
+    if (argc >= 3 && !strcmp(argv[1], "__deinterleave")) {   // hidden: soap4 -F text -> <file>_1.fq, <file>_2.fq as the next chunk reads them (no GPU)
+        FILE *in = fopen(argv[2], "rb"); if (!in) return 1;
+        std::string data; char tmp[65536]; size_t n;
+        while ((n = fread(tmp, 1, sizeof tmp, in)) > 0) data.append(tmp, n);
+        fclose(in);
+        std::string out[2]; deinterleave_text(data.data(), data.size(), out);
+        for (int m = 0; m < 2; ++m) {
+            FILE *o = fopen((std::string(argv[2]) + (m ? "_2.fq" : "_1.fq")).c_str(), "wb"); if (!o) return 1;
+            fwrite(out[m].data(), 1, out[m].size(), o); fclose(o);
+        }
         return 0;
     }
     if (argc >= 5 && !strcmp(argv[1], "__stage")) {          // hidden: batch boundaries of the device-ingest staging (no GPU): __stage file maxRec threads [bytesPerRec]
@@ -1321,24 +1373,63 @@ int main(int argc, char **argv)
         } else if (r1.end > r1.pos || r2.end > r2.pos) deviceIO = false;           // the first record is not a plain four-line one
     }
 
-    // one index replica per GPU (loaded in parallel), contextsPerGpu contexts sharing it (mp_clone)
+    // The steps of the run: the main index, then every -chain index.  A chunk's text goes to the next chunk as
+    // `soap4 ... | deinterleave | soap4 <next index> ...` would hand it over; only the last chunk's text is printed.
+    struct ChainStep {
+        std::string index, out; int ignoreComments = 0;        // -nc applies to the first index only (runMegaPath.sh:184-226)
+        std::vector<mp_context *> owners;                      // per GPU: the context that owns this chunk's resident index
+        Annotation ann; OutCtx octx; BamWriter bamDP, bamGout, bamUnpair; std::vector<uint8_t> hostPac;
+        uint64_t pairsAligned = 0;
+    };
+    std::vector<std::unique_ptr<ChainStep>> steps;
+    for (size_t k = 0; k <= opt.chain.size(); ++k) {
+        steps.emplace_back(new ChainStep);
+        ChainStep &c = *steps.back();
+        c.index = k ? opt.chain[k - 1].first : opt.indexName; c.out = k ? opt.chain[k - 1].second : opt.outputPrefix;
+        c.ignoreComments = k ? 0 : opt.ignoreComments; c.owners.assign(opt.numGpus, nullptr);
+    }
+    const size_t K = steps.size();
+    const bool chained = K > 1;
+    // one index replica per GPU (loaded in parallel), contextsPerGpu contexts sharing it (mp_clone).  A chain loads every chunk's index
+    // on every GPU into an owner context of its own, each within a share of the free HBM proportional to its text length once a working
+    // reserve per worker context is set aside (its batch, DP and traceback buffers; the traceback arena sizes itself from what is free),
+    // and its workers are clones that mp_index_bind carries from chunk to chunk.
+    const uint64_t chainReservePerContext = 16ull << 30;
     fprintf(stderr, "[Main] loading index into device...\n");
-    std::vector<mp_context *> owners(opt.numGpus, nullptr), contexts;
+    std::vector<mp_context *> contexts; std::vector<int> contextGpu;
     {
+        std::vector<uint64_t> textLen(K, 0); uint64_t textSum = 0;
+        for (size_t k = 0; chained && k < K; ++k) {                 // n from the .bwt header (BWT.c:139-152)
+            FILE *f = fopen((steps[k]->index + ".bwt").c_str(), "rb"); uint64_t hdr[5] = { 0, 0, 0, 0, 0 };
+            if (!f || fread(hdr, 8, 5, f) != 5) { fprintf(stderr, "cannot read %s.bwt\n", steps[k]->index.c_str()); if (f) fclose(f); return 1; }
+            fclose(f); textLen[k] = hdr[4]; textSum += hdr[4];
+        }
         std::vector<std::thread> loaders; std::vector<std::string> errs(opt.numGpus);
         for (int g = 0; g < opt.numGpus; ++g)
             loaders.emplace_back([&, g]() {
-                if (mp_init(opt.device + g, &owners[g]) || mp_index_load(owners[g], opt.indexName.c_str())) errs[g] = mp_last_error();
+                uint64_t avail = 0;
+                if (chained) {
+                    size_t freeB = 0, totalB = 0;
+                    const uint64_t reserve = chainReservePerContext * (uint64_t)opt.contextsPerGpu;
+                    if (cudaSetDevice(opt.device + g) != cudaSuccess || cudaMemGetInfo(&freeB, &totalB) != cudaSuccess) { errs[g] = "cannot query the free HBM of the GPU"; return; }
+                    if (freeB <= reserve) { errs[g] = "-chain: the GPU has less free HBM than the working reserve of its contexts"; return; }
+                    avail = freeB - reserve;
+                }
+                for (size_t k = 0; k < K; ++k) {
+                    ChainStep &c = *steps[k];
+                    const uint64_t budget = chained ? (uint64_t)((double)avail * (double)textLen[k] / (double)std::max<uint64_t>(textSum, 1)) : 0;
+                    if (mp_init(opt.device + g, &c.owners[g]) || mp_index_load_budget(c.owners[g], c.index.c_str(), budget)) { errs[g] = (chained ? c.index + ": " : std::string()) + mp_last_error(); return; }
+                }
             });
         for (std::thread &t : loaders) t.join();
         for (int g = 0; g < opt.numGpus; ++g) if (!errs[g].empty()) { fprintf(stderr, "%s\n", errs[g].c_str()); return 1; }
         for (int g = 0; g < opt.numGpus; ++g) {
-            if (mp_index_prepare(owners[g], &P)) { fprintf(stderr, "%s\n", mp_last_error()); return 1; }
-            contexts.push_back(owners[g]);
-            for (int k = 1; k < opt.contextsPerGpu; ++k) {
+            for (size_t k = 0; k < K; ++k) if (mp_index_prepare(steps[k]->owners[g], &P)) { fprintf(stderr, "%s\n", mp_last_error()); return 1; }
+            if (!chained) { contexts.push_back(steps[0]->owners[g]); contextGpu.push_back(g); }
+            for (int k = chained ? 0 : 1; k < opt.contextsPerGpu; ++k) {
                 mp_context *c = nullptr;
-                if (mp_clone(owners[g], &c)) { fprintf(stderr, "%s\n", mp_last_error()); return 1; }
-                contexts.push_back(c);
+                if (mp_clone(steps[0]->owners[g], &c)) { fprintf(stderr, "%s\n", mp_last_error()); return 1; }
+                contexts.push_back(c); contextGpu.push_back(g);
             }
         }
     }
@@ -1355,8 +1446,8 @@ int main(int argc, char **argv)
         }
     }
     if (pinThread.joinable()) pinThread.join();
-    Annotation ann;
-    if (!ann.load(opt.indexName)) return 1;
+    for (auto &c : steps) if (!c->ann.load(c->index)) return 1;
+    const Annotation &ann = steps[0]->ann;
     // -> 1: the next batch staged in page-locked memory (file positions advanced), 0: end of both files, -1: not for the device path
     auto stage_raw = [&](RawBatch &rb) -> int {
         static const bool ltiming = getenv("MP_DRIVER_TIMING") != nullptr;
@@ -1411,16 +1502,18 @@ int main(int argc, char **argv)
         return 1;
     };
     RawBatch firstRaw; bool haveFirstRaw = false;
-    if (deviceIO) {
-        std::vector<uint64_t> nameOff(ann.numSeq + 1, 0); std::string nameBlob;
-        for (uint32_t i = 0; i < ann.numSeq; ++i) { nameOff[i] = nameBlob.size(); nameBlob += ann.names[i]; }
-        nameOff[ann.numSeq] = nameBlob.size();
-        std::vector<uint64_t> trStart(ann.tr.size()); std::vector<uint32_t> trChr(ann.tr.size());
-        for (size_t k = 0; k < ann.tr.size(); ++k) { trStart[k] = ann.tr[k].startPos; trChr[k] = ann.tr[k].chrID; }
+    // the annotation each formatting context reads: its own, or on a chain every owner's (bound workers read their owner's)
+    for (size_t k = 0; deviceIO && k < K; ++k) {
+        const Annotation &an = steps[k]->ann;
+        std::vector<uint64_t> nameOff(an.numSeq + 1, 0); std::string nameBlob;
+        for (uint32_t i = 0; i < an.numSeq; ++i) { nameOff[i] = nameBlob.size(); nameBlob += an.names[i]; }
+        nameOff[an.numSeq] = nameBlob.size();
+        std::vector<uint64_t> trStart(an.tr.size()); std::vector<uint32_t> trChr(an.tr.size());
+        for (size_t t = 0; t < an.tr.size(); ++t) { trStart[t] = an.tr[t].startPos; trChr[t] = an.tr[t].chrID; }
         mp_annotation A; memset(&A, 0, sizeof A);
-        A.dnaLength = ann.dnaLength; A.numSeq = ann.numSeq; A.gridEntries = (uint32_t)ann.grid.size(); A.numTranslate = (uint32_t)ann.tr.size();
-        A.grid = ann.grid.data(); A.trStartPos = trStart.data(); A.trChrID = trChr.data(); A.names = nameBlob.data(); A.nameOffsets = nameOff.data();
-        for (mp_context *c : contexts) if (mp_annotation_upload(c, &A)) { fprintf(stderr, "[Main] %s; formatting on the host\n", mp_last_error()); deviceIO = false; break; }
+        A.dnaLength = an.dnaLength; A.numSeq = an.numSeq; A.gridEntries = (uint32_t)an.grid.size(); A.numTranslate = (uint32_t)an.tr.size();
+        A.grid = an.grid.data(); A.trStartPos = trStart.data(); A.trChrID = trChr.data(); A.names = nameBlob.data(); A.nameOffsets = nameOff.data();
+        for (mp_context *c : chained ? steps[k]->owners : contexts) if (mp_annotation_upload(c, &A)) { fprintf(stderr, "[Main] %s; formatting on the host\n", mp_last_error()); deviceIO = false; break; }
     }
     if (deviceIO) {
         // The first batch is staged and indexed here, as part of the set-up: its verdict decides between the device and the host loops
@@ -1450,44 +1543,46 @@ int main(int argc, char **argv)
     fprintf(stderr, "[Main] Loading time : %9.4f seconds\n\n", tIndex - t0);
     fprintf(stderr, "[Main] top_percentage: %f\n", top);
     fprintf(stderr, "[Main] Reference sequence length : %llu\n\n", (unsigned long long)ann.dnaLength);
-    OutCtx octx;
-    octx.ann = &ann; octx.megapathMode = opt.megapathMode; octx.top = top; octx.ignoreComments = opt.ignoreComments != 0;
-    octx.readGroup = opt.query1; octx.printMDNM = opt.printMDNM != 0; octx.alignmentType = opt.alignmentType;
-    octx.mismatchScore = P.mismatchScore; octx.matchScore = P.matchScore; octx.minMAPQ = ini.geti("Score:MinMAPQ", 1); octx.maxMAPQ = ini.geti("Score:MaxMAPQ", 40);
-    octx.bwaLike = ini.geti("Score:BWALikeScore", 0) != 0;
-    BamWriter bamDP, bamGout, bamUnpair;
-    std::vector<uint8_t> hostPac;
-    if (opt.outputBAM) {
-        if (!octx.bwaLike) { fprintf(stderr, "-b needs Score:BWALikeScore=1 (the only MAPQ scheme of the shipped .ini files)\n"); return 1; }
-        bwase_initialize();
+    if (opt.outputBAM && ini.geti("Score:BWALikeScore", 0) == 0) { fprintf(stderr, "-b needs Score:BWALikeScore=1 (the only MAPQ scheme of the shipped .ini files)\n"); return 1; }
+    if (opt.outputBAM) bwase_initialize();
+    for (auto &cp : steps) {
+        ChainStep &c = *cp;
+        OutCtx &octx = c.octx;
+        octx.ann = &c.ann; octx.megapathMode = opt.megapathMode; octx.top = top; octx.ignoreComments = c.ignoreComments != 0;
+        octx.readGroup = opt.query1; octx.printMDNM = opt.printMDNM != 0; octx.alignmentType = opt.alignmentType;
+        octx.mismatchScore = P.mismatchScore; octx.matchScore = P.matchScore; octx.minMAPQ = ini.geti("Score:MinMAPQ", 1); octx.maxMAPQ = ini.geti("Score:MaxMAPQ", 40);
+        octx.bwaLike = ini.geti("Score:BWALikeScore", 0) != 0;
+        if (!opt.outputBAM) continue;
         // SAMOutputHeaderConstruct (SAM.cpp:83-134)
         std::vector<std::string> tnames; std::vector<uint32_t> tlens; std::string sq;
-        for (uint32_t i = 0; i < ann.numSeq; ++i) {
-            std::string nm = ann.names[i]; size_t e = nm.find_first_of(" \t\r\n"); if (e != std::string::npos) nm.resize(e);
-            tnames.push_back(nm); tlens.push_back((uint32_t)ann.actualLen[i]);
+        for (uint32_t i = 0; i < c.ann.numSeq; ++i) {
+            std::string nm = c.ann.names[i]; size_t e = nm.find_first_of(" \t\r\n"); if (e != std::string::npos) nm.resize(e);
+            tnames.push_back(nm); tlens.push_back((uint32_t)c.ann.actualLen[i]);
             sq += "@SQ\tSN:" + nm + "\tLN:" + std::to_string(tlens.back()) + "\n";
         }
         std::string text = "@HD\tVN:1.3\tSO:unsorted\n@RG\tID:" + octx.readGroup + "\tSM:\t\n" + sq + "@PG\tID:soap4\tPN:soap4\tVN:megapath_b200\n";
-        bool ok = bamDP.open(opt.outputPrefix + ".dpout.1", text, tnames, tlens) && bamUnpair.open(opt.outputPrefix + ".unpair", text, tnames, tlens) &&
-                  bamGout.open(opt.outputPrefix + ".gout.1", text, tnames, tlens);
+        bool ok = c.bamDP.open(c.out + ".dpout.1", text, tnames, tlens) && c.bamUnpair.open(c.out + ".unpair", text, tnames, tlens) &&
+                  c.bamGout.open(c.out + ".gout.1", text, tnames, tlens);
         for (int t = 2; ok && t <= opt.numCpuThreads; ++t) {       // the reference opens one .gout file per CPU thread; the pipeline globs them
-            BamWriter extra; ok = extra.open(opt.outputPrefix + ".gout." + std::to_string(t), text, tnames, tlens); extra.close();
+            BamWriter extra; ok = extra.open(c.out + ".gout." + std::to_string(t), text, tnames, tlens); extra.close();
         }
-        if (!ok) { fprintf(stderr, "cannot create the BAM output files with prefix %s\n", opt.outputPrefix.c_str()); return 1; }
+        if (!ok) { fprintf(stderr, "cannot create the BAM output files with prefix %s\n", c.out.c_str()); return 1; }
         if (opt.printMDNM) {                                        // MD strings need the text
-            FILE *pf = fopen((opt.indexName + ".pac").c_str(), "rb");
-            if (!pf) { fprintf(stderr, "cannot open %s.pac\n", opt.indexName.c_str()); return 1; }
-            hostPac.resize((ann.dnaLength + 3) / 4 + 8);
-            if (fread(hostPac.data(), 1, (ann.dnaLength + 3) / 4, pf) != (ann.dnaLength + 3) / 4) { fprintf(stderr, "short .pac\n"); return 1; }
-            fclose(pf); octx.ax.pac = hostPac.data();
+            FILE *pf = fopen((c.index + ".pac").c_str(), "rb");
+            if (!pf) { fprintf(stderr, "cannot open %s.pac\n", c.index.c_str()); return 1; }
+            c.hostPac.resize((c.ann.dnaLength + 3) / 4 + 8);
+            if (fread(c.hostPac.data(), 1, (c.ann.dnaLength + 3) / 4, pf) != (c.ann.dnaLength + 3) / 4) { fprintf(stderr, "short .pac\n"); return 1; }
+            fclose(pf); octx.ax.pac = c.hostPac.data();
         }
     }
 
     // ---- pipeline: reader thread -> GPU workers (one per context; each formats its own batch) -> ordered writer (this thread).
     //      The reference overlaps read loading with alignment the same way (aio_thread.cpp:804, SOAP4.cpp:424-441, 576-585). ----
     struct Job {
-        uint64_t seq = 0; ReadBatch *b = nullptr; uint32_t nReads = 0; std::vector<std::string> fqParts; std::string log; std::vector<uint8_t> bam[3];
-        uint64_t pairsAligned = 0; double loadSeconds = 0, alignSeconds = 0; bool failed = false;
+        uint64_t seq = 0; ReadBatch *b = nullptr; uint32_t nReads = 0; std::vector<std::string> fqParts; std::string log;
+        std::vector<std::vector<uint8_t>> bam;                     // per chain step: .dpout.1, .gout.1, .unpair records as BGZF members
+        std::vector<uint64_t> pairsAligned;                        // per chain step
+        double loadSeconds = 0, alignSeconds = 0; bool failed = false;
         // device ingest / egress: the batch's FASTQ text staged in page-locked memory; the formatted text comes back into the same buffer
         bool dev = false, uploaded = false; RawBatch raw; uint64_t outBytes = 0;
     };
@@ -1541,8 +1636,7 @@ int main(int argc, char **argv)
         std::lock_guard<std::mutex> lk(mu); readerDone = true; cvIn.notify_all(); cvOut.notify_all();
     });
 
-    auto worker = [&](mp_context *gpu) {
-        OutCtx oc = octx;                                           // per-worker copy: own batch pointer
+    auto worker = [&](mp_context *gpu, int gpuIdx) {
         for (;;) {
             Job *j = nullptr;
             {
@@ -1554,11 +1648,17 @@ int main(int argc, char **argv)
             }
             const double ts = now_s();
             const uint32_t numQueries = j->nReads, nPairs = numQueries / 2;
-            mp_results R;
             static const bool timing = getenv("MP_DRIVER_TIMING") != nullptr;      // per-batch host breakdown on stderr
+            j->bam.assign(3 * K, std::vector<uint8_t>()); j->pairsAligned.assign(K, 0);
+            uint64_t fmtPrev = 0;                                   // size of the previous step's text, still on the device
+            for (size_t k = 0; k < K && !j->failed; ++k) {
+            const bool last = k + 1 == K;
+            const ChainStep &step = *steps[k];
+            mp_results R;
+            const double tk = now_s();
             double tUp = 0, tAl = 0, tFmt = 0, libWallMs = 0, tCmp = 0;
-            int rcUp = 0;
-            if (j->dev && !j->uploaded) {
+            int rcUp = chained ? mp_index_bind(gpu, step.owners[gpuIdx]) : 0;
+            if (!rcUp && k == 0 && j->dev && !j->uploaded) {
                 rcUp = mp_fastq_upload(gpu, j->raw.pin, j->raw.bytes1, j->raw.pin + j->raw.off2, j->raw.bytes2, nPairs, ((uint32_t)maxLen + 15) / 16, (uint32_t)maxLen, nullptr);
                 if (rcUp == MP_ERR_FORMAT) {
                     // the input stops being strict four-line FASTQ in mid-file: this batch goes through the host parser, from the staged
@@ -1576,29 +1676,59 @@ int main(int argc, char **argv)
                     j->dev = false; rcUp = 0;
                 }
             }
+            if (!rcUp && k > 0 && j->dev) {
+                // the previous step's text, rewritten as the next chunk reads it, becomes the batch on the device
+                rcUp = mp_fastq_chain(gpu, ((uint32_t)maxLen + 15) / 16, (uint32_t)maxLen, nullptr);
+                if (rcUp == MP_ERR_FORMAT) {                        // e.g. a header grown past the device record limit
+                    fprintf(stderr, "[Main] batch %llu, %s: %s: host parser and formatter for the rest of its chain\n", (unsigned long long)j->seq, step.index.c_str(), mp_last_error());
+                    std::string text(fmtPrev, '\0');
+                    rcUp = mp_format_fetch(gpu, &text[0], fmtPrev);
+                    j->fqParts.clear(); j->fqParts.push_back(std::move(text));
+                    j->dev = false;
+                }
+            }
+            if (!rcUp && k > 0 && !j->dev) {
+                // the previous step's host text, rewritten as the next chunk reads it, through the host parser
+                std::string t[2];
+                for (const std::string &part : j->fqParts) deinterleave_text(part.data(), part.size(), t);
+                j->fqParts.clear();
+                SeqReader m1, m2;
+                m1.base = &t[0][0]; m1.end = t[0].size(); m1.eof = true; m1.mapped = true;
+                m2.base = &t[1][0]; m2.end = t[1].size(); m2.eof = true; m2.mapped = true;
+                if (!j->b) { j->b = new ReadBatch; j->b->maxReadLength = (uint32_t)maxLen; j->b->wpq = ((uint32_t)maxLen + 15) / 16; }
+                const uint32_t got = load_batch(m1, m2, *j->b, numQueries, ioThreads);
+                if (got != numQueries || m1.pos != m1.end || m2.pos != m2.end) {
+                    j->log += "Error: the text of " + steps[k - 1]->index + " does not parse as " + std::to_string(numQueries) + " reads\n"; j->failed = true; continue;
+                }
+            }
             if (!j->dev && !rcUp) rcUp = mp_batch_upload(gpu, j->b->queries.data(), j->b->lens.data(), numQueries, j->b->wpq);
             mp_results_on_device(gpu, j->dev ? 1 : 0);               // the host formatter needs the result arrays, the device formatter does not
             tUp = now_s();
             if (rcUp || mp_align_pairs(gpu, &P, &R)) {
-                j->log = std::string(mp_last_error()) + "\n"; j->failed = true;
+                j->log += std::string(mp_last_error()) + "\n"; j->failed = true;
             } else {
+                if (chained) j->log += "[Main] chunk " + std::to_string(k) + ": index " + step.index + "\n";
                 char line[512];
                 snprintf(line, sizeof line, "[Main] %u pairs of reads are proceeded to deep DP Round 1.\n[Main] Number of pairs aligned by DP: %llu\n[Main] Number of alignments aligned by DP: %llu\n"
                          "[Main] Number of reads aligned by single-end DP: %llu\n[Main] Number of alignments aligned by DP: %llu\n[Main] Number of pairs aligned by DP: %llu\n[Main] Number of alignments aligned by DP: %llu\n",
                          nPairs, (unsigned long long)R.numDPAlignedPair, (unsigned long long)R.numDPAlignment, (unsigned long long)R.numSingleDPAligned,
                          (unsigned long long)R.numSingleDPAlignment, (unsigned long long)R.numRescuedPair, (unsigned long long)R.numRescuedAlignment);
-                j->log = line;
-                j->pairsAligned = R.numDPAlignedPair + R.numRescuedPair;
+                j->log += line;
+                j->pairsAligned[k] = R.numDPAlignedPair + R.numRescuedPair;
                 tAl = now_s();
                 if (timing) { mp_stats st; if (mp_last_stats(gpu, &st) == 0) libWallMs = st.ms_wall; }
                 // ---- output: stage order of the reference (deep DP pairs, rescued pairs, then everything else) ----
                 if (j->dev) {
                     // the batch's whole stdout text is composed on the device and DMA'd into the staging buffer the input came from
-                    mp_format_params F; F.top = top; F.megapathMode = opt.megapathMode; F.ignoreComments = opt.ignoreComments;
+                    mp_format_params F; F.top = top; F.megapathMode = opt.megapathMode; F.ignoreComments = step.ignoreComments;
                     uint64_t ob = 0;
                     const double tf0 = now_s();
                     int rc = mp_format_fastq(gpu, &F, &ob);
                     const double tf1 = now_s();
+                    if (!last) {                                    // stays on the device for the next step's mp_fastq_chain
+                        if (rc) { j->log += std::string(mp_last_error()) + "\n"; j->failed = true; }
+                        fmtPrev = ob;
+                    } else {
                     if (!rc && ob > j->raw.bytes1 + j->raw.bytes2) {       // later buffers are sized for this growth (+ 25 %)
                         const size_t g = (size_t)((ob - j->raw.bytes1 - j->raw.bytes2) / std::max<uint32_t>(numQueries, 1u)), want = g + g / 4 + 16;
                         size_t cur = growPerRead.load();
@@ -1614,9 +1744,11 @@ int main(int argc, char **argv)
                     if (rc) { j->log += std::string(mp_last_error()) + "\n"; j->failed = true; }
                     else if (opt.lsam < 0) j->outBytes = ob;
                     else lsam_pieces(j->raw.pin, (size_t)ob, fmtThreads, opt.lsam != 0, j->fqParts);      // -lsam: rewritten by the -T threads
+                    }
                 } else if (opt.megapathMode || opt.outputBAM) {
                     ReadBatch &b = *j->b;
-                    oc.b = &b;
+                    OutCtx oc = step.octx; oc.b = &b;
+                    const bool lsam = last && opt.lsam >= 0;        // -lsam rewrites the printed (last) step's text only
                     // Formatting is spread over the -T host threads: every chunk of pairs writes its own text / BAM records, and the
                     // chunks are concatenated in order, so the stream is the one a single thread would have produced.
                     struct Chunk { std::string fq; std::vector<uint8_t> bam, bamz; };   // bamz: the chunk's BAM records as BGZF blocks
@@ -1634,7 +1766,7 @@ int main(int argc, char **argv)
                             occ.bam = opt.outputBAM ? &capw : nullptr;
                             chunks[c].fq.reserve((size_t)(cut[c + 1] - cut[c]) * (size_t)(4 * maxLen + 160));
                             body(occ, chunks[c].fq, cut[c], cut[c + 1]);
-                            if (opt.lsam >= 0 && !chunks[c].fq.empty()) { std::string ls; fastq_chunk_to_lsam(chunks[c].fq.data(), chunks[c].fq.size(), opt.lsam != 0, ls); chunks[c].fq.swap(ls); }
+                            if (lsam && !chunks[c].fq.empty()) { std::string ls; fastq_chunk_to_lsam(chunks[c].fq.data(), chunks[c].fq.size(), opt.lsam != 0, ls); chunks[c].fq.swap(ls); }
                             if (!deviceBgzf && !chunks[c].bam.empty()) { BgzfWriter::compress_all(chunks[c].bam.data(), chunks[c].bam.size(), chunks[c].bamz); std::vector<uint8_t>().swap(chunks[c].bam); }
                         });
                         if (deviceBgzf) {
@@ -1646,7 +1778,7 @@ int main(int argc, char **argv)
                             auto flush = [&]() {
                                 uint64_t ob = 0;
                                 rc = mp_bgzf_compress(gpu, (const uint8_t *)sp.first, fill, (uint8_t *)dp.first, dp.second, &ob);
-                                if (!rc) j->bam[bamSlot].insert(j->bam[bamSlot].end(), (const uint8_t *)dp.first, (const uint8_t *)dp.first + ob);
+                                if (!rc) j->bam[3 * k + bamSlot].insert(j->bam[3 * k + bamSlot].end(), (const uint8_t *)dp.first, (const uint8_t *)dp.first + ob);
                                 fill = 0;
                             };
                             for (Chunk &c : chunks)
@@ -1661,7 +1793,7 @@ int main(int argc, char **argv)
                             tCmp += now_s() - tc0;
                         }
                         // the chunks stay separate strings (no 700 MB concatenation): the writer emits them in this order
-                        for (Chunk &c : chunks) { j->fqParts.emplace_back(std::move(c.fq)); j->bam[bamSlot].insert(j->bam[bamSlot].end(), c.bamz.begin(), c.bamz.end()); }
+                        for (Chunk &c : chunks) { j->fqParts.emplace_back(std::move(c.fq)); j->bam[3 * k + bamSlot].insert(j->bam[3 * k + bamSlot].end(), c.bamz.begin(), c.bamz.end()); }
                     };
                     std::vector<uint8_t> done(nPairs, 0);
                     for (int which = 0; which < 2; ++which) {
@@ -1707,7 +1839,8 @@ int main(int argc, char **argv)
                 mp_results_release(gpu, &R);
             }
             if (timing) fprintf(stderr, "[timing] batch %llu: upload %.3f align %.3f (lib wall %.3f) format %.3f (bgzf compress %.3f) release %.3f s; started at %.3f\n",
-                                (unsigned long long)j->seq, tUp - ts, tAl - tUp, libWallMs / 1e3, tFmt - tAl, tCmp, now_s() - tFmt, ts - t0);
+                                (unsigned long long)j->seq, tUp - tk, tAl - tUp, libWallMs / 1e3, tFmt - tAl, tCmp, now_s() - tFmt, tk - t0);
+            }
             j->alignSeconds = now_s() - ts;
             std::lock_guard<std::mutex> lk(mu);
             if (j->b) { batchPool.push_back(j->b); j->b = nullptr; }   // the text output no longer refers to the batch
@@ -1715,11 +1848,11 @@ int main(int argc, char **argv)
         }
     };
     std::vector<std::thread> workers;
-    for (mp_context *c : contexts) workers.emplace_back(worker, c);
+    for (size_t c = 0; c < contexts.size(); ++c) workers.emplace_back(worker, contexts[c], contextGpu[c]);
 
     // ---- ordered writer ----
     double totalLoad = 0, totalAlign = 0; const double tLoop0 = now_s();
-    uint64_t totalPairsAligned = 0, next = 0; bool failed = false, announced = false;
+    uint64_t next = 0; bool failed = false, announced = false;
     double writeSeconds = 0; uint64_t writtenBytes = 0;
     for (;;) {
         Job *j = nullptr;
@@ -1739,25 +1872,30 @@ int main(int argc, char **argv)
         for (const std::string &part : j->fqParts) if (!part.empty()) { fwrite(part.data(), 1, part.size(), stdout); writtenBytes += part.size(); }
         pin_give(j->raw.pin, j->raw.pinCap); j->raw.pin = nullptr;
         writeSeconds += now_s() - tw0;
-        if (opt.outputBAM) { bamDP.write_blocks(j->bam[0]); bamGout.write_blocks(j->bam[1]); bamUnpair.write_blocks(j->bam[2]); }
+        for (size_t k = 0; opt.outputBAM && k < K && j->bam.size() == 3 * K; ++k) {
+            ChainStep &c = *steps[k];
+            c.bamDP.write_blocks(j->bam[3 * k]); c.bamGout.write_blocks(j->bam[3 * k + 1]); c.bamUnpair.write_blocks(j->bam[3 * k + 2]);
+        }
         fprintf(stderr, "[Main] Elapsed time : %9.4f seconds\n\n", j->alignSeconds);
         if (getenv("MP_DRIVER_TIMING")) fprintf(stderr, "[timing] batch %llu written at %.3f\n", (unsigned long long)j->seq, now_s() - t0);
-        totalLoad += j->loadSeconds; totalAlign += j->alignSeconds; totalPairsAligned += j->pairsAligned;
+        totalLoad += j->loadSeconds; totalAlign += j->alignSeconds; for (size_t k = 0; k < j->pairsAligned.size(); ++k) steps[k]->pairsAligned += j->pairsAligned[k];
         delete j; ++next;
     }
     reader.join();
     for (std::thread &t : workers) t.join();
     fflush(stdout);
-    if (opt.outputBAM) { bamDP.close(); bamGout.close(); bamUnpair.close(); }
+    for (auto &c : steps) if (opt.outputBAM) { c->bamDP.close(); c->bamGout.close(); c->bamUnpair.close(); }
     const double tLoop1 = now_s();                                  // every batch aligned and written: the end of the batch loop
     for (ReadBatch *rb : batchPool) delete rb;
     // (the staging buffers are left to the end of the process: unlocking gigabytes page by page here would only delay the exit)
     if (failed) return 1;
     if (getenv("MP_DRIVER_TIMING")) fprintf(stderr, "[timing] writer: %.3f s in stdout writes, %.1f MB; batch loop from %.3f to %.3f\n", writeSeconds, writtenBytes / 1e6, tLoop0 - t0, tLoop1 - t0);
-    fprintf(stderr, "[Main] Overall number of pairs of reads aligned: %llu\n", (unsigned long long)totalPairsAligned);
+    if (!chained) fprintf(stderr, "[Main] Overall number of pairs of reads aligned: %llu\n", (unsigned long long)steps[0]->pairsAligned);
+    else for (size_t k = 0; k < K; ++k) fprintf(stderr, "[Main] Overall number of pairs of reads aligned (chunk %zu, index %s): %llu\n", k, steps[k]->index.c_str(), (unsigned long long)steps[k]->pairsAligned);
     fprintf(stderr, "[Main] Overall read load time : %9.4f seconds\n", totalLoad);
     fprintf(stderr, "[Main] Overall alignment time (excl. read loading) : %9.4f seconds\n", tLoop1 - tLoop0);
     for (size_t k = contexts.size(); k-- > 0;) mp_destroy(contexts[k]);
+    for (size_t k = 0; chained && k < K; ++k) for (mp_context *o : steps[k]->owners) mp_destroy(o);      // (unchained, the owners are contexts)
     fprintf(stderr, "[Main] Overall running time: %f\n", now_s() - t0);
     return 0;
 }

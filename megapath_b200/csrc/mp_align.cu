@@ -382,8 +382,32 @@ extern "C" void mp_destroy(mp_context *ctx)
 }
 extern "C" int mp_index_load(mp_context *ctx, const char *prefix)
 {
+    return mp_index_load_budget(ctx, prefix, 0);
+}
+extern "C" int mp_index_load_budget(mp_context *ctx, const char *prefix, uint64_t maxBytes)
+{
     if (!ctx || !prefix) { mp_set_error("mp_index_load: null argument"); return MP_ERR_ARG; }
+    if (ctx->sharedIndex) { mp_set_error("mp_index_load: the context shares another context's index (mp_clone)"); return MP_ERR_STATE; }
+    ctx->hbmBudget = maxBytes;
     return mpi_load(ctx, prefix);
+}
+// Points a clone at another owner's resident index, K-mer filter and annotation.  A filter the clone built for itself is released.
+extern "C" int mp_index_bind(mp_context *ctx, mp_context *owner)
+{
+    if (!ctx || !owner) { mp_set_error("mp_index_bind: null argument"); return MP_ERR_ARG; }
+    if (!ctx->sharedIndex) { mp_set_error("mp_index_bind: the context is not a clone (mp_clone)"); return MP_ERR_STATE; }
+    if (owner->sharedIndex || !owner->hasIndex || owner->device != ctx->device) {
+        mp_set_error("mp_index_bind: the owner must own a resident index on the clone's device"); return MP_ERR_ARG;
+    }
+    MP_CUDA(cudaSetDevice(ctx->device));
+    MP_CUDA(cudaStreamSynchronize(ctx->stream));              // nothing of this context may still read the previous index
+    if (ctx->dBloom.cap) ctx->dBloom.release(); else ctx->dBloom.p = nullptr;
+    ctx->ix = owner->ix; ctx->saInterval = owner->saInterval; ctx->hbmBytes = owner->hbmBytes;
+    ctx->bloomK = owner->bloomK; ctx->bloomStride = owner->bloomStride; ctx->bloomSeedMin = owner->bloomSeedMin; ctx->bloomWords = owner->bloomWords; ctx->bloomFor = owner->bloomFor;
+    ctx->dBloom.p = owner->dBloom.p; ctx->dBloom.cap = 0;
+    ctx->annSrc = owner;
+    ctx->seeded = false; ctx->resValid = false;
+    return 0;
 }
 extern "C" int mp_index_info(mp_context *ctx, uint64_t *textLength, uint64_t *inverseSa0, uint64_t cumFreq[5], uint64_t *hbmBytes)
 {

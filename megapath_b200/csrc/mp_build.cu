@@ -168,7 +168,7 @@ extern "C" int mp_index_build(mp_context *ctx, const uint8_t *text2bit, uint64_t
     const bool large = n + 1 >= 0xFFFFFFF0ull || (getenv("MP_BUILD_LARGE") && getenv("MP_BUILD_LARGE")[0] == '1');
     MP_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    ctx->hasIndex = false; ctx->bloomK = 0; ctx->ix.sa32 = nullptr; ctx->dSa32.release();
+    ctx->hasIndex = false; ctx->bloomK = 0; ctx->ix.sa32 = nullptr; ctx->dSa32.release(); ctx->hbmBudget = 0;
     const uint64_t N = n + 1;                       // suffixes incl. the '$' suffix
     const uint64_t pacBytes = (n + 3) / 4;
     // ---- packed text (kept as the index's .pac) ----

@@ -126,6 +126,7 @@ struct mp_context {
     DevBuf dBlocks, dSuper, dSa, dSa32, dSa40Lo, dSa40Hi, dLkt, dPac, dBloom;
     int bloomK = 0, bloomStride = 1, bloomSeedMin = 0; uint64_t bloomWords = 0; const void *bloomFor = nullptr;   // K-mer presence filter (mp_seed.cu)
     uint64_t hbmBytes = 0;
+    uint64_t hbmBudget = 0;                 // mp_index_load_budget: bound of the resident index + K-mer filter (0 = no bound)
     std::vector<uint64_t> hSa; uint64_t saInterval = 16;   // kept for mp_index_save
     // batch
     bool hasBatch = false, seeded = false;
@@ -161,6 +162,7 @@ struct mp_context {
     bool fqBatch = false;                   // the uploaded batch came through mp_fastq_upload: text + record index are resident
     uint64_t fqBase[2] = { 0, 0 }, fqBytes[2] = { 0, 0 };
     DevBuf dFqText, dFqCnt, dFqCntPos, dFqLines, dFqRec, dFqFlags;
+    const mp_context *annSrc = nullptr;     // mp_index_bind: the owner whose annotation mp_format_fastq reads (else this context's own)
     bool hasAnn = false; uint64_t annDnaLength = 0; uint32_t annGridEntries = 0, annNumTr = 0, annNumSeq = 0;
     DevBuf dAnnGrid, dAnnTrStart, dAnnTrChr, dAnnNames, dAnnNameOff;
     DevBuf dFmtKeys, dFmtGroups, dFmtRecLen, dFmtTail, dFmtTailText, dFmtSeg, dFmtDst, dFmtLen, dFmtOff, dFmtOut;
@@ -170,9 +172,12 @@ struct mp_context {
     DevBuf dBgzfIn, dBgzfSlots, dBgzfOut, dBgzfSizes, dBgzfOffs, dBgzfScratch;
 };
 
+// DevBuf::reserve(bytes) allocates bytes + bytes / 8 + 256: the largest request whose allocation stays within `room` bytes
+static inline uint64_t devbuf_fit(uint64_t room) { return room > 256 ? (room - 256) / 9 * 8 : 0; }
 // mp_index.cu
 int mpi_load(mp_context *ctx, const char *prefix);
-int mpi_finish_sa(mp_context *ctx);      // texts >= 2^32: 40-bit SA samples at the densest rate the HBM budget allows
+int mpi_finish_sa(mp_context *ctx);
+uint64_t mpi_index_bytes(const mp_context *ctx);      // texts >= 2^32: 40-bit SA samples at the densest rate the HBM budget allows
 int mpi_build_from_words(mp_context *ctx, const uint32_t *hBwtWords, uint64_t n, uint64_t inverseSa0, const uint64_t cum[5]);
 // mp_seed.cu
 int mps_seed_pairs(mp_context *ctx, const mp_align_params *P);

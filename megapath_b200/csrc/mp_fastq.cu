@@ -389,6 +389,59 @@ __global__ void k_fmt_write(FmtView V, const uint32_t *__restrict__ tailLen, con
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// chain: the formatted text of a batch -> the next chunk's two mate texts (the deinterleave rewrite)
+// Record r of the formatted text is lines 4r .. 4r+3 of lineEnd and belongs to mate (r & 1) + 1, pair r >> 1.  Its header
+// "@NAME<blanks>TAIL" becomes "@NAME'/<mate> TAIL": NAME is the first blank-delimited word after '@', NAME' is NAME without one trailing
+// "/1" or "/2", TAIL is the rest of the line after the blanks that follow NAME ("@NAME'/<mate>" alone when there is none).  The other
+// three lines are copied as they are (the formatter's third line is always "+").
+struct ChainHdr { uint32_t name, nameLen, comm, commLen; };
+__device__ __forceinline__ ChainHdr chain_header(const char *text, uint32_t s0, uint32_t e0)
+{
+    ChainHdr h;
+    uint32_t q = s0 + 1;
+    while (q < e0 && fq_isspace((unsigned char)text[q])) ++q;
+    h.name = q;
+    while (q < e0 && !fq_isspace((unsigned char)text[q])) ++q;
+    h.nameLen = q - h.name;
+    while (q < e0 && fq_isspace((unsigned char)text[q])) ++q;
+    h.comm = q; h.commLen = e0 - q;
+    if (h.nameLen >= 2 && text[h.name + h.nameLen - 2] == '/' && (text[h.name + h.nameLen - 1] == '1' || text[h.name + h.nameLen - 1] == '2')) h.nameLen -= 2;
+    return h;
+}
+__device__ __forceinline__ uint32_t chain_rec_start(const uint32_t *L, uint32_t r) { return r ? L[4 * r - 1] + 1 : 0; }
+// one thread per record: its rewritten size, stored mate-major (mate 1's pairs, then mate 2's) for one scan over both mates
+__global__ void k_chain_measure(const char *__restrict__ text, const uint32_t *__restrict__ L, uint32_t nReads, unsigned long long *__restrict__ len)
+{
+    const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= nReads) return;
+    const uint32_t s0 = chain_rec_start(L, r), e0 = L[4 * r];
+    const ChainHdr h = chain_header(text, s0, e0);
+    len[(uint64_t)(r & 1u) * (nReads >> 1) + (r >> 1)] = 1 + h.nameLen + 2 + (h.commLen ? 1 + h.commLen : 0) + 1 + (L[4 * r + 3] - e0);
+}
+// one warp per record: off = the scan of k_chain_measure's sizes; mate 2's text starts at base1
+__global__ void k_chain_write(const char *__restrict__ text, const uint32_t *__restrict__ L, uint32_t nReads, const unsigned long long *__restrict__ off,
+                              uint64_t base1, char *__restrict__ out)
+{
+    const uint32_t lane = threadIdx.x & 31u, nPairs = nReads >> 1;
+    const uint32_t nWarps = (gridDim.x * blockDim.x) >> 5;
+    const unsigned long long off2 = off[nPairs];
+    for (uint32_t r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < nReads; r += nWarps) {
+        const uint32_t m = r & 1u, s0 = chain_rec_start(L, r), e0 = L[4 * r];
+        const ChainHdr h = chain_header(text, s0, e0);
+        char *w = out + (m ? base1 + off[nPairs + (r >> 1)] - off2 : off[r >> 1]);
+        if (lane == 0) w[0] = '@';
+        warp_copy<false>(w + 1, text + h.name, h.nameLen, lane);
+        w += 1 + h.nameLen;
+        if (lane == 0) { w[0] = '/'; w[1] = (char)('1' + m); if (h.commLen) w[2] = ' '; }
+        w += h.commLen ? 3 : 2;
+        warp_copy<false>(w, text + h.comm, h.commLen, lane);
+        w += h.commLen;
+        if (lane == 0) w[0] = '\n';
+        warp_copy<false>(w + 1, text + e0 + 1, L[4 * r + 3] - e0, lane);
+    }
+}
+
 int scan_any(mp_context *ctx, const uint32_t *in, uint32_t *out, uint64_t n)
 {
     size_t tb = 0;
@@ -416,31 +469,32 @@ extern "C" void *mp_host_alloc(uint64_t bytes)
 }
 extern "C" void mp_host_free(void *p) { if (p) cudaFreeHost(p); }
 
-extern "C" int mp_fastq_upload(mp_context *ctx, const char *text1, uint64_t bytes1, const char *text2, uint64_t bytes2,
-                               uint32_t nPairs, uint32_t wpq, uint32_t maxReadLength, const uint32_t **readLengths)
+static int fq_check_args(const char *who, uint32_t nPairs, uint32_t wpq, uint32_t maxReadLength)
 {
-    if (!ctx || !text1 || !text2 || nPairs == 0 || wpq == 0 || maxReadLength < 2) { mp_set_error("mp_fastq_upload: bad argument"); return MP_ERR_ARG; }
-    if (maxReadLength - 1 > 16u * wpq) { mp_set_error("mp_fastq_upload: reads of up to %u bases do not fit %u words per query", maxReadLength - 1, wpq); return MP_ERR_ARG; }
-    if (nPairs > (1u << 29)) { mp_set_error("mp_fastq_upload: too many pairs"); return MP_ERR_ARG; }
+    if (nPairs == 0 || wpq == 0 || maxReadLength < 2) { mp_set_error("%s: bad argument", who); return MP_ERR_ARG; }
+    if (maxReadLength - 1 > 16u * wpq) { mp_set_error("%s: reads of up to %u bases do not fit %u words per query", who, maxReadLength - 1, wpq); return MP_ERR_ARG; }
+    if (nPairs > (1u << 29)) { mp_set_error("%s: too many pairs", who); return MP_ERR_ARG; }
+    return 0;
+}
+
+// Everything after the text is in dFqText (mate 1 at 0, mate 2 at base1): the record index, the checks, lengths and 2-bit rows, and the
+// batch state.  mp_fastq_upload and mp_fastq_chain share it.
+static int fq_ingest(mp_context *ctx, const char *who, uint64_t base1, uint64_t bytes1, uint64_t bytes2, uint32_t nPairs, uint32_t wpq,
+                     uint32_t maxReadLength, const uint32_t **readLengths)
+{
     // 32-bit offsets inside a mate's text; every record has at least 4 newlines + '@' + '+' + a base + a quality
-    if (bytes1 >= 0xFFFFFFF0ull || bytes2 >= 0xFFFFFFF0ull || bytes1 < 8ull * nPairs || bytes2 < 8ull * nPairs ||
-        text1[bytes1 - 1] != '\n' || text2[bytes2 - 1] != '\n') {
-        mp_set_error("mp_fastq_upload: not strict four-line FASTQ"); return MP_ERR_FORMAT;
+    if (bytes1 >= 0xFFFFFFF0ull || bytes2 >= 0xFFFFFFF0ull || bytes1 < 8ull * nPairs || bytes2 < 8ull * nPairs) {
+        mp_set_error("%s: not strict four-line FASTQ", who); return MP_ERR_FORMAT;
     }
-    MP_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    ctx->fqBatch = false; ctx->fmtReady = false;              // the resident text of the previous batch is overwritten from here on
     const uint32_t nReads = 2 * nPairs, maxLines = 4 * nPairs;
-    const uint64_t base1 = (bytes1 + 63) & ~63ull, total = base1 + bytes2;
     const uint64_t nT[2] = { (bytes1 + FQ_PIECE - 1) / FQ_PIECE, (bytes2 + FQ_PIECE - 1) / FQ_PIECE };
     const uint64_t cntOff1 = nT[0] + 1;
-    if (ctx->dFqText.reserve(total + 64) || ctx->dFqCnt.reserve((nT[0] + nT[1] + 2) * 4) || ctx->dFqCntPos.reserve((nT[0] + nT[1] + 2) * 4) ||
+    if (ctx->dFqCnt.reserve((nT[0] + nT[1] + 2) * 4) || ctx->dFqCntPos.reserve((nT[0] + nT[1] + 2) * 4) ||
         ctx->dFqLines.reserve((size_t)maxLines * 2 * 4) || ctx->dFqRec.reserve((size_t)nReads * sizeof(FqRec)) || ctx->dFqFlags.reserve(16)) return MP_ERR_CUDA;
     char *dText = ctx->dFqText.as<char>();
     uint32_t *dFlags = ctx->dFqFlags.as<uint32_t>();
     MP_CUDA(cudaMemsetAsync(dFlags, 0, 16, st));
-    MP_CUDA(cudaMemcpyAsync(dText, text1, bytes1, cudaMemcpyHostToDevice, st));
-    MP_CUDA(cudaMemcpyAsync(dText + base1, text2, bytes2, cudaMemcpyHostToDevice, st));
     uint32_t totals[2] = { 0, 0 };
     for (int m = 0; m < 2; ++m) {
         const char *t = dText + (m ? base1 : 0);
@@ -456,7 +510,7 @@ extern "C" int mp_fastq_upload(mp_context *ctx, const char *text1, uint64_t byte
     MP_CUDA(cudaGetLastError());
     MP_CUDA(cudaStreamSynchronize(st));
     if (flags[0] || totals[0] != maxLines || totals[1] != maxLines) {
-        mp_set_error("mp_fastq_upload: not strict four-line FASTQ (%u / %u lines for %u records%s)", totals[0], totals[1], nPairs, flags[0] ? ", CR or NUL bytes" : "");
+        mp_set_error("%s: not strict four-line FASTQ (%u / %u lines for %u records%s)", who, totals[0], totals[1], nPairs, flags[0] ? ", CR or NUL bytes" : "");
         return MP_ERR_FORMAT;
     }
     // the record views may overwrite the previous batch's only now: nothing has been consumed before this point
@@ -469,7 +523,7 @@ extern "C" int mp_fastq_upload(mp_context *ctx, const char *text1, uint64_t byte
     MP_CUDA(cudaStreamSynchronize(st));
     if (flags[0] & 2u) {
         ctx->hasBatch = false; ctx->fqBatch = false;          // dLens was overwritten
-        mp_set_error("mp_fastq_upload: not strict four-line FASTQ (a record is not '@' / bases / '+' / qualities of the same length)");
+        mp_set_error("%s: not strict four-line FASTQ (a record is not '@' / bases / '+' / qualities of the same length)", who);
         return MP_ERR_FORMAT;
     }
     MP_CUDA(cudaMemsetAsync(ctx->dReads.p, 0, rowBytes + 64, st));
@@ -485,6 +539,66 @@ extern "C" int mp_fastq_upload(mp_context *ctx, const char *text1, uint64_t byte
     ctx->fqBatch = true; ctx->fqBase[0] = 0; ctx->fqBase[1] = base1; ctx->fqBytes[0] = bytes1; ctx->fqBytes[1] = bytes2;
     ctx->resValid = false; ctx->fmtReady = false;
     return 0;
+}
+
+extern "C" int mp_fastq_upload(mp_context *ctx, const char *text1, uint64_t bytes1, const char *text2, uint64_t bytes2,
+                               uint32_t nPairs, uint32_t wpq, uint32_t maxReadLength, const uint32_t **readLengths)
+{
+    if (!ctx || !text1 || !text2) { mp_set_error("mp_fastq_upload: bad argument"); return MP_ERR_ARG; }
+    if (int rc = fq_check_args("mp_fastq_upload", nPairs, wpq, maxReadLength)) return rc;
+    if (bytes1 == 0 || bytes2 == 0 || text1[bytes1 - 1] != '\n' || text2[bytes2 - 1] != '\n') { mp_set_error("mp_fastq_upload: not strict four-line FASTQ"); return MP_ERR_FORMAT; }
+    if (bytes1 >= 0xFFFFFFF0ull || bytes2 >= 0xFFFFFFF0ull) { mp_set_error("mp_fastq_upload: not strict four-line FASTQ"); return MP_ERR_FORMAT; }
+    MP_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    ctx->fqBatch = false; ctx->fmtReady = false;              // the resident text of the previous batch is overwritten from here on
+    const uint64_t base1 = (bytes1 + 63) & ~63ull;
+    if (ctx->dFqText.reserve(base1 + bytes2 + 64)) return MP_ERR_CUDA;
+    MP_CUDA(cudaMemcpyAsync(ctx->dFqText.p, text1, bytes1, cudaMemcpyHostToDevice, st));
+    MP_CUDA(cudaMemcpyAsync(ctx->dFqText.as<char>() + base1, text2, bytes2, cudaMemcpyHostToDevice, st));
+    return fq_ingest(ctx, "mp_fastq_upload", base1, bytes1, bytes2, nPairs, wpq, maxReadLength, readLengths);
+}
+
+// The formatted text (dFmtOut) -> the deinterleave rewrite into the two mate texts of dFqText -> fq_ingest.  The formatted text is left
+// as it is, so that after MP_ERR_FORMAT mp_format_fetch still returns it.
+extern "C" int mp_fastq_chain(mp_context *ctx, uint32_t wpq, uint32_t maxReadLength, const uint32_t **readLengths)
+{
+    if (!ctx) { mp_set_error("mp_fastq_chain: bad argument"); return MP_ERR_ARG; }
+    if (!ctx->fmtReady) { mp_set_error("mp_fastq_chain: no formatted batch (call mp_format_fastq first)"); return MP_ERR_STATE; }
+    const uint32_t nPairs = ctx->nReads / 2, nReads = ctx->nReads, maxLines = 8 * nPairs;
+    if (int rc = fq_check_args("mp_fastq_chain", nPairs, wpq, maxReadLength)) return rc;
+    MP_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const char *src = ctx->dFmtOut.as<char>();
+    const uint64_t bytes = ctx->fmtBytes, nT = (bytes + FQ_PIECE - 1) / FQ_PIECE;
+    // the formatted text's line index in the ingest's own scratch (fq_ingest rebuilds it for the mate texts afterwards)
+    if (ctx->dFqCnt.reserve((nT + 1) * 4) || ctx->dFqCntPos.reserve((nT + 1) * 4) || ctx->dFqLines.reserve((size_t)maxLines * 4) || ctx->dFqFlags.reserve(16) ||
+        ctx->dFmtLen.reserve(((size_t)2 * nPairs + 1) * 8) || ctx->dFmtOff.reserve(((size_t)2 * nPairs + 1) * 8)) return MP_ERR_CUDA;
+    uint32_t *cnt = ctx->dFqCnt.as<uint32_t>(), *pos = ctx->dFqCntPos.as<uint32_t>(), *L = ctx->dFqLines.as<uint32_t>();
+    (++g_mp_launches), k_fq_count<<<(unsigned)((nT + 1 + 255) / 256), 256, 0, st>>>(src, bytes, cnt, ctx->dFqFlags.as<uint32_t>());
+    if (scan_any(ctx, cnt, pos, nT + 1)) return MP_ERR_CUDA;
+    (++g_mp_launches), k_fq_lines<<<(unsigned)((nT + 255) / 256), 256, 0, st>>>(src, bytes, pos, maxLines, L);
+    uint32_t lines = 0;
+    MP_CUDA(cudaMemcpyAsync(&lines, pos + nT, 4, cudaMemcpyDeviceToHost, st));
+    MP_CUDA(cudaStreamSynchronize(st));
+    if (lines != maxLines) { mp_set_error("mp_fastq_chain: the formatted text has %u lines for %u pairs", lines, nPairs); return MP_ERR_FORMAT; }
+    // sizes (dFmtLen, dFmtOff: the formatter's scratch, free once its text is written)
+    unsigned long long *len = ctx->dFmtLen.as<unsigned long long>(), *off = ctx->dFmtOff.as<unsigned long long>();
+    MP_CUDA(cudaMemsetAsync(len + 2 * (size_t)nPairs, 0, 8, st));
+    (++g_mp_launches), k_chain_measure<<<(nReads + 255) / 256, 256, 0, st>>>(src, L, nReads, len);
+    if (scan_any(ctx, len, off, 2ull * nPairs + 1)) return MP_ERR_CUDA;
+    unsigned long long tot[2] = { 0, 0 };
+    MP_CUDA(cudaMemcpyAsync(&tot[0], off + nPairs, 8, cudaMemcpyDeviceToHost, st));
+    MP_CUDA(cudaMemcpyAsync(&tot[1], off + 2 * (size_t)nPairs, 8, cudaMemcpyDeviceToHost, st));
+    MP_CUDA(cudaGetLastError());
+    MP_CUDA(cudaStreamSynchronize(st));
+    const uint64_t bytes1 = tot[0], bytes2 = tot[1] - tot[0], base1 = (bytes1 + 63) & ~63ull;
+    if (bytes1 >= 0xFFFFFFF0ull || bytes2 >= 0xFFFFFFF0ull) { mp_set_error("mp_fastq_chain: a mate's text exceeds 4 GB"); return MP_ERR_FORMAT; }
+    ctx->fqBatch = false;                                     // the resident text of this batch is overwritten from here on
+    if (ctx->dFqText.reserve(base1 + bytes2 + 64)) return MP_ERR_CUDA;
+    int dev = 0, sms = 148; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    (++g_mp_launches), k_chain_write<<<(unsigned)sms * 8, 256, 0, st>>>(src, L, nReads, off, base1, ctx->dFqText.as<char>());
+    MP_CUDA(cudaGetLastError());
+    return fq_ingest(ctx, "mp_fastq_chain", base1, bytes1, bytes2, nPairs, wpq, maxReadLength, readLengths);
 }
 
 // Sizes the ingest / egress buffers of a context before the batch loop, like mp_reserve does for the alignment buffers (the first
@@ -523,7 +637,7 @@ extern "C" int mp_annotation_upload(mp_context *ctx, const mp_annotation *a)
     if (nameBytes) MP_CUDA(cudaMemcpy(ctx->dAnnNames.p, a->names, nameBytes, cudaMemcpyHostToDevice));
     MP_CUDA(cudaMemcpy(ctx->dAnnNameOff.p, a->nameOffsets, ((size_t)a->numSeq + 1) * 8, cudaMemcpyHostToDevice));
     ctx->annDnaLength = a->dnaLength; ctx->annGridEntries = a->gridEntries; ctx->annNumTr = a->numTranslate; ctx->annNumSeq = a->numSeq;
-    ctx->hasAnn = true;
+    ctx->hasAnn = true; ctx->annSrc = nullptr;
     return 0;
 }
 
@@ -531,7 +645,8 @@ extern "C" int mp_format_fastq(mp_context *ctx, const mp_format_params *F, uint6
 {
     if (!ctx || !F || !bytes) { mp_set_error("mp_format_fastq: null argument"); return MP_ERR_ARG; }
     if (F->megapathMode != 1 && F->megapathMode != 2) { mp_set_error("mp_format_fastq: megapathMode must be 1 (-F) or 2 (-P)"); return MP_ERR_ARG; }
-    if (!ctx->hasAnn || !ctx->fqBatch || !ctx->resValid) {
+    const mp_context *an = ctx->annSrc ? ctx->annSrc : ctx;     // a bound clone reads its owner's annotation (mp_index_bind)
+    if (!an->hasAnn || !ctx->fqBatch || !ctx->resValid) {
         mp_set_error("mp_format_fastq: needs mp_annotation_upload, a batch from mp_fastq_upload and its mp_align_pairs results"); return MP_ERR_STATE;
     }
     MP_CUDA(cudaSetDevice(ctx->device));
@@ -548,8 +663,8 @@ extern "C" int mp_format_fastq(mp_context *ctx, const mp_format_params *F, uint6
     uint32_t *g = ctx->dFmtGroups.as<uint32_t>();
     uint32_t *pStart = g, *pEnd = g + nPairs, *rStart = g + 2 * (size_t)nPairs, *rEnd = g + 3 * (size_t)nPairs, *sStart = g + 4 * (size_t)nPairs, *sEnd = sStart + nReads;
     MP_CUDA(cudaMemsetAsync(g, 0, nGroups * 4, st));
-    AnnDev A = { ctx->dAnnGrid.as<uint32_t>(), ctx->dAnnTrStart.as<uint64_t>(), ctx->dAnnTrChr.as<uint32_t>(), ctx->dAnnNames.as<char>(), ctx->dAnnNameOff.as<uint64_t>(),
-                 ctx->annGridEntries };
+    AnnDev A = { an->dAnnGrid.as<uint32_t>(), an->dAnnTrStart.as<uint64_t>(), an->dAnnTrChr.as<uint32_t>(), an->dAnnNames.as<char>(), an->dAnnNameOff.as<uint64_t>(),
+                 an->annGridEntries };
     const uint32_t *lens = ctx->dLens.as<uint32_t>();
     if (nP) (++g_mp_launches), k_fmt_pair_keys<<<(unsigned)((nP + 127) / 128), 128, 0, st>>>(ctx->dRes2.as<mp_pair_result>(), (uint32_t)nP, lens, A, F->megapathMode, kP1, kP2, pStart, pEnd);
     if (nR) (++g_mp_launches), k_fmt_pair_keys<<<(unsigned)((nR + 127) / 128), 128, 0, st>>>(ctx->dRsOut.as<mp_pair_result>(), (uint32_t)nR, lens, A, F->megapathMode, kR1, kR2, rStart, rEnd);

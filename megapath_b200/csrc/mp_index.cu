@@ -140,23 +140,34 @@ __global__ void k_sa40_build(MpIndexView ix, uint32_t *__restrict__ lo, uint8_t 
     lo[i] = (uint32_t)v; hi[i] = (uint8_t)(v >> 32);
 }
 
+// bytes of the resident index this context owns (the K-mer filter is counted by mp_index_prepare)
+uint64_t mpi_index_bytes(const mp_context *ctx)
+{
+    return ctx->dBlocks.cap + ctx->dSuper.cap + ctx->dSa.cap + ctx->dSa32.cap + ctx->dSa40Lo.cap + ctx->dSa40Hi.cap + ctx->dLkt.cap + ctx->dPac.cap;
+}
+static uint64_t devbuf_bytes(uint64_t bytes) { return bytes + bytes / 8 + 256; }     // what DevBuf::reserve(bytes) allocates
+
 // Called once the u64 samples (ctx->dSa, ix.saShift) are resident.  Texts shorter than 2^32 keep them (the dense u32 array is built
 // by the callers); longer texts get 40-bit samples at the densest rate whose arrays fit 35 % of the free HBM -- every SA index
 // when possible (8 Gbp: 40 GB), so that an SA lookup is two small gathers instead of an LF walk -- and the u64 array is released.
+// With an HBM budget (mp_index_load_budget) and no dense u32 array, any text gets the densest 40-bit samples that keep the index
+// within the budget, or keeps the file's samples.
 // MP_DENSE_SA=0 keeps the file's samples; MP_SA40=<shift> forces the 40-bit arrays at that shift whatever the text length (tests).
 int mpi_finish_sa(mp_context *ctx)
 {
     ctx->ix.sa40lo = nullptr; ctx->ix.sa40hi = nullptr; ctx->dSa40Lo.release(); ctx->dSa40Hi.release();
-    const uint64_t n = ctx->ix.n;
+    const uint64_t n = ctx->ix.n, budget = ctx->hbmBudget;
     const char *dense = getenv("MP_DENSE_SA"), *force = getenv("MP_SA40");
     if (dense && dense[0] == '0') return 0;
     if (ctx->ix.sa32) return 0;
-    if (!force && n + 1 < 0xFFFFFFF0ull) return 0;
+    if (!force && !budget && n + 1 < 0xFFFFFFF0ull) return 0;
+    const uint64_t rest = mpi_index_bytes(ctx) - ctx->dSa.cap;      // what stays resident beside the 40-bit arrays
     size_t freeB = 0, totalB = 0; cudaMemGetInfo(&freeB, &totalB);
     for (uint32_t sh = 0; sh <= ctx->ix.saShift; ++sh) {
         if (force ? sh != (uint32_t)atoi(force) : (sh == ctx->ix.saShift && sh > 0)) continue;
         const uint64_t cnt = (n >> sh) + 1;
-        if (!force && (double)cnt * 5.0 > 0.35 * (double)freeB) continue;
+        if (!force && budget && rest + devbuf_bytes(cnt * 4) + devbuf_bytes(cnt) > budget) continue;
+        if (!force && !budget && (double)cnt * 5.0 > 0.35 * (double)freeB) continue;
         if (ctx->dSa40Lo.reserve(cnt * 4) || ctx->dSa40Hi.reserve(cnt)) return MP_ERR_CUDA;
         (++g_mp_launches), k_sa40_build<<<(unsigned)((cnt + 255) / 256), 256>>>(ctx->ix, ctx->dSa40Lo.as<uint32_t>(), ctx->dSa40Hi.as<uint8_t>(), cnt, sh);
         MP_CUDA(cudaGetLastError());
@@ -249,12 +260,21 @@ int mpi_load(mp_context *ctx, const char *prefix)
         if (rc) return rc;
     }
     ctx->ix.pac = ctx->dPac.as<uint8_t>();
+    const uint64_t fixed = mpi_index_bytes(ctx), budget = ctx->hbmBudget;      // BWT blocks, LKT, text and the file's SA samples
+    if (budget && fixed > budget) {
+        DevBuf *bufs[] = { &ctx->dBlocks, &ctx->dSuper, &ctx->dSa, &ctx->dLkt, &ctx->dPac };
+        for (DevBuf *b : bufs) b->release();
+        memset(&ctx->ix, 0, sizeof ctx->ix);
+        mp_set_error("%s: the index needs %llu bytes of HBM without a dense SA, the budget is %llu", prefix, (unsigned long long)fixed, (unsigned long long)budget);
+        return MP_ERR_CAPACITY;
+    }
     // ---- dense SA: resolve every SA index once at load time (LF walks to the file's 1/16 samples) so that
     //      lookups on the hot path are a single gather.  MP_DENSE_SA=0 keeps the sampled array only. ----
     ctx->ix.sa32 = nullptr; ctx->dSa32.release();
     const char *dense = getenv("MP_DENSE_SA");
     size_t freeB = 0, totalB = 0; cudaMemGetInfo(&freeB, &totalB);
-    if (!(dense && dense[0] == '0') && !getenv("MP_SA40") && n + 1 < 0xFFFFFFF0ull && (n + 1) * 4 < freeB / 2) {
+    const bool fits = budget ? fixed + devbuf_bytes((n + 1) * 4) <= budget : (n + 1) * 4 < freeB / 2;
+    if (!(dense && dense[0] == '0') && !getenv("MP_SA40") && n + 1 < 0xFFFFFFF0ull && fits) {
         if (ctx->dSa32.reserve((n + 1) * 4)) return MP_ERR_CUDA;
         (++g_mp_launches), k_densify_sa<<<(unsigned)((n + 1 + 255) / 256), 256>>>(ctx->ix, ctx->dSa32.as<uint32_t>(), n + 1);
         MP_CUDA(cudaGetLastError());
@@ -262,7 +282,7 @@ int mpi_load(mp_context *ctx, const char *prefix)
         ctx->ix.sa32 = ctx->dSa32.as<uint32_t>();
     }
     if (int rc = mpi_finish_sa(ctx)) return rc;
-    ctx->hbmBytes = ctx->dBlocks.cap + ctx->dSuper.cap + ctx->dSa.cap + ctx->dSa32.cap + ctx->dSa40Lo.cap + ctx->dSa40Hi.cap + ctx->dLkt.cap + ctx->dPac.cap;
+    ctx->hbmBytes = mpi_index_bytes(ctx);
     ctx->hasIndex = true;
     return 0;
 }

@@ -618,6 +618,10 @@ static int ensure_bloom(mp_context *ctx, int seedMinLength)
         size_t freeB = 0, totalB = 0; cudaMemGetInfo(&freeB, &totalB);
         const uint64_t room = (uint64_t)(freeB / 3) / 8;
         if (nWords > room) nWords = room;
+        if (ctx->hbmBudget) {                            // mp_index_load_budget: what the index left of its budget, or no filter
+            const uint64_t idx = mpi_index_bytes(ctx), left = ctx->hbmBudget > idx ? devbuf_fit(ctx->hbmBudget - idx) / 8 : 0;
+            if (nWords > left) nWords = left;
+        }
         if (nWords < 1024) { ctx->bloomK = 0; return 0; }
     }
     if (ctx->sharedIndex && ctx->dBloom.cap == 0) ctx->dBloom.p = nullptr;      // a borrowed filter with another K: build our own
