@@ -218,6 +218,22 @@ int  mp_dp_batch(mp_context *ctx,
                  const uint32_t *clipLtSizes, const uint32_t *clipRtSizes,
                  int32_t mismatchScore, int32_t openGapScore);
 
+/* ---- DP on tasks the way the alignment stages run it: the window is text [refStart, refStart + refLen) of the resident index, the
+ *      read is read readID of the uploaded batch, reverse-complemented for strand 2.  Tasks with valid == 0, refLen > maxRefLen or
+ *      readLen > maxReadLen are dropped (score 0).  diag is a hint only (the read's expected window offset, -1 = none): results do
+ *      not depend on it.  Outputs as mp_dp_batch; pattern has n*(maxRefLen+maxReadLen) bytes.  For checking the stages' DP path. */
+typedef struct {
+    uint64_t refStart;
+    uint32_t refLen, readID;
+    uint16_t readLen;
+    uint8_t  strand, valid;             /* strand 1 '+', 2 '-' */
+    int32_t  cutoff;
+    int16_t  diag;
+    uint16_t reserved_;
+} mp_dp_task;
+int  mp_dp_tasks(mp_context *ctx, const mp_dp_task *tasks, uint32_t n, uint32_t maxRefLen, uint32_t maxReadLen,
+                 uint32_t clipLt, uint32_t clipRt, int32_t *scores, uint32_t *hitLocs, uint32_t *maxScoreCounts, uint8_t *pattern);
+
 /* ---- whole stage sequence for the uploaded batch: replaces soap3_dp_pair_align's engines
  *      (alignment.cpp:29-355): PairEndAlignmentEngine / SingleEndAlignmentEngine /
  *      HalfEndAlignmentEngine::performAlignment (DV-DPfunctions.h:1558-1576, 976-991, 1205-1221).

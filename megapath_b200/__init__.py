@@ -53,6 +53,8 @@ class Stats(C.Structure):
 
 SEEDPOS = np.dtype([("pos", "<u8"), ("strand_readID", "<u4"), ("paired_seedLength", "<u4")])
 CAND = np.dtype([("readIDLeft", "<u4"), ("pad", "<u4"), ("pos0", "<u8"), ("pos1", "<u8")])
+DP_TASK = np.dtype([("refStart", "<u8"), ("refLen", "<u4"), ("readID", "<u4"), ("readLen", "<u2"), ("strand", "u1"), ("valid", "u1"),
+                    ("cutoff", "<i4"), ("diag", "<i2"), ("reserved_", "<u2")], align=True)      # mp_dp_task
 PAIR_RESULT = np.dtype([
     ("readID", "<u4"), ("insertSize", "<i4"), ("algnmt_1", "<u8"), ("algnmt_2", "<u8"),
     ("score_1", "<i4"), ("score_2", "<i4"), ("editdist_1", "<i4"), ("editdist_2", "<i4"),
@@ -148,6 +150,8 @@ def lib():
         L.mp_dp_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32,
                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
                                   C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]
+        L.mp_dp_tasks.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,
+                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.mp_align_pairs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         L.mp_results_release.argtypes = [C.c_void_p, C.c_void_p]
         L.mp_last_stats.argtypes = [C.c_void_p, C.c_void_p]
@@ -489,6 +493,17 @@ class Context:
         self._check(self.L.mp_dp_batch(self.h, _ptr(packed_dna), _ptr(dna_lens), max_dna, _ptr(packed_read), _ptr(read_lens),
                                        max_read, _ptr(cutoffs), _ptr(scores), _ptr(hits), _ptr(cnts), _ptr(pats), n,
                                        _ptr(cl), _ptr(cr), mismatch, gap_open))
+        return scores, hits, cnts, pats
+
+    def dp_tasks(self, tasks, max_ref, max_read, clip_lt=130, clip_rt=130):
+        """mp_dp_tasks: tasks (numpy array of DP_TASK) against the resident index and the uploaded batch -> scores, hits, counts, patterns."""
+        tasks = np.ascontiguousarray(tasks, dtype=DP_TASK)
+        n = len(tasks)
+        scores = np.zeros(n, dtype=np.int32)
+        hits = np.zeros(n, dtype=np.uint32)
+        cnts = np.zeros(n, dtype=np.uint32)
+        pats = np.zeros((n, max_ref + max_read), dtype=np.uint8)
+        self._check(self.L.mp_dp_tasks(self.h, _ptr(tasks), n, max_ref, max_read, clip_lt, clip_rt, _ptr(scores), _ptr(hits), _ptr(cnts), _ptr(pats)))
         return scores, hits, cnts, pats
 
     # ---- whole stage sequence ----

@@ -486,26 +486,26 @@ extern "C" int mp_dp_batch(mp_context *ctx,
         }
     MP_CUDA(cudaSetDevice(ctx->device));
     const uint32_t wDNA = (maxDNALength + 15) >> 4, wRead = (maxReadLength + 15) >> 4;
-    // un-interleave into one byte per base (host side of the seam; the kernels take bytes)
-    std::vector<uint8_t> hRef((size_t)n * maxDNALength), hRead((size_t)n * maxReadLength);
+    // un-interleave into the DP kernels' packed rows: 16 bases per word, first base in the low bits (host side of the seam)
+    std::vector<uint32_t> hRef((size_t)n * wDNA), hRead((size_t)n * wRead);
     for (uint32_t t = 0; t < n; ++t) {
         size_t dT = (size_t)(t / 32) * 32 * wDNA + (t % 32), rT = (size_t)(t / 32) * 32 * wRead + (t % 32);
         for (uint32_t i = 1; i <= DNALengths[t] && i <= maxDNALength; ++i)
-            hRef[(size_t)t * maxDNALength + i - 1] = (packedDNA[dT + ((i >> 4) << 5)] >> ((15 - (i & 15)) << 1)) & 3;
+            hRef[(size_t)t * wDNA + ((i - 1) >> 4)] |= ((packedDNA[dT + ((i >> 4) << 5)] >> ((15 - (i & 15)) << 1)) & 3) << (((i - 1) & 15) << 1);
         for (uint32_t i = 1; i <= readLengths[t] && i <= maxReadLength; ++i)
-            hRead[(size_t)t * maxReadLength + i - 1] = (packedRead[rT + ((i >> 4) << 5)] >> ((15 - (i & 15)) << 1)) & 3;
+            hRead[(size_t)t * wRead + ((i - 1) >> 4)] |= ((packedRead[rT + ((i >> 4) << 5)] >> ((15 - (i & 15)) << 1)) & 3) << (((i - 1) & 15) << 1);
     }
     DevBuf dRef, dRead, dRL, dDL, dCo, dOut, dPat;
     const uint32_t patStride = maxDNALength + maxReadLength;
-    if (dRef.reserve(hRef.size()) || dRead.reserve(hRead.size()) || dRL.reserve((size_t)n * 4) || dDL.reserve((size_t)n * 4) ||
+    if (dRef.reserve(hRef.size() * 4) || dRead.reserve(hRead.size() * 4) || dRL.reserve((size_t)n * 4) || dDL.reserve((size_t)n * 4) ||
         dCo.reserve((size_t)n * 4) || dOut.reserve((size_t)n * sizeof(MpDpOut)) || dPat.reserve((size_t)n * patStride)) return MP_ERR_CUDA;
-    MP_CUDA(cudaMemcpy(dRef.p, hRef.data(), hRef.size(), cudaMemcpyHostToDevice));
-    MP_CUDA(cudaMemcpy(dRead.p, hRead.data(), hRead.size(), cudaMemcpyHostToDevice));
+    MP_CUDA(cudaMemcpy(dRef.p, hRef.data(), hRef.size() * 4, cudaMemcpyHostToDevice));
+    MP_CUDA(cudaMemcpy(dRead.p, hRead.data(), hRead.size() * 4, cudaMemcpyHostToDevice));
     MP_CUDA(cudaMemcpy(dDL.p, DNALengths, (size_t)n * 4, cudaMemcpyHostToDevice));
     MP_CUDA(cudaMemcpy(dRL.p, readLengths, (size_t)n * 4, cudaMemcpyHostToDevice));
     MP_CUDA(cudaMemcpy(dCo.p, cutoffs, (size_t)n * 4, cudaMemcpyHostToDevice));
     MpDpParams P; P.clipLt = (int)clipLt[0]; P.clipRt = (int)clipRt[0]; P.mismatch = mismatchScore; P.open = openGapScore;
-    int rc = mpd_run_explicit(ctx, dRef.as<uint8_t>(), dDL.as<uint32_t>(), maxDNALength, dRead.as<uint8_t>(), dRL.as<uint32_t>(),
+    int rc = mpd_run_explicit(ctx, dRef.as<uint32_t>(), dDL.as<uint32_t>(), maxDNALength, dRead.as<uint32_t>(), dRL.as<uint32_t>(),
                               maxReadLength, dCo.as<int32_t>(), n, P, dOut.as<MpDpOut>(), dPat.as<uint8_t>(), patStride);
     if (rc) return rc;
     std::vector<MpDpOut> ho(n);
@@ -519,6 +519,40 @@ extern "C" int mp_dp_batch(mp_context *ctx,
         if (ho[t].patLen) memcpy(pattern + (size_t)t * patStride, hp.data() + (size_t)t * patStride, ho[t].patLen + 1);
     }
     dRef.release(); dRead.release(); dRL.release(); dDL.release(); dCo.release(); dOut.release(); dPat.release();
+    return 0;
+}
+
+static_assert(sizeof(mp_dp_task) == sizeof(MpDpTask), "mp_dp_task mirrors MpDpTask");
+extern "C" int mp_dp_tasks(mp_context *ctx, const mp_dp_task *tasks, uint32_t n, uint32_t maxRefLen, uint32_t maxReadLen,
+                           uint32_t clipLt, uint32_t clipRt, int32_t *scores, uint32_t *hitLocs, uint32_t *maxScoreCounts, uint8_t *pattern)
+{
+    if (!ctx || !tasks || !scores || !hitLocs || !maxScoreCounts || !pattern) { mp_set_error("mp_dp_tasks: null argument"); return MP_ERR_ARG; }
+    if (!ctx->hasIndex || !ctx->hasBatch) { mp_set_error("mp_dp_tasks: index and batch must be loaded first"); return MP_ERR_STATE; }
+    if (n == 0) return 0;
+    for (uint32_t t = 0; t < n; ++t) {
+        const mp_dp_task &k = tasks[t];
+        if (!k.valid || k.refLen > maxRefLen || k.readLen > maxReadLen) continue;           // dropped by the kernels
+        if (k.refStart + k.refLen > ctx->ix.n || k.readID >= ctx->nReads || k.readLen > 16 * ctx->wpq) {
+            mp_set_error("mp_dp_tasks: task %u lies outside the text or the batch", t); return MP_ERR_ARG;
+        }
+    }
+    MP_CUDA(cudaSetDevice(ctx->device));
+    DevBuf dT, dOut, dPat;
+    const uint32_t patStride = maxRefLen + maxReadLen;
+    if (dT.reserve((size_t)n * sizeof(MpDpTask)) || dOut.reserve((size_t)n * sizeof(MpDpOut)) || dPat.reserve((size_t)n * patStride)) return MP_ERR_CUDA;
+    MP_CUDA(cudaMemcpy(dT.p, tasks, (size_t)n * sizeof(MpDpTask), cudaMemcpyHostToDevice));
+    MpDpParams P; P.clipLt = (int)clipLt; P.clipRt = (int)clipRt; P.mismatch = -2; P.open = -3;
+    if (int rc = mpd_run_tasks(ctx, dT.as<MpDpTask>(), n, maxRefLen, maxReadLen, P, dOut.as<MpDpOut>(), dPat.as<uint8_t>(), patStride)) return rc;
+    std::vector<MpDpOut> ho(n);
+    std::vector<uint8_t> hp((size_t)n * patStride);
+    MP_CUDA(cudaMemcpyAsync(ho.data(), dOut.p, (size_t)n * sizeof(MpDpOut), cudaMemcpyDeviceToHost, ctx->stream));
+    MP_CUDA(cudaMemcpyAsync(hp.data(), dPat.p, hp.size(), cudaMemcpyDeviceToHost, ctx->stream));
+    MP_CUDA(cudaStreamSynchronize(ctx->stream));
+    ctx->evUsed = 0;
+    for (uint32_t t = 0; t < n; ++t) {
+        scores[t] = ho[t].score; hitLocs[t] = ho[t].hitLoc; maxScoreCounts[t] = ho[t].count;
+        if (ho[t].patLen) memcpy(pattern + (size_t)t * patStride, hp.data() + (size_t)t * patStride, ho[t].patLen + 1);
+    }
     return 0;
 }
 
@@ -547,8 +581,9 @@ extern "C" int mp_reserve(mp_context *ctx, const mp_align_params *P, uint32_t nR
     const uint32_t CH3 = (uint32_t)std::min<uint64_t>(1u << 17, (uint64_t)nReads + 1024);
     const bool big = CH >= (1u << 15);
     const size_t tableWant = std::min<size_t>(big ? (size_t)24 << 30 : (size_t)(CH + 1) * tableStride, std::min<size_t>((size_t)24 << 30, freeB / 2));
-    const size_t refSeqWant = std::max<size_t>((((size_t)CH * maxDNALength + 15) & ~(size_t)15) + (size_t)CH * 14 + 16,
-                                               big && !P->skipDefaultDP ? (((size_t)CH3 * maxDNALengthR + 15) & ~(size_t)15) + (size_t)CH3 * 14 + 16 : 0);
+    // packed DP rows (mpd_run_tasks): 16 bases per word, plus lengths, cutoffs and hints
+    const size_t refSeqWant = std::max<size_t>((size_t)CH * ((maxDNALength + 15) / 16) * 4 + (size_t)CH * 14 + 16,
+                                               big && !P->skipDefaultDP ? (size_t)CH3 * ((maxDNALengthR + 15) / 16) * 4 + (size_t)CH3 * 14 + 16 : 0);
     const size_t patWant = std::max<size_t>((size_t)CH * patStride, big && !P->skipDefaultDP ? (size_t)CH3 * rStride : 0);
     if (ctx->dReadsIl.reserve(nPad * wpq * 4) || ctx->dReads.reserve(nPad * wpq * 4 + 64) || ctx->dLens.reserve((size_t)nReads * 4) ||
         ctx->dCounters.reserve(16 * 8) || ctx->dHitsPerRead.reserve(((size_t)nReads + 1) * 4) || ctx->dHitStart.reserve(((size_t)nReads + 1) * 4) ||
@@ -564,7 +599,7 @@ extern "C" int mp_reserve(mp_context *ctx, const mp_align_params *P, uint32_t nR
         ctx->dOff.reserve(((size_t)CH + 1) * 4) || ctx->dRes.reserve(resCap * sizeof(mp_pair_result)) || ctx->dRes2.reserve(resCap * sizeof(mp_pair_result)) ||
         ctx->dKeep.reserve((resCap + 1) * 4) || ctx->dKeepPos.reserve((resCap + 1) * 4) || ctx->dTotals.reserve(16 * 4) ||
         ctx->dCig.reserve(std::max<size_t>(resCap * 40, (size_t)1 << 20)) || ctx->dAligned.reserve((size_t)nPairs + 8) ||
-        ctx->dRefSeq.reserve(refSeqWant) || ctx->dReadSeq.reserve((size_t)CH * maxReadLength) ||
+        ctx->dRefSeq.reserve(refSeqWant) || ctx->dReadSeq.reserve((size_t)CH * ((maxReadLength + 15) / 16) * 4) ||
         ctx->dFill.reserve((size_t)CH * 16) || ctx->dExFlag.reserve(((size_t)CH + 1) * 4) || ctx->dExPos.reserve(((size_t)CH + 1) * 4) ||
         ctx->dExIdx.reserve(((size_t)CH + 1) * 4) || ctx->dScanTmp.reserve((size_t)1 << 20) || ctx->dS2Counts.reserve(((size_t)nReads + 1) * 4) || ctx->dS2Start.reserve(((size_t)nReads + 1) * 4) ||
         (ctx->dTable.cap < tableWant && ctx->dTable.reserve(tableWant))) return MP_ERR_CUDA;

@@ -46,7 +46,7 @@ __host__ __device__ inline CigStats cigar_encode(const uint8_t *__restrict__ pat
 
 #ifdef __CUDACC__
 #include "mp_context.h"
-// The special CIGAR of a leg and the encoder's statistics.  The traceback (k_dp_tb) and the exact-occurrence test (k_dp_exact) build
+// The special CIGAR of a leg and the encoder's statistics.  The traceback (k_dp_tb) and the exact-occurrence test (k_dp_prepare) build
 // both while they emit the pattern and leave the text at the end of the task's pattern row; only when pattern and text would not both
 // fit the row (hundreds of one-base runs) is the text encoded here from the pattern.
 __device__ __forceinline__ CigStats leg_stats(const MpDpOut &o)

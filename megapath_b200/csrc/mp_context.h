@@ -188,7 +188,7 @@ int mpd_run_tasks(mp_context *ctx, const MpDpTask *dTasks, uint32_t nTasks, uint
                   const MpDpParams &P, MpDpOut *dOuts, uint8_t *dPatterns, uint32_t patStride);
 // mp_stages.cu: single-end DP + default DP for the pairs stage S1 left unaligned
 int mps_single_and_rescue(mp_context *ctx, const mp_align_params *P, mp_results *out, uint64_t &cells, uint64_t &tasksRun);
-// explicit sequences (one byte per base, stride maxRefLen / maxReadLen)
-int mpd_run_explicit(mp_context *ctx, const uint8_t *dRef, const uint32_t *dRefLens, uint32_t maxRefLen,
-                     const uint8_t *dRead, const uint32_t *dReadLens, uint32_t maxReadLen, const int32_t *dCutoffs,
-                     uint32_t nTasks, const MpDpParams &P, MpDpOut *dOuts, uint8_t *dPatterns, uint32_t patStride);
+// explicit sequences: packed rows of ceil(maxRefLen / 16) / ceil(maxReadLen / 16) words, 16 bases per word, first base in the low bits
+int mpd_run_explicit(mp_context *ctx, uint32_t *dRef, uint32_t *dRefLens, uint32_t maxRefLen, uint32_t *dRead, uint32_t *dReadLens,
+                     uint32_t maxReadLen, int32_t *dCutoffs, uint32_t nTasks, const MpDpParams &P, MpDpOut *dOuts, uint8_t *dPatterns,
+                     uint32_t patStride);

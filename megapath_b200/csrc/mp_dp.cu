@@ -21,8 +21,8 @@
 // column in packed registers and reduced across the warp at the end.
 // k_dp_tb<K>: one thread per task walks its own table (GPUBacktrack, CPU_DP.cpp:622-786) -- thousands of
 // independent walks in flight hide the dependent-load latency that a single walking lane cannot.
-// k_dp_exact<K>: runs first; tasks whose read occurs unchanged in its window get their (provably identical) answer
-// without the DP, the others are compacted for the two kernels above.
+// k_dp_prepare: runs first; writes the tasks' packed sequence rows, and tasks whose read occurs unchanged in its window get their
+// (provably identical) answer without the DP, the others are compacted for the two kernels above.
 #include "mp_context.h"
 #include "mp_cigar.h"
 #include <cub/device/device_scan.cuh>
@@ -43,6 +43,8 @@ __device__ __forceinline__ int h0_value(int j, int clipLt, int open)       // ro
 {
     return j <= clipLt ? 0 : open - (j - clipLt - 1);
 }
+// base x of a packed row: 16 bases per word, first base in the low bits (the read order of the batch's dReads rows)
+__device__ __forceinline__ uint32_t packed_base(const uint32_t *row, int x) { return (row[x >> 4] >> ((x & 15) * 2)) & 3u; }
 __device__ __forceinline__ uint32_t pack2(int v) { return ((uint32_t)v & 0xffffu) * 0x00010001u; }
 __device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel)
 {
@@ -161,8 +163,8 @@ __device__ __noinline__ void dp_resolve_lane(const uint8_t *tab, int S, int j0, 
 // it is skipped -- and follows the lane's own best.
 template <int K, int MM, int OPEN, bool MASKED>
 __global__ void __launch_bounds__(128, K <= 5 ? MP_FILL_MINBLOCKS : K <= 8 ? 5 : 4)
-k_dp_fill(const uint8_t *__restrict__ refSeq, const uint32_t *__restrict__ refLens, uint32_t refStride,
-          const uint8_t *__restrict__ readSeq, const uint32_t *__restrict__ readLens, uint32_t readStride,
+k_dp_fill(const uint32_t *__restrict__ refSeq, const uint32_t *__restrict__ refLens, uint32_t refStride,
+          const uint32_t *__restrict__ readSeq, const uint32_t *__restrict__ readLens, uint32_t readStride,
           const int32_t *__restrict__ cutoffs, const int16_t *__restrict__ hints, uint32_t taskBase, uint32_t nTasks, MpDpParams P,
           uint8_t *__restrict__ tables, size_t tableStride, int S, FillOut *__restrict__ fill,
           const uint32_t *__restrict__ active, const uint32_t *__restrict__ nActive, uint32_t one)
@@ -171,7 +173,7 @@ k_dp_fill(const uint8_t *__restrict__ refSeq, const uint32_t *__restrict__ refLe
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const uint32_t pairId = blockIdx.x * 4 + wib;
     const uint32_t lA = pairId * 2, lB = lA + 1;             // slots inside this launch: tables are indexed by slot
-    if (active) nTasks = *nActive;                           // only the tasks the exact-occurrence test left over (k_dp_exact)
+    if (active) nTasks = *nActive;                           // only the tasks the exact-occurrence test left over (k_dp_prepare)
     if (lA >= nTasks) return;
     const bool hasB = lB < nTasks;
     const uint32_t tA = taskBase + (active ? active[lA] : lA), tB = hasB ? taskBase + (active ? active[lB] : lB) : tA;
@@ -194,16 +196,16 @@ k_dp_fill(const uint8_t *__restrict__ refSeq, const uint32_t *__restrict__ refLe
     //      rows a task does not have mismatch everything ----
     uint2 *refS = refShared + (size_t)wib * S;
     {
-        const uint8_t *fa = refSeq + (size_t)tA * refStride, *fb = refSeq + (size_t)tB * refStride;
+        const uint32_t *fa = refSeq + (size_t)tA * refStride, *fb = refSeq + (size_t)tB * refStride;
         const uint32_t all = TMIS * 0x01010101u;
         for (int r = lane; r < maxN; r += 32) {
-            const uint32_t a = r < NA ? fa[r] : 4u, b = r < NB ? fb[r] : 4u;
+            const uint32_t a = r < NA ? packed_base(fa, r) : 4u, b = r < NB ? packed_base(fb, r) : 4u;
             refS[r] = make_uint2(a < 4u ? (all & ~(0xFFu << (8 * a))) | (TMATCH << (8 * a)) : all,
                                  b < 4u ? (all & ~(0xFFu << (8 * b))) | (TMATCH << (8 * b)) : all);
         }
     }
     __syncwarp();
-    const uint8_t *ra = readSeq + (size_t)tA * readStride, *rbp = readSeq + (size_t)tB * readStride;
+    const uint32_t *ra = readSeq + (size_t)tA * readStride, *rbp = readSeq + (size_t)tB * readStride;
     const int j0 = lane * K + 1;
     // per column: PRMT selector (nibble 0 = A's base, nibble 2 = 4 + B's base, nibbles 1 / 3 replicate the sign bit of the same
     // byte = 0), H of the row above in open form (H + open: what D and I consume, and with FOLD the diagonal too), D, clip floor
@@ -214,7 +216,7 @@ k_dp_fill(const uint8_t *__restrict__ refSeq, const uint32_t *__restrict__ refLe
 #pragma unroll
     for (int k = 0; k < K; ++k) {
         const int j = j0 + k;
-        const uint32_t a = j <= LA ? ra[j - 1] & 3u : 0u, b = j <= LB ? rbp[j - 1] & 3u : 0u;
+        const uint32_t a = j <= LA ? packed_base(ra, j - 1) : 0u, b = j <= LB ? packed_base(rbp, j - 1) : 0u;
         basesA |= a << (2 * k); basesB |= b << (2 * k);
         sel[k] = a | ((8u | a) << 4) | ((4u + b) << 8) | ((12u + b) << 12);
         // !MASKED (see the tracker below): a column beyond the read takes addend 0 -- a substitution score of `open`, below any real one
@@ -457,11 +459,11 @@ k_dp_fill(const uint8_t *__restrict__ refSeq, const uint32_t *__restrict__ refLe
 // ---- GPUBacktrack (CPU_DP.cpp:622-786), literal; one thread per task ----
 // The walk is bound by memory TRANSACTIONS (every lane of a warp touches its own sector), so all three streams go through
 // one-word register caches: the trace table (a diagonal run of four cells shares a word, see cell_offset), the two sequences
-// (aligned 4-base words) and the pattern (four bytes per store; WORDPAT needs patStride % 4 == 0).
+// (packed words of 16 bases) and the pattern (four bytes per store; WORDPAT needs patStride % 4 == 0).
 template <int K, bool WORDPAT>
 __global__ void __launch_bounds__(128)
-k_dp_tb(const uint8_t *__restrict__ refSeq, const uint32_t *__restrict__ refLens, uint32_t refStride,
-        const uint8_t *__restrict__ readSeq, const uint32_t *__restrict__ readLens, uint32_t readStride,
+k_dp_tb(const uint32_t *__restrict__ refSeq, const uint32_t *__restrict__ refLens, uint32_t refStride,
+        const uint32_t *__restrict__ readSeq, const uint32_t *__restrict__ readLens, uint32_t readStride,
         const int32_t *__restrict__ cutoffs, uint32_t taskBase, uint32_t nTasks, MpDpParams P,
         const uint8_t *__restrict__ tables, size_t tableStride, int S, const FillOut *__restrict__ fill,
         MpDpOut *__restrict__ outs, uint8_t *__restrict__ patterns, uint32_t patStride,
@@ -495,17 +497,15 @@ k_dp_tb(const uint8_t *__restrict__ refSeq, const uint32_t *__restrict__ refLens
         if (c == 0) return 0;
         return trace_h(cellAt(r, c));
     };
-    const size_t rsOff = (size_t)task * readStride, fsOff = (size_t)task * refStride;
-    uint32_t rsW = 0, fsW = 0; size_t rsIdx = ~(size_t)0, fsIdx = ~(size_t)0;
+    const uint32_t *rsRow = readSeq + (size_t)task * readStride, *fsRow = refSeq + (size_t)task * refStride;
+    uint32_t rsW = 0, fsW = 0; int rsIdx = -1, fsIdx = -1;
     auto readBase = [&](int x) -> uint32_t {
-        const size_t a = rsOff + x;
-        if ((a >> 2) != rsIdx) { rsIdx = a >> 2; rsW = __ldg((const uint32_t *)readSeq + rsIdx); }
-        return (rsW >> ((a & 3) * 8)) & 0xffu;
+        if ((x >> 4) != rsIdx) { rsIdx = x >> 4; rsW = __ldg(rsRow + rsIdx); }
+        return (rsW >> ((x & 15) * 2)) & 3u;
     };
     auto refBase = [&](int x) -> uint32_t {
-        const size_t a = fsOff + x;
-        if ((a >> 2) != fsIdx) { fsIdx = a >> 2; fsW = __ldg((const uint32_t *)refSeq + fsIdx); }
-        return (fsW >> ((a & 3) * 8)) & 0xffu;
+        if ((x >> 4) != fsIdx) { fsIdx = x >> 4; fsW = __ldg(fsRow + fsIdx); }
+        return (fsW >> ((x & 15) * 2)) & 3u;
     };
     uint32_t p = 0, pacc = 0;
     auto emit = [&](uint32_t byte) {
@@ -612,6 +612,13 @@ k_dp_tb(const uint8_t *__restrict__ refSeq, const uint32_t *__restrict__ refLens
 }
 
 // ------------------------------------------------------------------------------------
+// k_dp_prepare: one warp per task of a sub-batch, ahead of the DP kernels.
+//  * tasks != nullptr (mpd_run_tasks; replaces packRead / repackDNA): gathers the task's reference window from the packed text and its
+//    read from the batch, oriented (strand 2 reverse-complemented), into the task's two packed rows, and writes its scalars.  A task
+//    that does not fit its rows is dropped (refLen = readLen = 0, hint -1), never written past them.
+//  * tasks == nullptr (mpd_run_explicit): rows and scalars are already in place.
+//  * needDp != nullptr: runs the exact-occurrence test on the packed words and sets needDp for every slot of the sub-batch.
+//
 // Exact-occurrence test.  If the read occurs in its reference window without a single difference, the DP answer is known:
 //  * no cell can exceed its column index (a column adds at most the match score 1; clips, gaps and mismatches add <= 0), so the
 //    maximum over the eligible columns is L, reached only in column L, exactly at the rows where an occurrence ends;
@@ -619,45 +626,96 @@ k_dp_tb(const uint8_t *__restrict__ refSeq, const uint32_t *__restrict__ refLens
 //  * on the diagonal of an occurrence H = column index, so every traceback step sees H - Hdiag = 1 with equal bases, no cell of the
 //    diagonal was raised by the clip floor (H >= 1 there), and GPUBacktrack emits L times 'M'; it stops at column 0, and when that
 //    is also row 0 it appends the zero-length left clip "SV\0" (CPU_DP.cpp:788-871).
-// Such tasks skip k_dp_fill / k_dp_tb; the others are compacted into `active`.  One warp per task, one lane per window offset.
+// Such tasks skip k_dp_fill / k_dp_tb; the others are compacted into `active`.  Every lane screens window offsets o, o + 32, ...: one
+// XOR of a funnel-shifted pair of window words against a read word compares 16 bases.
 // ------------------------------------------------------------------------------------
-template <int K>
-__global__ void __launch_bounds__(128)
-k_dp_exact(const uint8_t *__restrict__ refSeq, const uint32_t *__restrict__ refLens, uint32_t refStride,
-           const uint8_t *__restrict__ readSeq, const uint32_t *__restrict__ readLens, uint32_t readStride,
-           const int32_t *__restrict__ cutoffs, uint32_t taskBase, uint32_t nTasks, MpDpParams P,
-           MpDpOut *__restrict__ outs, uint8_t *__restrict__ patterns, uint32_t patStride, uint32_t *__restrict__ needDp)
+// 16 bases of the packed text (4 bases per byte, first base in the top bits) as one little-endian word -> first base in the low bits
+__device__ __forceinline__ uint32_t pac_word(uint32_t x)
 {
+    x = ((x >> 4) & 0x0F0F0F0Fu) | ((x & 0x0F0F0F0Fu) << 4);
+    return ((x >> 2) & 0x33333333u) | ((x & 0x33333333u) << 2);
+}
+__device__ __forceinline__ uint32_t reverse_bases(uint32_t x)          // base k -> base 15 - k
+{
+    x = __brev(x);
+    return ((x >> 1) & 0x55555555u) | ((x & 0x55555555u) << 1);
+}
+__device__ __forceinline__ uint32_t base_mask(int n) { return n >= 16 ? 0xffffffffu : (1u << (2 * n)) - 1u; }   // the first n > 0 bases
+
+__global__ void __launch_bounds__(128)
+k_dp_prepare(MpIndexView ix, const uint32_t *__restrict__ reads, uint32_t wpq, const MpDpTask *__restrict__ tasks,
+             uint32_t maxRefLen, uint32_t maxReadLen, uint32_t *__restrict__ refSeq, uint32_t refStride,
+             uint32_t *__restrict__ readSeq, uint32_t readStride, uint32_t *__restrict__ refLens, uint32_t *__restrict__ readLens,
+             int32_t *__restrict__ cutoffs, int16_t *__restrict__ hints, uint32_t taskBase, uint32_t nTasks, int maxL, MpDpParams P,
+             MpDpOut *__restrict__ outs, uint8_t *__restrict__ patterns, uint32_t patStride, uint32_t *__restrict__ needDp)
+{
+    extern __shared__ uint32_t prepShared[];            // per warp: the window row + one zero word, the read row
     const int lane = threadIdx.x & 31;
     const uint32_t lt = blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (lt == 0 && lane == 0 && needDp) needDp[nTasks] = 0;      // the scan runs over nTasks + 1 flags: the last sum is the total
     if (lt >= nTasks) return;
     const uint32_t task = taskBase + lt;
-    const int N = (int)refLens[task], L = (int)readLens[task], cutoff = cutoffs[task];
-    // same admission test as the DP kernels; scores must be the usual kind (match 1, everything else <= 0)
-    const bool ok = !(cutoff > L || cutoff <= 0 || L >= 255 + P.open - 1 + cutoff || L > 32 * K) && L > 0 && N >= L &&
-                    P.mismatch <= 0 && P.open <= 0;
-    uint32_t occ = 0; int first = -1;
-    if (ok) {
-        const uint8_t *fs = refSeq + (size_t)task * refStride, *rs = readSeq + (size_t)task * readStride;
-        const int shifts = N - L + 1;
-        // every lane screens one window offset with the first bases of the read; the few offsets that survive are then verified by
-        // the whole warp, one base per lane and trip
-        const int PRE = L < 8 ? L : 8;
-        for (int base = 0; base < shifts; base += 32) {
-            const int o = base + lane;
-            bool alive = o < shifts;
-#pragma unroll
-            for (int k = 0; k < 8; ++k)
-                if (alive && k < PRE) alive = fs[o + k] == rs[k];
-            uint32_t cand = __ballot_sync(0xffffffffu, alive);
-            while (cand) {
-                const int oc = base + __ffs(cand) - 1;
-                cand &= cand - 1;
-                bool same = true;
-                for (int k = PRE + lane; k < L; k += 32) same = same && fs[oc + k] == rs[k];
-                if (__all_sync(0xffffffffu, same)) { if (first < 0) first = oc; ++occ; }
+    uint32_t *win = prepShared + (threadIdx.x >> 5) * (refStride + 1 + readStride), *rw = win + refStride + 1;
+    uint32_t *fo = refSeq + (size_t)task * refStride, *ro = readSeq + (size_t)task * readStride;
+    int N, L, cutoff;
+    if (tasks) {
+        MpDpTask tk = tasks[task];
+        if (!tk.valid || tk.refLen > maxRefLen || tk.readLen > maxReadLen) { tk.refLen = 0; tk.valid = 0; }
+        N = (int)tk.refLen; L = tk.valid ? (int)tk.readLen : 0; cutoff = tk.cutoff;
+        // window word w = text bases refStart + 16w .. + 15, from two aligned words of the text (the text buffer is allocation-aligned and
+        // padded behind its last byte)
+        const uint32_t *pac32 = (const uint32_t *)ix.pac;
+        for (int w = lane; w < (int)refStride; w += 32) {
+            uint32_t v = 0;
+            if (16 * w < N) {
+                const uint64_t p = tk.refStart + 16 * (uint32_t)w;
+                const uint32_t sh = (uint32_t)(p & 15) * 2;
+                const uint32_t lo = pac_word(__ldg(pac32 + (p >> 4))), hi = sh ? pac_word(__ldg(pac32 + (p >> 4) + 1)) : 0u;
+                v = __funnelshift_r(lo, hi, sh) & base_mask(N - 16 * w);
             }
+            fo[w] = v; win[w] = v;
         }
+        const uint32_t *rd = reads + (size_t)tk.readID * wpq;
+        for (int w = lane; w < (int)readStride; w += 32) {
+            uint32_t v = 0;
+            if (16 * w < L) {
+                if (tk.strand == 1) v = rd[w];
+                else {
+                    // reverse complement: base 16w + k = 3 - read[L-1-16w-k], the complement of read[s .. s+15] reversed, s = L-16-16w >= -15
+                    const int s = L - 16 - 16 * w, s0 = s < 0 ? 0 : s;
+                    uint32_t x = __funnelshift_r(rd[s0 >> 4], (s0 & 15) ? rd[(s0 >> 4) + 1] : 0u, (uint32_t)(s0 & 15) * 2);
+                    if (s < 0) x <<= 2 * (uint32_t)(-s);                      // base k = read[s + k]
+                    v = ~reverse_bases(x);
+                }
+                v &= base_mask(L - 16 * w);
+            }
+            ro[w] = v; rw[w] = v;
+        }
+        if (lane == 0) { refLens[task] = (uint32_t)N; readLens[task] = (uint32_t)L; cutoffs[task] = cutoff; hints[task] = tk.valid ? tk.diag : (int16_t)-1; }
+    } else {
+        N = (int)refLens[task]; L = (int)readLens[task]; cutoff = cutoffs[task];
+        for (int w = lane; w < (int)refStride; w += 32) win[w] = fo[w];
+        for (int w = lane; w < (int)readStride; w += 32) rw[w] = ro[w];
+    }
+    if (!needDp) return;
+    if (lane == 0) win[refStride] = 0u;                  // the funnel shift of the window's last word reads one word further
+    __syncwarp();
+    // same admission test as the DP kernels; scores must be the usual kind (match 1, everything else <= 0)
+    const bool ok = !(cutoff > L || cutoff <= 0 || L >= 255 + P.open - 1 + cutoff || L > maxL) && L > 0 && N >= L &&
+                    P.mismatch <= 0 && P.open <= 0;
+    uint32_t occ = 0, first = 0xffffffffu;
+    if (ok) {
+        const int nw = (L + 15) >> 4;
+        const uint32_t m0 = nw == 1 ? base_mask(L) : 0xffffffffu;
+        for (int o = lane; o <= N - L; o += 32) {
+            const uint32_t *wq = win + (o >> 4), sh = (uint32_t)(o & 15) * 2;
+            bool same = ((__funnelshift_r(wq[0], wq[1], sh) ^ rw[0]) & m0) == 0;
+            for (int k = 1; same && k < nw; ++k)
+                same = ((__funnelshift_r(wq[k], wq[k + 1], sh) ^ rw[k]) & (k + 1 == nw ? base_mask(L - 16 * k) : 0xffffffffu)) == 0;
+            if (same) { first = min(first, (uint32_t)o); ++occ; }
+        }
+        occ = __reduce_add_sync(0xffffffffu, occ);
+        first = __reduce_min_sync(0xffffffffu, first);
     }
     if (occ == 0) { if (lane == 0) needDp[lt] = 1; return; }
     uint8_t *pat = patterns + (size_t)task * patStride;
@@ -667,7 +725,7 @@ k_dp_exact(const uint8_t *__restrict__ refSeq, const uint32_t *__restrict__ refL
         if (first == 0) { pat[p++] = 'S'; pat[p++] = 'V'; pat[p++] = 0; }      // j == 0: min(clipLt, i = 0) = 0 clipped bases
         pat[p] = 0;
         MpDpOut o; memset(&o, 0, sizeof o);
-        o.score = L; o.hitLoc = (uint32_t)first; o.count = min(occ, 255u); o.patLen = p;
+        o.score = L; o.hitLoc = first; o.count = min(occ, 255u); o.patLen = p;
         // its CIGAR is "<L>M" (a zero-length clip prints nothing), kept at the end of the pattern row like k_dp_tb does
         const int nd = ndigits(L);
         if (P.cigText && p + 8 + nd + 1 <= patStride) {
@@ -696,66 +754,15 @@ __global__ void k_dp_compact(const uint32_t *__restrict__ needDp, const uint32_t
     if ((threadIdx.x & 31) == 0 && counters) { if (cells) atomicAdd(&counters[15], cells); if (exact) atomicAdd(&counters[14], (unsigned long long)exact); }
 }
 
-// ------------------------------------------------------------------------------------
-// task sequence extraction (replaces packRead / repackDNA): one byte per base
-// ------------------------------------------------------------------------------------
-__global__ void k_extract(MpIndexView ix, const uint32_t *__restrict__ reads, uint32_t wpq, const MpDpTask *__restrict__ tasks,
-                          uint32_t nTasks, uint8_t *__restrict__ refSeq, uint32_t refStride, uint8_t *__restrict__ readSeq,
-                          uint32_t readStride, uint32_t *__restrict__ refLens, uint32_t *__restrict__ readLens, int32_t *__restrict__ cutoffs,
-                          int16_t *__restrict__ hints)
-{
-    const uint32_t task = blockIdx.x;
-    if (task >= nTasks) return;
-    MpDpTask tk = tasks[task];
-    // a task that does not fit its rows is dropped, never written past them (callers size the strides from -L / -u)
-    if (!tk.valid || tk.refLen > refStride || tk.readLen > readStride) { tk.refLen = 0; tk.valid = 0; }
-    const uint32_t *rd = reads + (size_t)tk.readID * wpq;
-    if (((refStride | readStride) & 3u) == 0) {
-        // four bases per thread and trip: one packed byte's worth of text (or of the read) becomes one 32-bit store.  Rows are
-        // multiples of four bytes long, so the last word of a row may carry up to three bases nobody reads.
-        uint32_t *fo = (uint32_t *)(refSeq + (size_t)task * refStride), *ro = (uint32_t *)(readSeq + (size_t)task * readStride);
-        for (uint32_t a = threadIdx.x * 4; a < tk.refLen; a += blockDim.x * 4) {
-            const uint64_t p = tk.refStart + a;
-            const uint32_t x = ((uint32_t)__ldg(ix.pac + (p >> 2)) << 8) | __ldg(ix.pac + (p >> 2) + 1);      // first base in the top bits
-            const uint32_t v = (x >> (8 - 2 * (uint32_t)(p & 3))) & 0xFFu;
-            fo[a >> 2] = (v >> 6) | (((v >> 4) & 3u) << 8) | (((v >> 2) & 3u) << 16) | ((v & 3u) << 24);
-        }
-        const uint32_t L = tk.valid ? tk.readLen : 0;
-        for (uint32_t a = threadIdx.x * 4; a < L; a += blockDim.x * 4) {
-            uint32_t w;
-            if (tk.strand == 1) {
-                const uint32_t v = (rd[a >> 4] >> ((a & 15) << 1)) & 0xFFu;                                     // bases a .. a+3, first in the low bits
-                w = (v & 3u) | (((v >> 2) & 3u) << 8) | (((v >> 4) & 3u) << 16) | ((v >> 6) << 24);
-            } else {
-                // reverse complement: output a+k = 3 - read[L-1-a-k]; the four source bases start at s = L-4-a (may reach below 0)
-                const int s = (int)L - 4 - (int)a;
-                const int s0 = s < 0 ? 0 : s;
-                const uint32_t lo = rd[s0 >> 4], hi = rd[(s0 >> 4) + ((s0 & 15) > 12 ? 1 : 0)];
-                uint32_t v = (__funnelshift_r(lo, hi, (s0 & 15) << 1)) & 0xFFu;                                 // read[s0 .. s0+3], first in the low bits
-                if (s < 0) v <<= (uint32_t)(-s) * 2;                                                            // keep read[L-1-a] in the top pair
-                v = ~v & 0xFFu;
-                w = (v >> 6) | (((v >> 4) & 3u) << 8) | (((v >> 2) & 3u) << 16) | ((v & 3u) << 24);
-            }
-            ro[a >> 2] = w;
-        }
-    } else {
-        for (uint32_t a = threadIdx.x; a < tk.refLen; a += blockDim.x)
-            refSeq[(size_t)task * refStride + a] = (uint8_t)mp_text_base(ix, tk.refStart + a);
-        for (uint32_t a = threadIdx.x; tk.valid && a < tk.readLen; a += blockDim.x) {
-            uint32_t p = tk.strand == 1 ? a : tk.readLen - 1 - a;
-            uint32_t b = (rd[p >> 4] >> ((p & 15) << 1)) & 3;
-            readSeq[(size_t)task * readStride + a] = (uint8_t)(tk.strand == 1 ? b : 3 - b);
-        }
-    }
-    if (threadIdx.x == 0) { refLens[task] = tk.refLen; readLens[task] = tk.valid ? tk.readLen : 0; cutoffs[task] = tk.cutoff; hints[task] = tk.valid ? tk.diag : (int16_t)-1; }
-}
-
-static int launch_dp(mp_context *ctx, const uint8_t *dRef, const uint32_t *dRefLens, uint32_t refStride,
-                     const uint8_t *dRead, const uint32_t *dReadLens, uint32_t readStride, const int32_t *dCutoffs,
-                     uint32_t nTasks, uint32_t maxRefLen, uint32_t maxReadLen, const MpDpParams &Pin,
-                     MpDpOut *dOuts, uint8_t *dPatterns, uint32_t patStride, const int16_t *dHints)
+// Packed rows (k_dp_prepare, k_dp_fill, k_dp_tb): per task a window row of ceil(maxRefLen / 16) and a read row of ceil(maxReadLen / 16)
+// words, 16 bases per word, first base in the low bits; the read already oriented.  Bases beyond a row's length are zero.
+// dTasks != nullptr: k_dp_prepare fills rows, lengths, cutoffs and hints from the tasks; otherwise they are in place (dHints may be null).
+static int launch_dp(mp_context *ctx, const MpDpTask *dTasks, uint32_t *dRef, uint32_t *dRefLens, uint32_t *dRead, uint32_t *dReadLens,
+                     int32_t *dCutoffs, int16_t *dHints, uint32_t nTasks, uint32_t maxRefLen, uint32_t maxReadLen, const MpDpParams &Pin,
+                     MpDpOut *dOuts, uint8_t *dPatterns, uint32_t patStride)
 {
     if (nTasks == 0) return 0;
+    const uint32_t refStride = (maxRefLen + 15) >> 4, readStride = (maxReadLen + 15) >> 4;
     MpDpParams P = Pin;
     if (const char *e = getenv("MP_CIG_TEXT")) if (e[0] == '0') P.cigText = 0;       // tests: the assembly pass encodes every CIGAR from its pattern
     const int K = maxReadLen <= 160 ? 5 : maxReadLen <= 256 ? 8 : 10;
@@ -782,7 +789,7 @@ static int launch_dp(mp_context *ctx, const uint8_t *dRef, const uint32_t *dRefL
     uint8_t *tab = ctx->dTable.as<uint8_t>();
     FillOut *fill = ctx->dFill.as<FillOut>();
     const size_t smem = (size_t)4 * S * sizeof(uint2);          // one 8-byte substitution table per reference row and warp
-    // exact-occurrence shortcut (k_dp_exact): MP_DP_EXACT=0 sends every task through the DP kernels
+    // exact-occurrence shortcut (k_dp_prepare): MP_DP_EXACT=0 sends every task through the DP kernels
     static const bool useExact = !(getenv("MP_DP_EXACT") && getenv("MP_DP_EXACT")[0] == '0');
     // the lean tracker of k_dp_fill takes a lane's row maximum over all of its columns: legal when no column left of the eligible range
     // (j < L - clipRt) can reach a cutoff, i.e. L - clipRt - 1 < 30 <= cutoff for every read length of the batch (definitions.h:166-167)
@@ -790,24 +797,29 @@ static int launch_dp(mp_context *ctx, const uint8_t *dRef, const uint32_t *dRefL
     const uint32_t perMax = std::min<uint32_t>(per, nTasks);
     if (useExact && (ctx->dExFlag.reserve(((size_t)perMax + 1) * 4) || ctx->dExPos.reserve(((size_t)perMax + 1) * 4) ||
                      ctx->dExIdx.reserve(((size_t)perMax + 1) * 4) || ctx->dCounters.reserve(16 * 8))) return MP_ERR_CUDA;
+    const size_t prepSmem = (size_t)4 * (refStride + 1 + readStride) * 4;
     for (uint32_t base = 0; base < nTasks; base += per) {
         const uint32_t n = std::min<uint32_t>(per, nTasks - base);
         dim3 gridF((n + 7) / 8), gridT((n + 127) / 128), block(128);
         const uint32_t *active = nullptr, *nActive = nullptr;
-#define LAUNCH_EXACT(KK) do { \
-        cudaEvent_t stop_ = ctx->ev_begin(2); \
-        MP_CUDA(cudaMemsetAsync(ctx->dExFlag.p, 0, ((size_t)n + 1) * 4, ctx->stream)); \
-        (++g_mp_launches), k_dp_exact<KK><<<(n + 3) / 4, block, 0, ctx->stream>>>(dRef, dRefLens, refStride, dRead, dReadLens, readStride, dCutoffs, \
-            base, n, P, dOuts, dPatterns, patStride, ctx->dExFlag.as<uint32_t>()); \
-        { size_t tb_ = 0; cub::DeviceScan::ExclusiveSum(nullptr, tb_, ctx->dExFlag.as<uint32_t>(), ctx->dExPos.as<uint32_t>(), (int64_t)n + 1, ctx->stream); \
-          if (ctx->dScanTmp.reserve(tb_)) return MP_ERR_CUDA; \
-          cub::DeviceScan::ExclusiveSum(ctx->dScanTmp.p, tb_, ctx->dExFlag.as<uint32_t>(), ctx->dExPos.as<uint32_t>(), (int64_t)n + 1, ctx->stream); } \
-        (++g_mp_launches), k_dp_compact<<<(n + 255) / 256, 256, 0, ctx->stream>>>(ctx->dExFlag.as<uint32_t>(), ctx->dExPos.as<uint32_t>(), n, base, \
-            dRefLens, dReadLens, ctx->dExIdx.as<uint32_t>(), ctx->dCounters.as<unsigned long long>()); \
-        active = ctx->dExIdx.as<uint32_t>(); nActive = ctx->dExPos.as<uint32_t>() + n; \
-        ctx->ev_end(stop_); } while (0)
+        if (dTasks || useExact) {
+            cudaEvent_t stop_ = ctx->ev_begin(2);
+            uint32_t *needDp = useExact ? ctx->dExFlag.as<uint32_t>() : nullptr;
+            (++g_mp_launches), k_dp_prepare<<<(n + 3) / 4, block, prepSmem, ctx->stream>>>(ctx->ix, ctx->dReads.as<uint32_t>(), ctx->wpq, dTasks,
+                maxRefLen, maxReadLen, dRef, refStride, dRead, readStride, dRefLens, dReadLens, dCutoffs, dHints, base, n, 32 * K, P,
+                dOuts, dPatterns, patStride, needDp);
+            if (useExact) {
+                size_t tb = 0;
+                cub::DeviceScan::ExclusiveSum(nullptr, tb, needDp, ctx->dExPos.as<uint32_t>(), (int64_t)n + 1, ctx->stream);
+                if (ctx->dScanTmp.reserve(tb)) return MP_ERR_CUDA;
+                cub::DeviceScan::ExclusiveSum(ctx->dScanTmp.p, tb, needDp, ctx->dExPos.as<uint32_t>(), (int64_t)n + 1, ctx->stream);
+                (++g_mp_launches), k_dp_compact<<<(n + 255) / 256, 256, 0, ctx->stream>>>(needDp, ctx->dExPos.as<uint32_t>(), n, base,
+                    dRefLens, dReadLens, ctx->dExIdx.as<uint32_t>(), ctx->dCounters.as<unsigned long long>());
+                active = ctx->dExIdx.as<uint32_t>(); nActive = ctx->dExPos.as<uint32_t>() + n;
+            }
+            ctx->ev_end(stop_);
+        }
 #define LAUNCH(KK) do { \
-        if (useExact) LAUNCH_EXACT(KK); \
         cudaEvent_t stop_ = ctx->ev_begin(0); \
         if (P.mismatch == -2 && P.open == -3 && rowMaxOk) { \
             if (smem > 48 * 1024) MP_CUDA(cudaFuncSetAttribute(k_dp_fill<KK, -2, -3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
@@ -832,19 +844,18 @@ static int launch_dp(mp_context *ctx, const uint8_t *dRef, const uint32_t *dRefL
         ctx->ev_end(stop_); } while (0)
         if (K == 5) LAUNCH(5); else if (K == 8) LAUNCH(8); else LAUNCH(10);
 #undef LAUNCH
-#undef LAUNCH_EXACT
         MP_CUDA(cudaGetLastError());
     }
     return 0;
 }
 
-int mpd_run_explicit(mp_context *ctx, const uint8_t *dRef, const uint32_t *dRefLens, uint32_t maxRefLen,
-                     const uint8_t *dRead, const uint32_t *dReadLens, uint32_t maxReadLen, const int32_t *dCutoffs,
-                     uint32_t nTasks, const MpDpParams &P, MpDpOut *dOuts, uint8_t *dPatterns, uint32_t patStride)
+int mpd_run_explicit(mp_context *ctx, uint32_t *dRef, uint32_t *dRefLens, uint32_t maxRefLen, uint32_t *dRead, uint32_t *dReadLens,
+                     uint32_t maxReadLen, int32_t *dCutoffs, uint32_t nTasks, const MpDpParams &P, MpDpOut *dOuts, uint8_t *dPatterns,
+                     uint32_t patStride)
 {
     // The SemiGlobalAligner seam carries no seed diagonal: the fill kernel's threshold starts at the cutoff.  MP_DP_TEST_HINT=<d> (parity
     // tests) hands every task the same diagonal hint instead, right or wrong -- results must not depend on it.
-    const int16_t *dHints = nullptr;
+    int16_t *dHints = nullptr;
     if (const char *e = getenv("MP_DP_TEST_HINT")) {
         std::vector<int16_t> h(nTasks, (int16_t)atoi(e));
         if (ctx->dHintTest.reserve((size_t)nTasks * 2)) return MP_ERR_CUDA;
@@ -852,24 +863,22 @@ int mpd_run_explicit(mp_context *ctx, const uint8_t *dRef, const uint32_t *dRefL
         MP_CUDA(cudaStreamSynchronize(ctx->stream));
         dHints = ctx->dHintTest.as<int16_t>();
     }
-    return launch_dp(ctx, dRef, dRefLens, maxRefLen, dRead, dReadLens, maxReadLen, dCutoffs, nTasks, maxRefLen, maxReadLen, P,
-                     dOuts, dPatterns, patStride, dHints);
+    return launch_dp(ctx, nullptr, dRef, dRefLens, dRead, dReadLens, dCutoffs, dHints, nTasks, maxRefLen, maxReadLen, P,
+                     dOuts, dPatterns, patStride);
 }
 
 int mpd_run_tasks(mp_context *ctx, const MpDpTask *dTasks, uint32_t nTasks, uint32_t maxRefLen, uint32_t maxReadLen,
                   const MpDpParams &P, MpDpOut *dOuts, uint8_t *dPatterns, uint32_t patStride)
 {
     if (nTasks == 0) return 0;
-    size_t refB = ((size_t)nTasks * maxRefLen + 15) & ~(size_t)15, readB = (size_t)nTasks * maxReadLen;
-    if (ctx->dRefSeq.reserve(refB + (size_t)nTasks * 14 + 16) || ctx->dReadSeq.reserve(readB)) return MP_ERR_CUDA;
-    uint8_t *dRef = ctx->dRefSeq.as<uint8_t>();
-    uint32_t *dRefLens = (uint32_t *)(dRef + refB);
+    // packed rows (launch_dp), then lengths, cutoffs and hints of every task
+    const size_t refW = (size_t)nTasks * ((maxRefLen + 15) >> 4), readW = (size_t)nTasks * ((maxReadLen + 15) >> 4);
+    if (ctx->dRefSeq.reserve(refW * 4 + (size_t)nTasks * 14 + 16) || ctx->dReadSeq.reserve(readW * 4)) return MP_ERR_CUDA;
+    uint32_t *dRef = ctx->dRefSeq.as<uint32_t>();
+    uint32_t *dRefLens = dRef + refW;
     uint32_t *dReadLens = dRefLens + nTasks;
     int32_t *dCutoffs = (int32_t *)(dReadLens + nTasks);
     int16_t *dHints = (int16_t *)(dCutoffs + nTasks);
-    (++g_mp_launches), k_extract<<<nTasks, 64, 0, ctx->stream>>>(ctx->ix, ctx->dReads.as<uint32_t>(), ctx->wpq, dTasks, nTasks, dRef, maxRefLen,
-                                             ctx->dReadSeq.as<uint8_t>(), maxReadLen, dRefLens, dReadLens, dCutoffs, dHints);
-    MP_CUDA(cudaGetLastError());
-    return launch_dp(ctx, dRef, dRefLens, maxRefLen, ctx->dReadSeq.as<uint8_t>(), dReadLens, maxReadLen, dCutoffs, nTasks,
-                     maxRefLen, maxReadLen, P, dOuts, dPatterns, patStride, dHints);
+    return launch_dp(ctx, dTasks, dRef, dRefLens, ctx->dReadSeq.as<uint32_t>(), dReadLens, dCutoffs, dHints, nTasks, maxRefLen, maxReadLen, P,
+                     dOuts, dPatterns, patStride);
 }
